@@ -2,6 +2,7 @@
 """Benchmark of the batched ICP hot path: ICP scan-pair alignments / second.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -49,6 +50,7 @@ METRIC = "icp_scan_pair_alignments_per_sec"
 UNIT = "pairs/s"
 SEED = 467002
 EPS, MAX_ITERS = 0.05, 100
+DUMP_BYTES = 64_000_000                                      # cap on what --dump-outputs writes
 # counters of the timed kernel from a committed `ncu --set full` capture of this same command
 # (written by tools/ncu_summary.py; carries the commit it was taken at)
 NCU_SUMMARY = os.path.join(ROOT, "profiles", "r02_align_ncu_summary.json")
@@ -72,7 +74,11 @@ def parse():
     ap.add_argument("--no-sustained", action="store_true", help="skip the sustained-clock segment")
     ap.add_argument("--no-exhaustive", action="store_true", help="skip the pruning-off launches (long workloads)")
     ap.add_argument("--threads", type=int, default=0, help="tuning: cap on the CTA width (icpb_set_tuning)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     dflt = {"chain": (5000, 1024), "proximity": (5000, 1024), "allpairs": (600, 1024), "highres": (48, 4096)}
     args.scans = args.scans or dflt[args.workload][0]
     args.beams = args.beams or dflt[args.workload][1]
@@ -206,6 +212,21 @@ def identity_init(n):
     return np.broadcast_to(np.eye(3), (n, 3, 3)).copy()
 
 
+def dump_outputs(out_dir, rows, T6, err, passes):
+    """--dump-outputs: what the last timed step returned, one float64 .npy per array: T (n, 6), the top
+    two rows of each 3x3 transform; error (n,); passes (n,); rows (n,), each row's index in the step's
+    problem list.  The inputs are seeded, so two builds run with the same arguments can be compared file
+    by file.  Past 64 MB, a seeded sample of the rows (the same rows on every run)."""
+    rows = np.asarray(rows)
+    keep = (DUMP_BYTES - 4096) // (9 * 8)                     # 9 float64 per row; 4096: the .npy headers
+    sel = np.arange(len(rows))
+    if len(rows) > keep:
+        sel = np.sort(np.random.default_rng(SEED).choice(len(rows), keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("T", T6), ("error", err), ("passes", passes), ("rows", rows)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(np.asarray(a)[sel], dtype=np.float64))
+
+
 def cpu_port_rate(scans, pairs, init, seconds, threads=0, all_pairs=False):
     """Time the C port of the reference algorithm on a bounded sample of the same workload."""
     from oracle import c_oracle
@@ -296,8 +317,11 @@ def run_reference(args, rank, world):
         c_oracle.icp_batch(xy, off, pairs[sel], init[sel], epsilon=EPS, max_iters=MAX_ITERS, n_threads=nthr)
     t = time.perf_counter()
     for _ in range(args.steps):
-        c_oracle.icp_batch(xy, off, pairs[sel], init[sel], epsilon=EPS, max_iters=MAX_ITERS, n_threads=nthr)
+        T, err, passes = c_oracle.icp_batch(xy, off, pairs[sel], init[sel], epsilon=EPS, max_iters=MAX_ITERS,
+                                            n_threads=nthr)
     dt = time.perf_counter() - t
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sel, c_oracle.to6(T), err, passes)
     rate = n * args.steps / dt
     sample = (f"{n} of {len(pairs)} pairs per step" + ("" if n == len(pairs) else ", seeded random subsample") +
               f", C port oracle/icp_oracle.c on {nthr} threads")
@@ -314,6 +338,7 @@ def run_reference(args, rank, world):
 
 
 def main():
+    sys.dont_write_bytecode = True                           # the tree may be read-only: no __pycache__ in it
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -437,6 +462,13 @@ def main():
         ev[k][1].record()
     barrier()
     t_wall1 = time.time()
+    if args.dump_outputs and rank == 0:                      # before any later launch rewrites the outputs
+        if gather is not None and not args.exhaustive:        # every rank's records, as every rank holds them
+            rec = gather.records().cpu().numpy()
+            dump_outputs(args.dump_outputs, np.arange(n_global), rec[:, :6], rec[:, 6], rec[:, 7])
+        else:
+            dump_outputs(args.dump_outputs, mine, out_T.cpu().numpy(), out_err.cpu().numpy(),
+                         out_pass.cpu().numpy())
     launches = eng.launch_count - launches0
     step_ms = np.array([e[0].elapsed_time(e[1]) for e in ev])
     total_ms = torch.tensor([step_ms.sum()], dtype=torch.float64, device=dev)

@@ -110,6 +110,34 @@ def test_config5_highres_multistart():
     assert abs(th[best]) < 1.0                                   # the sweep finds the small-motion basin
 
 
+def test_bench_dump_outputs_device_arm(tmp_path):
+    """`bench.py --dump-outputs DIR` on the device: the last timed step's transforms, errors and pass
+    counts for every pair of the seeded chain, as the C oracle computes them."""
+    import argparse
+    import os
+    import subprocess
+    import sys
+    from oracle import c_oracle
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+                          "--scans", "120", "--beams", "360", "--no-cpu", "--no-e2e", "--no-sustained",
+                          "--no-exhaustive", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-3000:]
+    z = {n: np.load(tmp_path / f"{n}.npy") for n in ("T", "error", "passes", "rows")}
+    assert all(a.dtype == np.float64 for a in z.values())
+    assert z["T"].shape == (119, 6) and z["rows"].tolist() == list(range(119))
+    args = argparse.Namespace(workload="chain", scans=120, beams=360, strong=False, pairs=0)
+    scans, pairs, init = bench.workload(args, 0, 1)
+    xy, off = c_oracle.pack(scans)
+    T, err, passes = c_oracle.icp_batch(xy, off, pairs, init, epsilon=bench.EPS, max_iters=bench.MAX_ITERS)
+    np.testing.assert_array_equal(z["passes"], passes)
+    dt, dth = pose_diff(c_oracle.to33(z["T"]), T)
+    assert dt < 1e-9 and dth < 1e-9
+    np.testing.assert_allclose(z["error"], err, rtol=1e-9)
+
+
 def test_parity_campaign_reduced():
     """tools/parity_campaign.py at 4 % of its size (chains, rotation-only, all pairs, ragged clouds
     incl. tie-laden lattices and far-from-origin coordinates): no pass-count mismatch, no differing

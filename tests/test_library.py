@@ -119,6 +119,56 @@ def test_bench_reference_arm_contract():
     assert "workload" in d["config"]
 
 
+def test_bench_dump_outputs_reference_arm(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the last timed step's results as float64 .npy files; the
+    inputs are seeded, so runs with different step counts write the same arrays, and they are what the
+    C port returns for the same pairs."""
+    import argparse
+    import subprocess
+    import sys
+    from oracle import c_oracle
+    sys.path.insert(0, ROOT)
+    import bench
+    dirs = []
+    for steps in (1, 2):
+        d = tmp_path / f"s{steps}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps",
+                              str(steps), "--warmup", "0", "--scans", "30", "--beams", "128", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=300)
+        assert out.returncode == 0, out.stderr[-2000:]
+        dirs.append(d)
+    z = [{n: np.load(d / f"{n}.npy") for n in ("T", "error", "passes", "rows")} for d in dirs]
+    for n in z[0]:
+        assert z[0][n].dtype == np.float64
+        np.testing.assert_array_equal(z[0][n], z[1][n])
+    assert z[0]["T"].shape == (29, 6) and z[0]["rows"].tolist() == list(range(29))
+    args = argparse.Namespace(workload="chain", scans=30, beams=128, strong=False, pairs=0)
+    scans, pairs, init = bench.workload(args, 0, 1)
+    xy, off = c_oracle.pack(scans)
+    T, err, passes = c_oracle.icp_batch(xy, off, pairs, init, epsilon=bench.EPS, max_iters=bench.MAX_ITERS)
+    np.testing.assert_array_equal(z[0]["T"], c_oracle.to6(T))
+    np.testing.assert_array_equal(z[0]["error"], err)
+    np.testing.assert_array_equal(z[0]["passes"], passes)
+
+
+def test_bench_dump_outputs_samples_past_the_cap(tmp_path, monkeypatch):
+    """Past the size cap, --dump-outputs keeps a sorted seeded sample of the rows, the same on every call."""
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 72 * 100)
+    n = 1000
+    T6 = np.arange(6 * n, dtype=np.float64).reshape(n, 6)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), np.arange(n), T6, np.arange(n) * 0.5, np.arange(n, dtype=np.int32))
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert len(rows) == 100 and np.all(np.diff(rows) > 0)
+    np.testing.assert_array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "T.npy"), T6[rows.astype(np.int64)])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "passes.npy"), rows)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= bench.DUMP_BYTES
+
+
 def test_upload_plan_pieces_end_on_sector_boundaries():
     """icpb_plan_upload (the host logic that cuts the scan table for the streaming upload): pieces
     are contiguous, cover every scan, and every interior boundary sits on an even point offset (a
