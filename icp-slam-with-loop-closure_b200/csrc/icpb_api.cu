@@ -124,6 +124,8 @@ struct LaunchCfg {
     int threads, smem, ctas_per_sm;
     icpb::SmemLayout L;
     int cluster;   // CTAs per problem (1 = ordinary launch)
+    bool big;      // large-scan variant: the arrays before L.o_tw live in per-CTA device scratch
+    int64_t big_stride;   // bytes of one CTA's scratch region
 };
 
 typedef void (*kernel_fn)(const icpb::KernelArgs);
@@ -139,6 +141,16 @@ kernel_fn pick_kernel(const icpb_params *p)
                             : icpb::icp_align_kernel<kPointsPerThread, true, false>;
 }
 kernel_fn cluster_kernel() { return icpb::icp_align_kernel<kPointsPerThread, true, true>; }
+// the large-scan variants (KernelArgs::big_scratch): same code, arrays in device scratch
+kernel_fn big_kernel(const icpb_params *p)
+{
+    return is_exhaustive(p) ? icpb::icp_align_kernel<kPointsExhaustive, false, false, true>
+                            : icpb::icp_align_kernel<kPointsPerThread, true, false, true>;
+}
+kernel_fn big_cluster_kernel() { return icpb::icp_align_kernel<kPointsPerThread, true, true, true>; }
+// Scratch of the large-scan variant: one region per resident CTA, the grid capped so that all regions
+// together stay within this budget (a 100,000-point scan needs ~1.7 MB per CTA: ~600 CTAs).
+constexpr int64_t kBigScratchBudget = int64_t(1) << 30;
 
 }  // namespace
 
@@ -309,6 +321,8 @@ struct icpb_ctx {
     DevBuf s_sgd;                                   // pose-graph SGD: poses, edges, transforms, scratch
     DevBuf s_grid;                                  // occupancy grid: poses, per-cell words, the grid
     DevBuf s_accept;                                // acceptance epilogue: [appended, CTAs left] counters
+    DevBuf s_big;                                   // large-scan variant: one scratch region per CTA
+    DevBuf s_order;                                 // queue order of a batch split by scan length
     // per-scan staging images of the resident table (KernelArgs::prep_in), built on first use
     DevBuf prep;
     const double *prep_for = nullptr;               // the table (h->xy) the images were built from
@@ -316,15 +330,18 @@ struct icpb_ctx {
     PinnedBuf stage_xy;                             // pinned copy of a scan table packed from a list of arrays
     PackPool *pool = nullptr;                       // host threads that pack scans into stage_xy
     // tuning / test hooks (icpb_set_tuning); 0 or -1 = the library's own choice
-    int tune_threads = 0, tune_cluster = -1, tune_segments = 0, tune_pack_threads = 0;
+    int tune_threads = 0, tune_cluster = -1, tune_segments = 0, tune_pack_threads = 0, tune_large = -1;
     bool tune_flag_copy = false, tune_drop_counter = false, tune_trace = false;
 };
 
 namespace {
 
-int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, kernel_fn fn, int R = kPointsPerThread)
+// Launch geometry for a batch whose longest scan has `longest` points.  When the layout does not fit
+// one CTA's shared memory (or `big` asks for it) the launch uses the large-scan variant.
+int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, const icpb_params *p, bool big = false)
 {
     if (longest <= 0) return fail(ICPB_EINVAL, "empty scan table%s");
+    const int R = points_per_thread(p);
     const int64_t ntile = (longest + 63) / 64;              // 64-point reduction tiles (independent of R)
     const int64_t nwork = (ntile + R / 2 - 1) / (R / 2);    // warp work items of 32*R points
     // Warps per CTA.  Small CTAs keep more independent problems in flight per SM (less idling at the
@@ -346,13 +363,17 @@ int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, kernel_fn fn
     }
     int threads = warps * 32;
     const icpb::SmemLayout L = icpb::smem_layout(longest, threads / 32);
-    const int64_t smem = L.bytes;
-    if (smem > h->smem_limit) {
-        snprintf(g_err, sizeof g_err, "scan of %lld points needs %lld B of shared memory (limit %d)",
-                 (long long)longest, (long long)smem, h->smem_limit);
+    if (L.bytes == 0x7fffffff) {
+        snprintf(g_err, sizeof g_err, "scan of %lld points is beyond the kernel's 32-bit layout offsets",
+                 (long long)longest);
         return ICPB_ETOOLONG;
     }
-    c->threads = threads; c->smem = (int)smem; c->L = L;
+    if (L.bytes > h->smem_limit) big = true;
+    const kernel_fn fn = big ? big_kernel(p) : pick_kernel(p);
+    // large-scan variant: Tw, S0 and the transpose scratch stay in shared memory, at offsets from 0
+    const int64_t smem = big ? L.bytes - L.o_tw : L.bytes;
+    c->threads = threads; c->smem = (int)smem; c->L = L; c->big = big;
+    c->big_stride = big ? ((int64_t)L.o_tw + 255) & ~int64_t(255) : 0;
     // Latency mode: when every CTA of every cluster can have an SM of its own and a CTA's eight warps
     // would each get more than one tile per pass, spread each problem over a thread-block cluster (a
     // power of two, at most 8 CTAs) so that every tile has a warp.  Measured with one cluster per
@@ -361,7 +382,7 @@ int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, kernel_fn fn
     // two, 80 pairs 0.41 -> 0.38; from 120 pairs on (more CTAs than SMs) single CTAs win; one 4,096-point
     // pair 0.78 -> 0.41 ms in a cluster of eight.
     c->cluster = 1;
-    if (fn == pick_kernel(nullptr) && nwork > 8) {
+    if (!is_exhaustive(p) && nwork > 8) {
         int cl = 2;
         while (cl < 8 && (int64_t)cl * 8 < nwork) cl *= 2;
         while (cl > 1 && B * cl > h->sm_count) cl /= 2;
@@ -370,7 +391,7 @@ int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, kernel_fn fn
     if (h->tune_cluster >= 0) {                           // icpb_set_tuning("cluster"): force a size (0 = never)
         const int v = h->tune_cluster;
         if (v == 0 || v == 1) c->cluster = 1;
-        else if ((v == 2 || v == 4 || v == 8) && fn == pick_kernel(nullptr)) c->cluster = v;
+        else if ((v == 2 || v == 4 || v == 8) && !is_exhaustive(p)) c->cluster = v;
     }
     // (the kernels' dynamic shared-memory limit is raised to the device maximum once, in icpb_create: the
     // attribute belongs to the function, not to a handle, so it must not follow one handle's history)
@@ -379,6 +400,14 @@ int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, kernel_fn fn
     if (per_sm < 1) return fail(ICPB_EINVAL, "kernel does not fit on an SM%s");
     c->ctas_per_sm = per_sm;
     return 0;
+}
+
+// A pair fits the shared-memory kernel when the layout of its longer scan fits at the widest CTA a
+// launch may pick (8 warps), so that it fits whatever width the launch settles on.
+bool fits_smem(const icpb_ctx *h, int64_t n)
+{
+    const icpb::SmemLayout L = icpb::smem_layout(n, 8);
+    return L.bytes != 0x7fffffff && L.bytes <= h->smem_limit;
 }
 
 int check_params(const icpb_params *p, int64_t B)
@@ -413,20 +442,29 @@ int check_epilogue(const icpb_epilogue *ep, const icpb_params *p)
 
 int ensure_prep(icpb_ctx *h, cudaStream_t stream);
 
+// One of the (at most two) launches of a batch split by scan length (launch_split).
+struct LaunchPart {
+    int64_t B_all;            // pairs of the whole batch: epilogue rows are pair ids of it
+    bool big;                 // the large-scan variant
+    bool accept_continue;     // the acceptance count goes on from the previous launch of the batch
+};
+
 int launch(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scans, int64_t longest,
            const int32_t *d_pairs, const double *d_init, int64_t B, const icpb_params *p,
            double *d_T, double *d_err, int32_t *d_passes, double *d_hist, int32_t *d_corr,
            cudaStream_t stream, int64_t B_total = 0, const int32_t *d_seg_of_pair = nullptr,
            const int32_t *d_arrived = nullptr, const icpb_epilogue *ep = nullptr,
            const int32_t *d_order = nullptr, int32_t *d_upload_timeout = nullptr,
-           unsigned char *prep_out = nullptr, int64_t prep_stride_out = 0)
+           unsigned char *prep_out = nullptr, int64_t prep_stride_out = 0, const LaunchPart *part = nullptr)
 {
     const bool prep_building = prep_out != nullptr;
     if (B == 0) return 0;
     LaunchCfg cfg;
-    kernel_fn fn = pick_kernel(p);
-    int rc = make_cfg(h, longest, B_total > B ? B_total : B, &cfg, fn, points_per_thread(p));
+    const bool force_big = part ? part->big : (h->tune_large == 1 && !prep_building);
+    int rc = make_cfg(h, longest, B_total > B ? B_total : B, &cfg, p, force_big);
     if (rc) return rc;
+    const kernel_fn fn = cfg.big ? big_kernel(p) : pick_kernel(p);
+    const kernel_fn cfn = cfg.big ? big_cluster_kernel() : cluster_kernel();
     icpb::KernelArgs a;
     a.xy = xy; a.offsets = offsets; a.pairs = d_pairs; a.init = d_init; a.B = B; a.n_scans = n_scans;
     a.p = *p;
@@ -437,17 +475,19 @@ int launch(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scan
     a.n2pad_cap = cfg.L.n2pad; a.n1_cap = cfg.L.n1c; a.nchunk_cap = cfg.L.nchunk; a.ntile_cap = cfg.L.ntile;
     a.o_tqy = cfg.L.o_tqy; a.o_cb = cfg.L.o_cb; a.o_tc = cfg.L.o_tc; a.o_mm = cfg.L.o_mm; a.o_corr = cfg.L.o_corr;
     a.o_red = cfg.L.o_red; a.o_tw = cfg.L.o_tw; a.o_s0 = cfg.L.o_s0; a.o_scr = cfg.L.o_scr;
+    a.big_scratch = nullptr; a.big_stride = 0;
+    if (cfg.big) { a.o_tw = 0; a.o_s0 = cfg.L.o_s0 - cfg.L.o_tw; a.o_scr = cfg.L.o_scr - cfg.L.o_tw; }
     a.executed = h->executed;
     a.seg_of_pair = d_seg_of_pair; a.arrived = d_arrived; a.order = d_order; a.upload_timeout = d_upload_timeout;
     a.prep_out = nullptr; a.prep_in = nullptr; a.prep_stride = 0;
-    if (d_arrived == nullptr && xy == h->xy && h->xy != nullptr && !prep_building) {
+    if (d_arrived == nullptr && xy == h->xy && h->xy != nullptr && !prep_building && longest == h->longest) {
         // a resident table: stage every pair by copy from the per-scan images (built once per table)
         int rc2 = ensure_prep(h, stream);
         if (rc2) return rc2;
         if (h->prep_for == h->xy) { a.prep_in = (const unsigned char *)h->prep.p; a.prep_stride = h->prep_stride; }
     }
     if (prep_out) { a.prep_out = prep_out; a.prep_stride = prep_stride_out; }
-    a.peers = nullptr; a.n_peers = 0; a.rec_row0 = 0; a.rec_block = B > 0 ? B : 1; a.rec_stride = 0;
+    a.peers = nullptr; a.n_peers = 0; a.rec_row0 = 0; a.rec_block = part ? part->B_all : B; a.rec_stride = 0;
     a.accept_thresh = 0.0; a.accept_rec = nullptr; a.accept_peers = nullptr; a.accept_ctr = nullptr;
     a.accept_count_out = nullptr; a.accept_count_peers = nullptr; a.accept_cap = 0; a.accept_rank = 0;
     if (ep) {
@@ -463,12 +503,31 @@ int launch(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scan
             a.accept_count_peers = (long long *const *)ep->d_accept_count_peer_ptrs;
             a.accept_count_out = (long long *)ep->d_accept_count;
             a.accept_ctr = (unsigned long long *)h->s_accept.p;
-            CU(cudaMemsetAsync(a.accept_ctr, 0, 2 * sizeof(unsigned long long), stream));
+            // [0] rows appended: zeroed by the first launch of a batch only; [1] CTAs that have left: per launch
+            const bool cont = part && part->accept_continue;
+            CU(cudaMemsetAsync(a.accept_ctr + (cont ? 1 : 0), 0, (cont ? 1 : 2) * sizeof(unsigned long long), stream));
         }
     }
     CU(cudaMemsetAsync(a.queue, 0, sizeof(unsigned long long), stream));
     int64_t grid = (int64_t)cfg.ctas_per_sm * h->sm_count;
     if (grid > B) grid = B;
+    int64_t max_ctas = grid * cfg.cluster;                    // CTAs the launch may have
+    if (cfg.big) {
+        // one scratch region per CTA, within kBigScratchBudget; with less device memory free, fewer
+        // CTAs, down to one cluster (or CTA) -- only if that cannot be had does the call fail
+        int64_t cap = kBigScratchBudget / cfg.big_stride / cfg.cluster * cfg.cluster;
+        if (cap < cfg.cluster) cap = cfg.cluster;
+        if (max_ctas > cap) max_ctas = cap;
+        for (;;) {
+            const int rc2 = h->s_big.reserve((size_t)(max_ctas * cfg.big_stride));
+            if (rc2 == 0) break;
+            cudaGetLastError();
+            if (max_ctas <= cfg.cluster) return rc2;          // g_err names the allocation that failed
+            max_ctas = (max_ctas / 2 + cfg.cluster - 1) / cfg.cluster * cfg.cluster;
+        }
+        a.big_scratch = (unsigned char *)h->s_big.p; a.big_stride = cfg.big_stride;
+        if (grid > max_ctas) grid = max_ctas;
+    }
     if (cfg.cluster > 1) {
         cudaLaunchConfig_t lc = {};
         cudaLaunchAttribute attr[1];
@@ -480,11 +539,12 @@ int launch(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scan
         // grid that is a multiple of the cluster size; it answers in clusters)
         lc.gridDim = dim3((unsigned)cfg.cluster);
         int max_clusters = 0;
-        CU(cudaOccupancyMaxActiveClusters(&max_clusters, cluster_kernel(), &lc));
+        CU(cudaOccupancyMaxActiveClusters(&max_clusters, cfn, &lc));
         int64_t clusters = max_clusters > 0 ? max_clusters : 1;
         if (clusters > B) clusters = B;
+        if (clusters > max_ctas / cfg.cluster) clusters = max_ctas / cfg.cluster;
         lc.gridDim = dim3((unsigned)(clusters * cfg.cluster));
-        CU(cudaLaunchKernelEx(&lc, cluster_kernel(), a));
+        CU(cudaLaunchKernelEx(&lc, cfn, a));
     } else {
         fn<<<(unsigned)grid, cfg.threads, cfg.smem, stream>>>(a);
     }
@@ -498,7 +558,9 @@ int launch(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scan
 // alignment kernel in prep mode the first time the table is used.  A pair's staging is then a 10 KB copy
 // instead of ~11,000 warp instructions; scans that take part in many pairs (loop-closure candidates, all
 // pairs) are prepared once instead of once per pair.  Tables whose images would exceed 8 GB are staged
-// per pair as before.
+// per pair as before.  So are tables whose longest scan does not fit shared memory (the images are laid
+// out for the table's longest scan, and a launch reads them at its own layout's offsets: the short pairs
+// of such a table run at a smaller layout, its long pairs stage into scratch per pair).
 int ensure_prep(icpb_ctx *h, cudaStream_t stream)
 {
     if (h->prep_for == h->xy && h->prep_scans == h->n_scans && h->prep_longest == h->longest) return 0;
@@ -507,16 +569,78 @@ int ensure_prep(icpb_ctx *h, cudaStream_t stream)
     const int64_t stride = ((int64_t)L.o_mm + 32 + 15) & ~int64_t(15);
     if (stride * h->n_scans > (int64_t(8) << 30)) return 0;
     int rc;
-    if ((rc = h->prep.reserve((size_t)(stride * h->n_scans)))) return rc;
     icpb_params p;
     icpb_default_params(&p);
     p.k_block = h->n_scans;
+    LaunchCfg cfg;
+    if ((rc = make_cfg(h, h->longest, h->n_scans, &cfg, &p))) return rc;
+    if (cfg.big) return 0;
+    if ((rc = h->prep.reserve((size_t)(stride * h->n_scans)))) return rc;
     rc = launch(h, h->xy, h->offsets, h->n_scans, h->longest, nullptr, nullptr, h->n_scans, &p,
                 nullptr, nullptr, nullptr, nullptr, nullptr, stream, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
                 (unsigned char *)h->prep.p, stride);
     if (rc) return rc;
     h->prep_for = h->xy; h->prep_stride = stride; h->prep_scans = h->n_scans; h->prep_longest = h->longest;
     return 0;
+}
+
+// A batch whose longest scan does not fit shared memory, on an entry point that sees the pairs, runs as
+// two launches: the pairs that fit (fits_smem of the longer scan) on the shared-memory kernel at the
+// layout of the longest scan among them, then the others on the large-scan variant.  Both write the
+// outputs by pair id; the queue holds the first part's pairs, then the second's, each in its original
+// order.  The two variants give the same bits, so the split decides speed only.
+struct Split {
+    int64_t ns = 0;            // pairs in the first part
+    int64_t Ls = 0, Ll = 0;    // longest scan of each part
+};
+
+// Whether a batch has to be split: its longest scan does not fit and "large" does not force the variant.
+bool needs_split(icpb_ctx *h, int64_t longest, int64_t B, const icpb_params *p)
+{
+    if (h->tune_large == 1 || B < 1 || p->pair_mode != 0) return false;
+    LaunchCfg cfg;
+    return make_cfg(h, longest, B, &cfg, p) == 0 && cfg.big;
+}
+
+// order[q] (queue position q -> pair id) for the split; queue: the queue before it (nullptr: identity).
+// seg (by queue position, optional) is permuted along.
+Split split_queue(const icpb_ctx *h, const int64_t *off, const int32_t *pairs, int64_t B, const int32_t *queue,
+                  int32_t *order, int32_t *seg)
+{
+    Split sp;
+    std::vector<int32_t> lo, hi, slo, shi;
+    for (int64_t q = 0; q < B; ++q) {
+        const int32_t b = queue ? queue[q] : (int32_t)q;
+        const int64_t n1 = off[pairs[2 * b] + 1] - off[pairs[2 * b]], n2 = off[pairs[2 * b + 1] + 1] - off[pairs[2 * b + 1]];
+        const int64_t n = n1 > n2 ? n1 : n2;
+        const bool fit = fits_smem(h, n);
+        (fit ? lo : hi).push_back(b);
+        if (seg) (fit ? slo : shi).push_back(seg[q]);
+        int64_t &L = fit ? sp.Ls : sp.Ll;
+        if (n > L) L = n;
+    }
+    sp.ns = (int64_t)lo.size();
+    std::copy(lo.begin(), lo.end(), order);
+    std::copy(hi.begin(), hi.end(), order + sp.ns);
+    if (seg) { std::copy(slo.begin(), slo.end(), seg); std::copy(shi.begin(), shi.end(), seg + sp.ns); }
+    return sp;
+}
+
+int launch_split(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scans, const Split &sp,
+                 const int32_t *d_pairs, const double *d_init, int64_t B, const icpb_params *p,
+                 double *d_T, double *d_err, int32_t *d_passes, double *d_hist, int32_t *d_corr,
+                 cudaStream_t stream, const int32_t *d_seg, const int32_t *d_arrived, const icpb_epilogue *ep,
+                 const int32_t *d_order, int32_t *d_upload_timeout)
+{
+    LaunchPart part = {B, false, false};
+    int rc = launch(h, xy, offsets, n_scans, sp.Ls, d_pairs, d_init, sp.ns, p, d_T, d_err, d_passes, d_hist, d_corr,
+                    stream, 0, d_seg, d_arrived, ep, d_order, d_upload_timeout, nullptr, 0, &part);
+    if (rc) return rc;
+    part.big = true;
+    part.accept_continue = sp.ns > 0;
+    return launch(h, xy, offsets, n_scans, sp.Ll, d_pairs, d_init, B - sp.ns, p, d_T, d_err, d_passes, d_hist, d_corr,
+                  stream, 0, d_seg ? d_seg + sp.ns : nullptr, d_arrived, ep, d_order + sp.ns, d_upload_timeout,
+                  nullptr, 0, &part);
 }
 
 }  // namespace
@@ -574,6 +698,15 @@ int icpb_create(int device, icpb_handle *out)
         e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
         if (lim < h->smem_limit) h->smem_limit = lim;
     }
+    // the large-scan variants keep only a few KB in shared memory, but ask for the same maximum
+    for (kernel_fn fn : {big_kernel(nullptr), big_cluster_kernel(),
+                         (kernel_fn)icpb::icp_align_kernel<kPointsExhaustive, false, false, true>}) {
+        cudaFuncAttributes fa;
+        if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, fn);
+        if (e != cudaSuccess) break;
+        e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)prop.sharedMemPerBlockOptin - (int)fa.sharedSizeBytes);
+    }
     if (e == cudaSuccess) e = cudaMalloc(&h->arrived_dev, sizeof(int32_t));
     if (e == cudaSuccess) e = cudaHostAlloc(&h->seg_vals_pinned, sizeof(int32_t) * (kMaxSegments + 1), cudaHostAllocDefault);
     if (e == cudaSuccess) for (int k = 0; k <= kMaxSegments; ++k) h->seg_vals_pinned[k] = k;
@@ -601,6 +734,7 @@ int icpb_set_tuning(icpb_handle h, const char *key, int64_t value)
     const int v = (int)value;
     if (!strcmp(key, "threads")) h->tune_threads = v;
     else if (!strcmp(key, "cluster")) h->tune_cluster = v;
+    else if (!strcmp(key, "large")) h->tune_large = v;
     else if (!strcmp(key, "segments")) h->tune_segments = v;
     else if (!strcmp(key, "pack_threads")) {
         if (h->pool && (int)h->pool->workers.size() != v - 1) { delete h->pool; h->pool = nullptr; }
@@ -626,7 +760,7 @@ int icpb_destroy(icpb_handle h)
     if (h->arrived_dev) cudaFree(h->arrived_dev);
     if (h->seg_vals_pinned) cudaFreeHost(h->seg_vals_pinned);
     h->s_seg.release(); h->stage.release(); h->s_sgd.release(); h->s_grid.release();
-    h->s_accept.release(); h->stage_xy.release(); h->prep.release();
+    h->s_accept.release(); h->stage_xy.release(); h->prep.release(); h->s_big.release(); h->s_order.release();
     h->own_xy.release(); h->own_off.release();
     h->s_pairs.release(); h->s_init.release(); h->s_T.release(); h->s_err.release();
     h->s_passes.release(); h->s_hist.release(); h->s_corr.release();
@@ -749,6 +883,20 @@ static int run_host_common(icpb_handle h, const double *xy, const int64_t *offse
     if ((rc = h->s_passes.reserve(sizeof(int32_t) * (size_t)B))) return rc;
     if (nbH) { if ((rc = h->s_hist.reserve(nbH))) return rc; CU(cudaMemsetAsync(h->s_hist.p, 0, nbH, st)); }
     if (nbC) { if ((rc = h->s_corr.reserve(nbC))) return rc; CU(cudaMemsetAsync(h->s_corr.p, 0xff, nbC, st)); }
+    if (needs_split(h, longest, B, p)) {
+        std::vector<int64_t> off((size_t)n_scans + 1);
+        std::vector<int32_t> order((size_t)B);
+        CU(cudaMemcpyAsync(off.data(), offsets, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        const Split sp = split_queue(h, off.data(), h_pairs, B, nullptr, order.data(), nullptr);
+        if ((rc = h->s_order.reserve(sizeof(int32_t) * (size_t)B))) return rc;
+        CU(cudaMemcpyAsync(h->s_order.p, order.data(), sizeof(int32_t) * (size_t)B, cudaMemcpyHostToDevice, st));
+        rc = launch_split(h, xy, offsets, n_scans, sp, (const int32_t *)h->s_pairs.p,
+                          h_init ? (const double *)h->s_init.p : nullptr, B, p,
+                          (double *)h->s_T.p, (double *)h->s_err.p, (int32_t *)h->s_passes.p,
+                          (double *)h->s_hist.p, (int32_t *)h->s_corr.p, st, nullptr, nullptr, nullptr,
+                          (const int32_t *)h->s_order.p, nullptr);
+    } else
     rc = launch(h, xy, offsets, n_scans, longest,
                 p->pair_mode == 0 ? (const int32_t *)h->s_pairs.p : nullptr,
                 h_init ? (const double *)h->s_init.p : nullptr, B, p,
@@ -1077,6 +1225,16 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
             }
         }
     }
+    // a table whose longest scan does not fit shared memory: the queue is split by scan length, each part
+    // keeping its arrival order (launch_split)
+    Split sp;
+    const bool split = needs_split(h, longest, B, p);
+    if (split) {
+        std::vector<int32_t> queue(in_order ? 0 : (size_t)B);
+        if (!in_order) memcpy(queue.data(), porder, nb4);
+        sp = split_queue(h, h_offsets, h_pairs, B, in_order ? nullptr : queue.data(), porder, pseg);
+        in_order = false;
+    }
     memcpy(ppairs, h_pairs, 2 * nb4);
     if (h_init) {
         if (init_ld == 6) {
@@ -1096,6 +1254,10 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     // ONE launch over all pairs, in arrival order; its CTAs wait on the segment counter
     CUP(cudaStreamWaitEvent(cs, h->seg_ev[0], 0));
     CUP(cudaStreamWaitEvent(cs, h->seg_ev[1], 0));
+    if (split)
+        rc = launch_split(h, d_xy, d_off, n_scans, sp, d_pairs, h_init ? d_init : nullptr, B, p, d_T, d_err, d_passes,
+                          nullptr, nullptr, cs, d_seg, h->arrived_dev, ep, d_order, d_passes + B);
+    else
     rc = launch(h, d_xy, d_off, n_scans, longest, d_pairs, h_init ? d_init : nullptr, B, p,
                 d_T, d_err, d_passes, nullptr, nullptr, cs, B, d_seg, h->arrived_dev, ep,
                 in_order ? nullptr : d_order, d_passes + B);
@@ -1145,6 +1307,10 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     if (tP[B] != 0) {
         // a CTA gave up waiting for its scans (see the kernel): by now the whole table is resident,
         // so run the batch again without the streaming protocol
+        if (split)
+            rc = launch_split(h, d_xy, d_off, n_scans, sp, d_pairs, h_init ? d_init : nullptr, B, p, d_T, d_err,
+                              d_passes, nullptr, nullptr, cp, nullptr, nullptr, ep, d_order, nullptr);
+        else
         rc = launch(h, d_xy, d_off, n_scans, longest, d_pairs, h_init ? d_init : nullptr, B, p,
                     d_T, d_err, d_passes, nullptr, nullptr, cp, 0, nullptr, nullptr, ep);
         if (rc) return align_abort(h, rc);
@@ -1670,9 +1836,9 @@ int icpb_get_kernel_info(icpb_handle h, int64_t B, icpb_kernel_info *out)
     if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
     ON_DEVICE(h);
     LaunchCfg cfg;
-    kernel_fn fn = pick_kernel(nullptr);
-    int rc = make_cfg(h, h->longest, B > 0 ? B : (int64_t)1 << 40, &cfg, fn);
+    int rc = make_cfg(h, h->longest, B > 0 ? B : (int64_t)1 << 40, &cfg, nullptr, h->tune_large == 1);
     if (rc) return rc;
+    const kernel_fn fn = cfg.big ? big_kernel(nullptr) : pick_kernel(nullptr);
     cudaFuncAttributes fa;
     CU(cudaFuncGetAttributes(&fa, fn));
     int64_t grid = (int64_t)cfg.ctas_per_sm * h->sm_count;

@@ -145,6 +145,12 @@ struct KernelArgs {
     unsigned char       *prep_out;   // != nullptr: problem b is scan b (source = target = b); build its record, no ICP
     const unsigned char *prep_in;
     int64_t              prep_stride;
+    // Large-scan variant (BIG): the arrays that SmemLayout places before o_tw (target SoA, chunk and group
+    // circles, mm, correspondences, red) live in a per-CTA region of device scratch, CTA k's at
+    // big_scratch + k * big_stride, at the same byte offsets; o_tw, o_s0 and o_scr are offsets into the
+    // small dynamic shared memory that is left (Tw, S0, transpose scratch).
+    unsigned char       *big_scratch;
+    int64_t              big_stride;
 };
 
 // ---- fp32 filter distance: one definition, used by the sweep and by the refine step ----------
@@ -292,12 +298,13 @@ __device__ __noinline__ int exact_decide_chunk(int j0, unsigned cand, double Px,
 // point may hold a candidate (chunks ascend, so the first-index rule still holds across chunks)
 // (the shared arrays are addressed by their byte offsets: a generic pointer argument would make the
 // caller form -- and keep rematerialising -- 64-bit generic addresses of shared memory)
-__device__ __noinline__ int exact_decide_all(int nchunks, int n2, int fallback, float thr, float px, float py,
-                                             double Px, double Py, int o_tqy, int o_cb, const double2 *dst)
+__device__ __forceinline__ int exact_decide_all_from(const unsigned char *base, int nchunks, int n2, int fallback,
+                                                     float thr, float px, float py, double Px, double Py,
+                                                     int o_tqy, int o_cb, const double2 *dst)
 {
-    const float *tqx = reinterpret_cast<const float *>(smem_raw);
-    const float *tqy = reinterpret_cast<const float *>(smem_raw + o_tqy);
-    const float4 *cb = reinterpret_cast<const float4 *>(smem_raw + o_cb);
+    const float *tqx = reinterpret_cast<const float *>(base);
+    const float *tqy = reinterpret_cast<const float *>(base + o_tqy);
+    const float4 *cb = reinterpret_cast<const float4 *>(base + o_cb);
     double best = __longlong_as_double(0x7ff0000000000000LL);
     int idx = fallback;
     const float s = sqrt_fast(thr) * 1.0001f + 1e-30f;
@@ -308,6 +315,18 @@ __device__ __noinline__ int exact_decide_all(int nchunks, int n2, int fallback, 
             exact_range(c * kChunk, min(c * kChunk + kChunk, n2), thr, px, py, Px, Py, tqx, tqy, dst, best, idx);
     }
     return idx;
+}
+__device__ __noinline__ int exact_decide_all(int nchunks, int n2, int fallback, float thr, float px, float py,
+                                             double Px, double Py, int o_tqy, int o_cb, const double2 *dst)
+{
+    return exact_decide_all_from(smem_raw, nchunks, n2, fallback, thr, px, py, Px, Py, o_tqy, o_cb, dst);
+}
+// the same decision on arrays in device memory (large-scan variant): base = the CTA's scratch region
+__device__ __noinline__ int exact_decide_all_at(const unsigned char *base, int nchunks, int n2, int fallback, float thr,
+                                                float px, float py, double Px, double Py, int o_tqy, int o_cb,
+                                                const double2 *dst)
+{
+    return exact_decide_all_from(base, nchunks, n2, fallback, thr, px, py, Px, Py, o_tqy, o_cb, dst);
 }
 
 __device__ __forceinline__ double warp_sum(double v)
@@ -424,23 +443,36 @@ __device__ __forceinline__ double stretch_of(const double *T)
 // (tile t belongs to CTA t mod cluster size); the per-tile partial sums stay in their owner's
 // shared memory and every CTA folds them over distributed shared memory after the pass's
 // cluster barrier -- in the same tile order as the single-CTA kernel, so the two give the same bits.
-template <int R, bool PRUNE, bool CLUSTER>
+//
+// BIG = true (scans whose layout exceeds one CTA's shared memory): the same kernel with every per-point
+// and per-tile array in the CTA's region of device scratch (KernelArgs::big_scratch) instead of shared
+// memory; only Tw, S0 and the transpose scratch stay on chip.  The decision, the reduction order, the
+// fit and the stop rules are this code, so both variants give the same bits.  Chunk loads come from
+// L1/L2, so a group's next chunk is loaded while the current one is swept.  In latency mode the partial
+// sums and match ranges are read from the owning CTA's scratch (through L2) after the cluster barrier.
+template <int R, bool PRUNE, bool CLUSTER, bool BIG = false>
 #ifndef ICPB_MIN_CTAS
 #define ICPB_MIN_CTAS 3
 #endif
 #ifndef ICPB_EXH_CTAS
 #define ICPB_EXH_CTAS 2
 #endif
-__global__ void __launch_bounds__(256, (CLUSTER ? 1 : (R >= 4 ? ICPB_EXH_CTAS : ICPB_MIN_CTAS)))
+// large-scan variant: the prefetched chunk needs 32 more registers than the shared-memory sweep, and
+// shared memory does not limit its occupancy
+#ifndef ICPB_BIG_CTAS
+#define ICPB_BIG_CTAS 2
+#endif
+__global__ void __launch_bounds__(256, (CLUSTER ? 1 : (BIG && PRUNE ? ICPB_BIG_CTAS : (R >= 4 ? ICPB_EXH_CTAS : ICPB_MIN_CTAS))))
 icp_align_kernel(const KernelArgs a)
 {
-    float  *tqx    = reinterpret_cast<float *>(smem_raw);
-    float  *tqy    = reinterpret_cast<float *>(smem_raw + a.o_tqy);
-    float4 *cb     = reinterpret_cast<float4 *>(smem_raw + a.o_cb);          // chunk circle (cx, cy, r', -)
-    float4 *tc     = reinterpret_cast<float4 *>(smem_raw + a.o_tc);          // group circles, untransformed source
-    int2   *mm     = reinterpret_cast<int2 *>(smem_raw + a.o_mm);            // [2][ntile_cap] (min, max) matched index per tile
-    int    *corr_s = reinterpret_cast<int *>(smem_raw + a.o_corr);
-    double *red    = reinterpret_cast<double *>(smem_raw + a.o_red);         // [2][ntile_cap][8]
+    unsigned char *const arr = BIG ? a.big_scratch + (size_t)blockIdx.x * (size_t)a.big_stride : smem_raw;
+    float  *tqx    = reinterpret_cast<float *>(arr);
+    float  *tqy    = reinterpret_cast<float *>(arr + a.o_tqy);
+    float4 *cb     = reinterpret_cast<float4 *>(arr + a.o_cb);               // chunk circle (cx, cy, r', -)
+    float4 *tc     = reinterpret_cast<float4 *>(arr + a.o_tc);               // group circles, untransformed source
+    int2   *mm     = reinterpret_cast<int2 *>(arr + a.o_mm);                 // [2][ntile_cap] (min, max) matched index per tile
+    int    *corr_s = reinterpret_cast<int *>(arr + a.o_corr);
+    double *red    = reinterpret_cast<double *>(arr + a.o_red);              // [2][ntile_cap][8]
     double *Tw     = reinterpret_cast<double *>(smem_raw + a.o_tw);          // [kMaxWarps][8] per-warp copy of T
     double *S0     = reinterpret_cast<double *>(smem_raw + a.o_s0);          // sum of (source - first source point)
     __shared__ long long s_pid;
@@ -722,10 +754,11 @@ icp_align_kernel(const KernelArgs a)
                     return fminf(cm, d[15]);
                 };
                 // one sweep step: chunk c (per lane: the lanes of a group agree, groups differ)
-                auto sweep = [&](int c) {
-                    float4 X[4], Y[4];
+                auto load_chunk = [&](int c, float4 (&X)[4], float4 (&Y)[4]) {
 #pragma unroll
                     for (int v = 0; v < 4; ++v) { X[v] = qx4[4 * c + v]; Y[v] = qy4[4 * c + v]; }
+                };
+                auto sweep_xy = [&](int c, const float4 (&X)[4], const float4 (&Y)[4]) {
 #pragma unroll
                     for (int r = 0; r < R; ++r) {
                         const float cm = chunk_min(X, Y, r);
@@ -733,6 +766,28 @@ icp_align_kernel(const KernelArgs a)
                         m2[r] = fminf(m2[r], better ? m1[r] : cm);
                         m1[r] = fminf(m1[r], cm);
                         c1[r] = better ? c : c1[r];
+                    }
+                };
+                auto sweep = [&](int c) {
+                    float4 X[4], Y[4];
+                    load_chunk(c, X, Y);
+                    sweep_xy(c, X, Y);
+                };
+                // BIG, pruned: chunk c is swept while the next one is on its way from L1/L2 (the last step
+                // loads the all-padding chunk, which is staged like any other)
+                auto sweep_prefetched = [&](int steps, auto next) {
+                    int c0 = next(), c1;
+                    float4 X0[4], Y0[4], X1[4], Y1[4];           // ping-pong: no register copies
+                    load_chunk(c0, X0, Y0);
+#pragma unroll 1
+                    for (int st = 0; st < steps; st += 2) {
+                        c1 = next();
+                        load_chunk(c1, X1, Y1);
+                        sweep_xy(c0, X0, Y0);
+                        if (st + 1 == steps) break;
+                        c0 = next();
+                        load_chunk(c0, X0, Y0);
+                        sweep_xy(c1, X1, Y1);
                     }
                 };
                 if (PRUNE) {
@@ -821,11 +876,19 @@ icp_align_kernel(const KernelArgs a)
                         // chunks sweeps the all-padding chunk (index nchunks), which changes nothing
                         const int steps = __reduce_max_sync(0xffffffffu, __popc(mask));
                         executed += (unsigned)steps;
+                        if constexpr (BIG) {
+                            sweep_prefetched(steps, [&]() {
+                                const int c = mask ? cbase + __ffs(mask) - 1 : nchunks;
+                                mask &= mask - 1;
+                                return c;
+                            });
+                        } else {
 #pragma unroll 1
                         for (int st = 0; st < steps; ++st) {
                             const int c = mask ? cbase + __ffs(mask) - 1 : nchunks;
                             mask &= mask - 1;
                             sweep(c);
+                        }
                         }
                     }
                 } else {
@@ -836,6 +899,8 @@ icp_align_kernel(const KernelArgs a)
                     pm = warp_max_nonneg(pm);
                     tol_e = 2.0f * 5.9604645e-8f * (pm + qmax) * 1.0001f;
                     executed += (unsigned)nchunks;
+                    // (BIG included: consecutive chunks, so the loads mostly hit L1; a prefetched chunk
+                    // would not fit the register budget of R = 4 without spills)
 #pragma unroll kExhUnroll
                     for (int c = 0; c < nchunks; ++c) sweep(c);
                 }
@@ -877,9 +942,12 @@ icp_align_kernel(const KernelArgs a)
                             static_assert(kChunk == 16, "the candidate mask is written out for 16 targets");
                             const unsigned acc = (acc0 << 8) | acc1;
                             int idx = j0 + __clz((int)acc) - 16;  // unique candidate: no fp64 needed
-                            if (m2[r] <= thr)                    // another chunk is within the bound
-                                idx = exact_decide_all(nchunks, n2, j0, thr, px[r], py[r], Px, Py, a.o_tqy, a.o_cb, dst);
-                            else if (acc & (acc - 1))            // more than one candidate in the chunk
+                            if (m2[r] <= thr) {                  // another chunk is within the bound
+                                if constexpr (BIG)
+                                    idx = exact_decide_all_at(arr, nchunks, n2, j0, thr, px[r], py[r], Px, Py, a.o_tqy, a.o_cb, dst);
+                                else
+                                    idx = exact_decide_all(nchunks, n2, j0, thr, px[r], py[r], Px, Py, a.o_tqy, a.o_cb, dst);
+                            } else if (acc & (acc - 1))            // more than one candidate in the chunk
                                 idx = exact_decide_chunk(j0, __brev(acc) >> 16, Px, Py, dst);
                             else if (acc == 0)                   // (non-finite input: keep a valid index)
                                 idx = j0;
@@ -924,6 +992,7 @@ icp_align_kernel(const KernelArgs a)
             }
 
             // =========== fit (src/icp.py:22-52): deterministic reduction, one barrier per pass ===========
+            if constexpr (BIG && CLUSTER) __threadfence();     // the other CTAs read this pass's sums from L2
             sync_all();
             if (tid == 0) s_tile_ctr[passes & 1] = 0;          // next used two passes from now
             // every warp folds the tile partials in the same fixed order and updates its own copy of T:
@@ -938,6 +1007,18 @@ icp_align_kernel(const KernelArgs a)
                 if (!CLUSTER) {
                     for (int t = lane >> 3; t < ntiles; t += 4) col += redp[t * kNumSums + k];
                     for (int t = lane; t < ntiles; t += 32) { const int2 v = mmp[t]; mn = min(mn, v.x); mx = max(mx, v.y); }
+                } else if constexpr (BIG) {                            // tile t lives in the scratch of CTA (t / SUBT) mod csize
+                    // (the cluster's CTAs are consecutive blocks with consecutive regions; __ldcg: from L2,
+                    // never a line this SM cached in an earlier pass)
+                    auto peer = [&](auto *p, int t) {
+                        const ptrdiff_t d = (ptrdiff_t)((t / SUBT) % csize - crank) * (ptrdiff_t)a.big_stride;
+                        return reinterpret_cast<decltype(p)>(reinterpret_cast<unsigned char *>(p) + d);
+                    };
+                    for (int t = lane >> 3; t < ntiles; t += 4) col += __ldcg(peer(redp, t) + t * kNumSums + k);
+                    for (int t = lane; t < ntiles; t += 32) {
+                        const int2 v = __ldcg(peer(mmp, t) + t);
+                        mn = min(mn, v.x); mx = max(mx, v.y);
+                    }
                 } else {                                     // tile t lives in CTA (t / SUBT) mod csize
                     cg::cluster_group cluster = cg::this_cluster();
                     for (int t = lane >> 3; t < ntiles; t += 4)

@@ -32,7 +32,8 @@ extern "C" {
 #define ICPB_ABI_VERSION 2
 
 #define ICPB_EINVAL   10001   /* bad argument (null pointer, empty scan, negative size ...)   */
-#define ICPB_ETOOLONG 10002   /* a scan does not fit the kernel's shared-memory staging       */
+#define ICPB_ETOOLONG 10002   /* a scan beyond the kernel's 32-bit layout offsets (~100 M points);
+                                 scans that do not fit shared memory run on the large-scan variant */
 #define ICPB_ENOSCANS 10003   /* run called before a scan table was set                       */
 
 /* icpb_params.flags: sweep every target for every source point (the reference's brute force,
@@ -320,7 +321,15 @@ int icpb_get_kernel_info(icpb_handle h, int64_t B, icpb_kernel_info *out);
  * width cap, multiple of 32), "cluster" (force a cluster size: 0/1 never, 2/4/8), "segments" (upload
  * pieces), "pack_threads" (host threads of icpb_align_host_scans, default min(8, cpus)),
  * "flag_copy" (arrival counter by 4-byte copies), "drop_counter" (tests: never
- * advance the arrival counter), "trace" (host timings on stderr).  0 / -1 restore the default. */
+ * advance the arrival counter), "trace" (host timings on stderr), "large" (1: every pair on the
+ * large-scan variant, arrays in device scratch instead of shared memory -- same results; 0 / -1: only
+ * pairs whose scans do not fit shared memory).  0 / -1 restore the default.
+ *
+ * Scans of any length: a pair whose longer scan does not fit one CTA's shared memory runs on the
+ * large-scan variant of the kernel.  Where the host sees the pairs (icpb_run_host, icpb_align_host*,
+ * icpb_icp_pair_host) a batch is split: the pairs that fit run on the shared-memory kernel, the others
+ * on the large variant; icpb_run_device* and pair_mode 1 send the whole batch to the large variant
+ * when the table's longest scan does not fit.  Both variants give the same bits. */
 int icpb_set_tuning(icpb_handle h, const char *key, int64_t value);
 
 /* Number of alignment-kernel launches made through this handle (bench.py's gpu_launches). */
