@@ -135,19 +135,20 @@ typedef void (*kernel_fn)(const icpb::KernelArgs);
 constexpr int kPointsExhaustive = 4;
 bool is_exhaustive(const icpb_params *p) { return p && (p->flags & ICPB_FLAG_EXHAUSTIVE); }
 int points_per_thread(const icpb_params *p) { return is_exhaustive(p) ? kPointsExhaustive : kPointsPerThread; }
-kernel_fn pick_kernel(const icpb_params *p)
+// The six instances of the alignment kernel: exhaustive, pruned, pruned in a cluster; the first three keep
+// their arrays in shared memory, the last three are the large-scan variants (KernelArgs::big_scratch: same
+// code, arrays in device scratch).
+const kernel_fn kAlignKernels[6] = {
+    icpb::icp_align_kernel<kPointsExhaustive, false, false>, icpb::icp_align_kernel<kPointsPerThread, true, false>,
+    icpb::icp_align_kernel<kPointsPerThread, true, true>,
+    icpb::icp_align_kernel<kPointsExhaustive, false, false, true>,
+    icpb::icp_align_kernel<kPointsPerThread, true, false, true>,
+    icpb::icp_align_kernel<kPointsPerThread, true, true, true>};
+// (make_cfg never gives an exhaustive run a cluster: the cluster instance is a pruned one)
+kernel_fn align_kernel(bool big, bool exhaustive, bool cluster)
 {
-    return is_exhaustive(p) ? icpb::icp_align_kernel<kPointsExhaustive, false, false>
-                            : icpb::icp_align_kernel<kPointsPerThread, true, false>;
+    return kAlignKernels[(big ? 3 : 0) + (cluster ? 2 : exhaustive ? 0 : 1)];
 }
-kernel_fn cluster_kernel() { return icpb::icp_align_kernel<kPointsPerThread, true, true>; }
-// the large-scan variants (KernelArgs::big_scratch): same code, arrays in device scratch
-kernel_fn big_kernel(const icpb_params *p)
-{
-    return is_exhaustive(p) ? icpb::icp_align_kernel<kPointsExhaustive, false, false, true>
-                            : icpb::icp_align_kernel<kPointsPerThread, true, false, true>;
-}
-kernel_fn big_cluster_kernel() { return icpb::icp_align_kernel<kPointsPerThread, true, true, true>; }
 // Scratch of the large-scan variant: one region per resident CTA, the grid capped so that all regions
 // together stay within this budget (a 100,000-point scan needs ~1.7 MB per CTA: ~600 CTAs).
 constexpr int64_t kBigScratchBudget = int64_t(1) << 30;
@@ -290,6 +291,21 @@ struct PackPool {
     }
 };
 
+// The workers of a PackPool write through a PackJob on the dispatching call's stack frame: this guard,
+// declared after the job and what it points to, stops them on every way out of that call.
+struct PackGuard {
+    PackJob *job = nullptr;                             // set while workers may be running it
+    PackPool *pool = nullptr;
+    void finish()                                       // hand out no more jobs, wait for the workers
+    {
+        if (!job) return;
+        job->next.store(job->n_jobs, std::memory_order_relaxed);
+        if (pool) pool->finish();
+        job = nullptr;
+    }
+    ~PackGuard() { finish(); }
+};
+
 }  // namespace
 
 struct icpb_ctx {
@@ -369,7 +385,7 @@ int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, const icpb_p
         return ICPB_ETOOLONG;
     }
     if (L.bytes > h->smem_limit) big = true;
-    const kernel_fn fn = big ? big_kernel(p) : pick_kernel(p);
+    const kernel_fn fn = align_kernel(big, is_exhaustive(p), false);
     // large-scan variant: Tw, S0 and the transpose scratch stay in shared memory, at offsets from 0
     const int64_t smem = big ? L.bytes - L.o_tw : L.bytes;
     c->threads = threads; c->smem = (int)smem; c->L = L; c->big = big;
@@ -421,7 +437,7 @@ int check_params(const icpb_params *p, int64_t B)
     return 0;
 }
 
-int check_epilogue(const icpb_epilogue *ep, const icpb_params *p)
+int check_epilogue(const icpb_epilogue *ep)
 {
     if (!ep) return 0;
     const bool gather = ep->d_peer_ptrs != nullptr;
@@ -436,120 +452,166 @@ int check_epilogue(const icpb_epilogue *ep, const icpb_params *p)
             return fail(ICPB_EINVAL, "epilogue: peer acceptance needs the peers' count arrays and a rank in range%s");
         if (!ep->d_accept_peer_ptrs && !ep->d_accept_count) return fail(ICPB_EINVAL, "epilogue: d_accept_count is null%s");
     }
-    (void)p;
+    return 0;
+}
+
+// The checks of icpb_run_device, icpb_run_device_ex and icpb_run_host, in this order: handle, parameters,
+// table, then the (host or device) buffers.  empty_ok: a batch of no pairs needs no buffers.
+int run_check(const icpb_ctx *h, const icpb_params *p, int64_t B, bool empty_ok, const void *pairs,
+              const void *T, const void *err, const void *passes, const void *hist, const void *corr)
+{
+    if (!h) return fail(ICPB_EINVAL, "handle is null%s");
+    int rc = check_params(p, B);
+    if (rc) return rc;
+    if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
+    if (B == 0 && empty_ok) return 0;
+    if (B > 0 && (!T || !err || !passes)) return fail(ICPB_EINVAL, "output pointer is null%s");
+    if (B > 0 && p->pair_mode == 0 && !pairs) return fail(ICPB_EINVAL, "pairs is null with pair_mode 0%s");
+    if (p->hist_cap > 0 && !hist) return fail(ICPB_EINVAL, "hist_cap > 0 without a history buffer%s");
+    if (p->corr_stride > 0 && !corr) return fail(ICPB_EINVAL, "corr_stride > 0 without a correspondence buffer%s");
+    if (p->corr_stride > 0 && p->corr_stride < h->longest)
+        return fail(ICPB_EINVAL, "corr_stride is smaller than the longest scan%s");
     return 0;
 }
 
 int ensure_prep(icpb_ctx *h, cudaStream_t stream);
 
-// One of the (at most two) launches of a batch split by scan length (launch_split).
-struct LaunchPart {
-    int64_t B_all;            // pairs of the whole batch: epilogue rows are pair ids of it
-    bool big;                 // the large-scan variant
-    bool accept_continue;     // the acceptance count goes on from the previous launch of the batch
+// A batch whose longest scan does not fit shared memory, on an entry point that sees the pairs, runs as
+// two launches: the pairs that fit (fits_smem of the longer scan) on the shared-memory kernel at the
+// layout of the longest scan among them, then the others on the large-scan variant.  Both write the
+// outputs by pair id; the queue holds the first part's pairs, then the second's, each in its original
+// order.  The two variants give the same bits, so the split decides speed only.
+struct Split {
+    int64_t ns = 0;            // pairs in the first part
+    int64_t Ls = 0, Ll = 0;    // longest scan of each part
 };
 
-int launch(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scans, int64_t longest,
-           const int32_t *d_pairs, const double *d_init, int64_t B, const icpb_params *p,
-           double *d_T, double *d_err, int32_t *d_passes, double *d_hist, int32_t *d_corr,
-           cudaStream_t stream, int64_t B_total = 0, const int32_t *d_seg_of_pair = nullptr,
-           const int32_t *d_arrived = nullptr, const icpb_epilogue *ep = nullptr,
-           const int32_t *d_order = nullptr, int32_t *d_upload_timeout = nullptr,
-           unsigned char *prep_out = nullptr, int64_t prep_stride_out = 0, const LaunchPart *part = nullptr)
+// One batch of alignment problems as launch() enqueues it.  Fields a caller does not set stay null / 0.
+struct Batch {
+    const double *xy = nullptr;                     // the scan table
+    const int64_t *offsets = nullptr;
+    int64_t n_scans = 0, longest = 0;
+    const int32_t *pairs = nullptr;                 // the problems
+    const double *init = nullptr;
+    int64_t B = 0;
+    const icpb_params *p = nullptr;
+    double *T = nullptr, *err = nullptr, *hist = nullptr;   // the outputs, by pair id
+    int32_t *passes = nullptr, *corr = nullptr;
+    cudaStream_t stream = nullptr;
+    const icpb_epilogue *ep = nullptr;
+    const int32_t *order = nullptr;                 // queue position -> pair id (nullptr: identity)
+    // streaming upload: a pair waits until *arrived > seg_of_pair[its queue position]
+    const int32_t *seg_of_pair = nullptr, *arrived = nullptr;
+    int32_t *upload_timeout = nullptr;
+    unsigned char *prep_out = nullptr;              // prep mode: build the table's staging images (ensure_prep)
+    int64_t prep_stride = 0;
+    const Split *split = nullptr;                   // split by scan length; `order` holds the split queue
+};
+
+// Enqueues a batch: one kernel launch, or two for a split batch (queue positions [0, ns) on the
+// shared-memory kernel at the layout of Ls, the others on the large-scan variant at Ll).  A batch
+// without a split is one whose first part holds every pair.
+int launch(icpb_ctx *h, const Batch &b)
 {
-    const bool prep_building = prep_out != nullptr;
-    if (B == 0) return 0;
-    LaunchCfg cfg;
-    const bool force_big = part ? part->big : (h->tune_large == 1 && !prep_building);
-    int rc = make_cfg(h, longest, B_total > B ? B_total : B, &cfg, p, force_big);
-    if (rc) return rc;
-    const kernel_fn fn = cfg.big ? big_kernel(p) : pick_kernel(p);
-    const kernel_fn cfn = cfg.big ? big_cluster_kernel() : cluster_kernel();
-    icpb::KernelArgs a;
-    a.xy = xy; a.offsets = offsets; a.pairs = d_pairs; a.init = d_init; a.B = B; a.n_scans = n_scans;
-    a.p = *p;
-    a.T_out = d_T; a.err_out = d_err; a.passes_out = d_passes;
-    a.hist = p->hist_cap > 0 ? d_hist : nullptr;
-    a.corr = p->corr_stride > 0 ? d_corr : nullptr;
-    a.queue = h->queue + (h->launches % kQueueRing);
-    a.n2pad_cap = cfg.L.n2pad; a.n1_cap = cfg.L.n1c; a.nchunk_cap = cfg.L.nchunk; a.ntile_cap = cfg.L.ntile;
-    a.o_tqy = cfg.L.o_tqy; a.o_cb = cfg.L.o_cb; a.o_tc = cfg.L.o_tc; a.o_mm = cfg.L.o_mm; a.o_corr = cfg.L.o_corr;
-    a.o_red = cfg.L.o_red; a.o_tw = cfg.L.o_tw; a.o_s0 = cfg.L.o_s0; a.o_scr = cfg.L.o_scr;
-    a.big_scratch = nullptr; a.big_stride = 0;
-    if (cfg.big) { a.o_tw = 0; a.o_s0 = cfg.L.o_s0 - cfg.L.o_tw; a.o_scr = cfg.L.o_scr - cfg.L.o_tw; }
-    a.executed = h->executed;
-    a.seg_of_pair = d_seg_of_pair; a.arrived = d_arrived; a.order = d_order; a.upload_timeout = d_upload_timeout;
-    a.prep_out = nullptr; a.prep_in = nullptr; a.prep_stride = 0;
-    if (d_arrived == nullptr && xy == h->xy && h->xy != nullptr && !prep_building && longest == h->longest) {
-        // a resident table: stage every pair by copy from the per-scan images (built once per table)
-        int rc2 = ensure_prep(h, stream);
-        if (rc2) return rc2;
-        if (h->prep_for == h->xy) { a.prep_in = (const unsigned char *)h->prep.p; a.prep_stride = h->prep_stride; }
-    }
-    if (prep_out) { a.prep_out = prep_out; a.prep_stride = prep_stride_out; }
-    a.peers = nullptr; a.n_peers = 0; a.rec_row0 = 0; a.rec_block = part ? part->B_all : B; a.rec_stride = 0;
-    a.accept_thresh = 0.0; a.accept_rec = nullptr; a.accept_peers = nullptr; a.accept_ctr = nullptr;
-    a.accept_count_out = nullptr; a.accept_count_peers = nullptr; a.accept_cap = 0; a.accept_rank = 0;
-    if (ep) {
-        a.peers = (double *const *)ep->d_peer_ptrs; a.n_peers = ep->n_peers;
-        a.rec_row0 = ep->row0; a.rec_stride = ep->row_stride;
-        if (ep->row_block > 0) a.rec_block = ep->row_block;
-        if (ep->d_accept_rec || ep->d_accept_peer_ptrs) {
-            int rc2;
-            if ((rc2 = h->s_accept.reserve(2 * sizeof(unsigned long long)))) return rc2;
-            a.accept_thresh = ep->accept_thresh; a.accept_cap = ep->accept_cap; a.accept_rank = ep->rank;
-            a.accept_rec = ep->d_accept_peer_ptrs ? nullptr : ep->d_accept_rec;
-            a.accept_peers = (double *const *)ep->d_accept_peer_ptrs;
-            a.accept_count_peers = (long long *const *)ep->d_accept_count_peer_ptrs;
-            a.accept_count_out = (long long *)ep->d_accept_count;
-            a.accept_ctr = (unsigned long long *)h->s_accept.p;
-            // [0] rows appended: zeroed by the first launch of a batch only; [1] CTAs that have left: per launch
-            const bool cont = part && part->accept_continue;
-            CU(cudaMemsetAsync(a.accept_ctr + (cont ? 1 : 0), 0, (cont ? 1 : 2) * sizeof(unsigned long long), stream));
+    const icpb_params *p = b.p;
+    const bool prep_building = b.prep_out != nullptr;
+    const Split whole = {b.B, b.longest, 0};
+    const Split &sp = b.split ? *b.split : whole;
+    for (int part = 0; part < 2; ++part) {
+        const int64_t q0 = part ? sp.ns : 0;                  // queue position of the part's first pair
+        const int64_t B = part ? b.B - sp.ns : sp.ns, longest = part ? sp.Ll : sp.Ls;
+        if (B == 0) continue;
+        LaunchCfg cfg;
+        int rc = make_cfg(h, longest, B, &cfg, p, part == 1 || (h->tune_large == 1 && !prep_building));
+        if (rc) return rc;
+        const kernel_fn fn = align_kernel(cfg.big, is_exhaustive(p), cfg.cluster > 1);
+        icpb::KernelArgs a;
+        a.xy = b.xy; a.offsets = b.offsets; a.pairs = b.pairs; a.init = b.init; a.B = B; a.n_scans = b.n_scans;
+        a.p = *p;
+        a.T_out = b.T; a.err_out = b.err; a.passes_out = b.passes;
+        a.hist = p->hist_cap > 0 ? b.hist : nullptr;
+        a.corr = p->corr_stride > 0 ? b.corr : nullptr;
+        a.queue = h->queue + (h->launches % kQueueRing);
+        a.n2pad_cap = cfg.L.n2pad; a.n1_cap = cfg.L.n1c; a.nchunk_cap = cfg.L.nchunk; a.ntile_cap = cfg.L.ntile;
+        a.o_tqy = cfg.L.o_tqy; a.o_cb = cfg.L.o_cb; a.o_tc = cfg.L.o_tc; a.o_mm = cfg.L.o_mm; a.o_corr = cfg.L.o_corr;
+        a.o_red = cfg.L.o_red; a.o_tw = cfg.L.o_tw; a.o_s0 = cfg.L.o_s0; a.o_scr = cfg.L.o_scr;
+        a.big_scratch = nullptr; a.big_stride = 0;
+        if (cfg.big) { a.o_tw = 0; a.o_s0 = cfg.L.o_s0 - cfg.L.o_tw; a.o_scr = cfg.L.o_scr - cfg.L.o_tw; }
+        a.executed = h->executed;
+        a.seg_of_pair = b.seg_of_pair ? b.seg_of_pair + q0 : nullptr; a.arrived = b.arrived;
+        a.order = b.order ? b.order + q0 : nullptr; a.upload_timeout = b.upload_timeout;
+        a.prep_out = b.prep_out; a.prep_in = nullptr; a.prep_stride = b.prep_stride;
+        if (b.arrived == nullptr && b.xy == h->xy && h->xy != nullptr && !prep_building && longest == h->longest) {
+            // a resident table: stage every pair by copy from the per-scan images (built once per table)
+            int rc2 = ensure_prep(h, b.stream);
+            if (rc2) return rc2;
+            if (h->prep_for == h->xy) { a.prep_in = (const unsigned char *)h->prep.p; a.prep_stride = h->prep_stride; }
         }
-    }
-    CU(cudaMemsetAsync(a.queue, 0, sizeof(unsigned long long), stream));
-    int64_t grid = (int64_t)cfg.ctas_per_sm * h->sm_count;
-    if (grid > B) grid = B;
-    int64_t max_ctas = grid * cfg.cluster;                    // CTAs the launch may have
-    if (cfg.big) {
-        // one scratch region per CTA, within kBigScratchBudget; with less device memory free, fewer
-        // CTAs, down to one cluster (or CTA) -- only if that cannot be had does the call fail
-        int64_t cap = kBigScratchBudget / cfg.big_stride / cfg.cluster * cfg.cluster;
-        if (cap < cfg.cluster) cap = cfg.cluster;
-        if (max_ctas > cap) max_ctas = cap;
-        for (;;) {
-            const int rc2 = h->s_big.reserve((size_t)(max_ctas * cfg.big_stride));
-            if (rc2 == 0) break;
-            cudaGetLastError();
-            if (max_ctas <= cfg.cluster) return rc2;          // g_err names the allocation that failed
-            max_ctas = (max_ctas / 2 + cfg.cluster - 1) / cfg.cluster * cfg.cluster;
+        // epilogue rows are pair ids of the whole batch
+        a.peers = nullptr; a.n_peers = 0; a.rec_row0 = 0; a.rec_block = b.B; a.rec_stride = 0;
+        a.accept_thresh = 0.0; a.accept_rec = nullptr; a.accept_peers = nullptr; a.accept_ctr = nullptr;
+        a.accept_count_out = nullptr; a.accept_count_peers = nullptr; a.accept_cap = 0; a.accept_rank = 0;
+        if (const icpb_epilogue *ep = b.ep) {
+            a.peers = (double *const *)ep->d_peer_ptrs; a.n_peers = ep->n_peers;
+            a.rec_row0 = ep->row0; a.rec_stride = ep->row_stride;
+            if (ep->row_block > 0) a.rec_block = ep->row_block;
+            if (ep->d_accept_rec || ep->d_accept_peer_ptrs) {
+                int rc2;
+                if ((rc2 = h->s_accept.reserve(2 * sizeof(unsigned long long)))) return rc2;
+                a.accept_thresh = ep->accept_thresh; a.accept_cap = ep->accept_cap; a.accept_rank = ep->rank;
+                a.accept_rec = ep->d_accept_peer_ptrs ? nullptr : ep->d_accept_rec;
+                a.accept_peers = (double *const *)ep->d_accept_peer_ptrs;
+                a.accept_count_peers = (long long *const *)ep->d_accept_count_peer_ptrs;
+                a.accept_count_out = (long long *)ep->d_accept_count;
+                a.accept_ctr = (unsigned long long *)h->s_accept.p;
+                // [0] rows appended: zeroed by the first launch of a batch only; [1] CTAs that have left: per launch
+                const bool cont = q0 > 0;
+                CU(cudaMemsetAsync(a.accept_ctr + (cont ? 1 : 0), 0, (cont ? 1 : 2) * sizeof(unsigned long long), b.stream));
+            }
         }
-        a.big_scratch = (unsigned char *)h->s_big.p; a.big_stride = cfg.big_stride;
-        if (grid > max_ctas) grid = max_ctas;
+        CU(cudaMemsetAsync(a.queue, 0, sizeof(unsigned long long), b.stream));
+        int64_t grid = (int64_t)cfg.ctas_per_sm * h->sm_count;
+        if (grid > B) grid = B;
+        int64_t max_ctas = grid * cfg.cluster;                    // CTAs the launch may have
+        if (cfg.big) {
+            // one scratch region per CTA, within kBigScratchBudget; with less device memory free, fewer
+            // CTAs, down to one cluster (or CTA) -- only if that cannot be had does the call fail
+            int64_t cap = kBigScratchBudget / cfg.big_stride / cfg.cluster * cfg.cluster;
+            if (cap < cfg.cluster) cap = cfg.cluster;
+            if (max_ctas > cap) max_ctas = cap;
+            for (;;) {
+                const int rc2 = h->s_big.reserve((size_t)(max_ctas * cfg.big_stride));
+                if (rc2 == 0) break;
+                cudaGetLastError();
+                if (max_ctas <= cfg.cluster) return rc2;          // g_err names the allocation that failed
+                max_ctas = (max_ctas / 2 + cfg.cluster - 1) / cfg.cluster * cfg.cluster;
+            }
+            a.big_scratch = (unsigned char *)h->s_big.p; a.big_stride = cfg.big_stride;
+            if (grid > max_ctas) grid = max_ctas;
+        }
+        if (cfg.cluster > 1) {
+            cudaLaunchConfig_t lc = {};
+            cudaLaunchAttribute attr[1];
+            attr[0].id = cudaLaunchAttributeClusterDimension;
+            attr[0].val.clusterDim.x = (unsigned)cfg.cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+            lc.blockDim = dim3((unsigned)cfg.threads);
+            lc.dynamicSmemBytes = (size_t)cfg.smem; lc.stream = b.stream; lc.attrs = attr; lc.numAttrs = 1;
+            // one cluster per problem, as many as the device can co-schedule (the occupancy query needs a
+            // grid that is a multiple of the cluster size; it answers in clusters)
+            lc.gridDim = dim3((unsigned)cfg.cluster);
+            int max_clusters = 0;
+            CU(cudaOccupancyMaxActiveClusters(&max_clusters, fn, &lc));
+            int64_t clusters = max_clusters > 0 ? max_clusters : 1;
+            if (clusters > B) clusters = B;
+            if (clusters > max_ctas / cfg.cluster) clusters = max_ctas / cfg.cluster;
+            lc.gridDim = dim3((unsigned)(clusters * cfg.cluster));
+            CU(cudaLaunchKernelEx(&lc, fn, a));
+        } else {
+            fn<<<(unsigned)grid, cfg.threads, cfg.smem, b.stream>>>(a);
+        }
+        CU(cudaGetLastError());
+        h->launches++;
     }
-    if (cfg.cluster > 1) {
-        cudaLaunchConfig_t lc = {};
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)cfg.cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        lc.blockDim = dim3((unsigned)cfg.threads);
-        lc.dynamicSmemBytes = (size_t)cfg.smem; lc.stream = stream; lc.attrs = attr; lc.numAttrs = 1;
-        // one cluster per problem, as many as the device can co-schedule (the occupancy query needs a
-        // grid that is a multiple of the cluster size; it answers in clusters)
-        lc.gridDim = dim3((unsigned)cfg.cluster);
-        int max_clusters = 0;
-        CU(cudaOccupancyMaxActiveClusters(&max_clusters, cfn, &lc));
-        int64_t clusters = max_clusters > 0 ? max_clusters : 1;
-        if (clusters > B) clusters = B;
-        if (clusters > max_ctas / cfg.cluster) clusters = max_ctas / cfg.cluster;
-        lc.gridDim = dim3((unsigned)(clusters * cfg.cluster));
-        CU(cudaLaunchKernelEx(&lc, cfn, a));
-    } else {
-        fn<<<(unsigned)grid, cfg.threads, cfg.smem, stream>>>(a);
-    }
-    CU(cudaGetLastError());
-    h->launches++;
     return 0;
 }
 
@@ -576,23 +638,14 @@ int ensure_prep(icpb_ctx *h, cudaStream_t stream)
     if ((rc = make_cfg(h, h->longest, h->n_scans, &cfg, &p))) return rc;
     if (cfg.big) return 0;
     if ((rc = h->prep.reserve((size_t)(stride * h->n_scans)))) return rc;
-    rc = launch(h, h->xy, h->offsets, h->n_scans, h->longest, nullptr, nullptr, h->n_scans, &p,
-                nullptr, nullptr, nullptr, nullptr, nullptr, stream, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
-                (unsigned char *)h->prep.p, stride);
-    if (rc) return rc;
+    Batch b;
+    b.xy = h->xy; b.offsets = h->offsets; b.n_scans = h->n_scans; b.longest = h->longest;
+    b.B = h->n_scans; b.p = &p; b.stream = stream;
+    b.prep_out = (unsigned char *)h->prep.p; b.prep_stride = stride;
+    if ((rc = launch(h, b))) return rc;
     h->prep_for = h->xy; h->prep_stride = stride; h->prep_scans = h->n_scans; h->prep_longest = h->longest;
     return 0;
 }
-
-// A batch whose longest scan does not fit shared memory, on an entry point that sees the pairs, runs as
-// two launches: the pairs that fit (fits_smem of the longer scan) on the shared-memory kernel at the
-// layout of the longest scan among them, then the others on the large-scan variant.  Both write the
-// outputs by pair id; the queue holds the first part's pairs, then the second's, each in its original
-// order.  The two variants give the same bits, so the split decides speed only.
-struct Split {
-    int64_t ns = 0;            // pairs in the first part
-    int64_t Ls = 0, Ll = 0;    // longest scan of each part
-};
 
 // Whether a batch has to be split: its longest scan does not fit and "large" does not force the variant.
 bool needs_split(icpb_ctx *h, int64_t longest, int64_t B, const icpb_params *p)
@@ -624,23 +677,6 @@ Split split_queue(const icpb_ctx *h, const int64_t *off, const int32_t *pairs, i
     std::copy(hi.begin(), hi.end(), order + sp.ns);
     if (seg) { std::copy(slo.begin(), slo.end(), seg); std::copy(shi.begin(), shi.end(), seg + sp.ns); }
     return sp;
-}
-
-int launch_split(icpb_ctx *h, const double *xy, const int64_t *offsets, int64_t n_scans, const Split &sp,
-                 const int32_t *d_pairs, const double *d_init, int64_t B, const icpb_params *p,
-                 double *d_T, double *d_err, int32_t *d_passes, double *d_hist, int32_t *d_corr,
-                 cudaStream_t stream, const int32_t *d_seg, const int32_t *d_arrived, const icpb_epilogue *ep,
-                 const int32_t *d_order, int32_t *d_upload_timeout)
-{
-    LaunchPart part = {B, false, false};
-    int rc = launch(h, xy, offsets, n_scans, sp.Ls, d_pairs, d_init, sp.ns, p, d_T, d_err, d_passes, d_hist, d_corr,
-                    stream, 0, d_seg, d_arrived, ep, d_order, d_upload_timeout, nullptr, 0, &part);
-    if (rc) return rc;
-    part.big = true;
-    part.accept_continue = sp.ns > 0;
-    return launch(h, xy, offsets, n_scans, sp.Ll, d_pairs, d_init, B - sp.ns, p, d_T, d_err, d_passes, d_hist, d_corr,
-                  stream, 0, d_seg ? d_seg + sp.ns : nullptr, d_arrived, ep, d_order + sp.ns, d_upload_timeout,
-                  nullptr, 0, &part);
 }
 
 }  // namespace
@@ -687,25 +723,17 @@ int icpb_create(int device, icpb_handle *out)
     for (int k = 0; k < 16 && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&h->seg_ev[k], cudaEventDisableTiming);
     for (int k = 0; k < 2 && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&h->done_ev[k], cudaEventDisableTiming);
     // dynamic shared memory up to the device's opt-in maximum minus each kernel's static part, set
-    // once: the attribute belongs to the function, not to a handle
+    // once: the attribute belongs to the function, not to a handle.  The large-scan variants keep only
+    // a few KB in shared memory but ask for the same maximum; the limit a layout must fit comes from
+    // the three shared-memory instances.
     h->smem_limit = (int)prop.sharedMemPerBlockOptin;
-    for (kernel_fn fn : {pick_kernel(nullptr), cluster_kernel(),
-                         (kernel_fn)icpb::icp_align_kernel<kPointsExhaustive, false, false>}) {
+    for (int k = 0; k < 6 && e == cudaSuccess; ++k) {
         cudaFuncAttributes fa;
-        if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, fn);
+        e = cudaFuncGetAttributes(&fa, kAlignKernels[k]);
         if (e != cudaSuccess) break;
         const int lim = (int)prop.sharedMemPerBlockOptin - (int)fa.sharedSizeBytes;
-        e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
-        if (lim < h->smem_limit) h->smem_limit = lim;
-    }
-    // the large-scan variants keep only a few KB in shared memory, but ask for the same maximum
-    for (kernel_fn fn : {big_kernel(nullptr), big_cluster_kernel(),
-                         (kernel_fn)icpb::icp_align_kernel<kPointsExhaustive, false, false, true>}) {
-        cudaFuncAttributes fa;
-        if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, fn);
-        if (e != cudaSuccess) break;
-        e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)prop.sharedMemPerBlockOptin - (int)fa.sharedSizeBytes);
+        e = cudaFuncSetAttribute(kAlignKernels[k], cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
+        if (k < 3 && lim < h->smem_limit) h->smem_limit = lim;
     }
     if (e == cudaSuccess) e = cudaMalloc(&h->arrived_dev, sizeof(int32_t));
     if (e == cudaSuccess) e = cudaHostAlloc(&h->seg_vals_pinned, sizeof(int32_t) * (kMaxSegments + 1), cudaHostAllocDefault);
@@ -817,36 +845,32 @@ int icpb_run_device(icpb_handle h, const int32_t *d_pairs, const double *d_init,
                     const icpb_params *p, double *d_T, double *d_err, int32_t *d_passes,
                     double *d_hist, int32_t *d_corr, void *stream)
 {
-    if (!h) return fail(ICPB_EINVAL, "handle is null%s");
-    int rc = check_params(p, B);
+    int rc = run_check(h, p, B, false, d_pairs, d_T, d_err, d_passes, d_hist, d_corr);
     if (rc) return rc;
-    if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
-    if (B > 0 && (!d_T || !d_err || !d_passes)) return fail(ICPB_EINVAL, "output pointer is null%s");
-    if (B > 0 && p->pair_mode == 0 && !d_pairs) return fail(ICPB_EINVAL, "pairs is null with pair_mode 0%s");
-    if (p->hist_cap > 0 && !d_hist) return fail(ICPB_EINVAL, "hist_cap > 0 but hist is null%s");
-    if (p->corr_stride > 0 && !d_corr) return fail(ICPB_EINVAL, "corr_stride > 0 but corr is null%s");
-    if (p->corr_stride > 0 && p->corr_stride < h->longest)
-        return fail(ICPB_EINVAL, "corr_stride is smaller than the longest scan%s");
     ON_DEVICE(h);
-    return launch(h, h->xy, h->offsets, h->n_scans, h->longest, d_pairs, d_init, B, p,
-                  d_T, d_err, d_passes, d_hist, d_corr, (cudaStream_t)stream);
+    Batch b;
+    b.xy = h->xy; b.offsets = h->offsets; b.n_scans = h->n_scans; b.longest = h->longest;
+    b.pairs = d_pairs; b.init = d_init; b.B = B; b.p = p;
+    b.T = d_T; b.err = d_err; b.passes = d_passes; b.hist = d_hist; b.corr = d_corr;
+    b.stream = (cudaStream_t)stream;
+    return launch(h, b);
 }
 
 int icpb_run_device_ex(icpb_handle h, const int32_t *d_pairs, const double *d_init, int64_t B,
                        const icpb_params *p, double *d_T, double *d_err, int32_t *d_passes,
                        const icpb_epilogue *ep, void *stream)
 {
-    if (!h) return fail(ICPB_EINVAL, "handle is null%s");
-    int rc = check_params(p, B);
+    int rc = check_epilogue(ep);
+    // no history or correspondence buffers here: the shared check rejects hist_cap or corr_stride > 0
+    if (rc == 0) rc = run_check(h, p, B, false, d_pairs, d_T, d_err, d_passes, nullptr, nullptr);
     if (rc) return rc;
-    if ((rc = check_epilogue(ep, p))) return rc;
-    if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
-    if (B > 0 && (!d_T || !d_err || !d_passes)) return fail(ICPB_EINVAL, "output pointer is null%s");
-    if (B > 0 && p->pair_mode == 0 && !d_pairs) return fail(ICPB_EINVAL, "pairs is null with pair_mode 0%s");
-    if (p->hist_cap > 0 || p->corr_stride > 0) return fail(ICPB_EINVAL, "icpb_run_device_ex: no history/correspondences%s");
     ON_DEVICE(h);
-    return launch(h, h->xy, h->offsets, h->n_scans, h->longest, d_pairs, d_init, B, p, d_T, d_err, d_passes,
-                  nullptr, nullptr, (cudaStream_t)stream, 0, nullptr, nullptr, ep);
+    Batch b;
+    b.xy = h->xy; b.offsets = h->offsets; b.n_scans = h->n_scans; b.longest = h->longest;
+    b.pairs = d_pairs; b.init = d_init; b.B = B; b.p = p;
+    b.T = d_T; b.err = d_err; b.passes = d_passes;
+    b.stream = (cudaStream_t)stream; b.ep = ep;
+    return launch(h, b);
 }
 
 int icpb_run_device_gather(icpb_handle h, const int32_t *d_pairs, const double *d_init, int64_t B,
@@ -883,26 +907,24 @@ static int run_host_common(icpb_handle h, const double *xy, const int64_t *offse
     if ((rc = h->s_passes.reserve(sizeof(int32_t) * (size_t)B))) return rc;
     if (nbH) { if ((rc = h->s_hist.reserve(nbH))) return rc; CU(cudaMemsetAsync(h->s_hist.p, 0, nbH, st)); }
     if (nbC) { if ((rc = h->s_corr.reserve(nbC))) return rc; CU(cudaMemsetAsync(h->s_corr.p, 0xff, nbC, st)); }
+    Batch b;
+    b.xy = xy; b.offsets = offsets; b.n_scans = n_scans; b.longest = longest;
+    b.pairs = p->pair_mode == 0 ? (const int32_t *)h->s_pairs.p : nullptr;
+    b.init = h_init ? (const double *)h->s_init.p : nullptr; b.B = B; b.p = p;
+    b.T = (double *)h->s_T.p; b.err = (double *)h->s_err.p; b.passes = (int32_t *)h->s_passes.p;
+    b.hist = (double *)h->s_hist.p; b.corr = (int32_t *)h->s_corr.p; b.stream = st;
+    Split sp;
     if (needs_split(h, longest, B, p)) {
         std::vector<int64_t> off((size_t)n_scans + 1);
         std::vector<int32_t> order((size_t)B);
         CU(cudaMemcpyAsync(off.data(), offsets, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
-        const Split sp = split_queue(h, off.data(), h_pairs, B, nullptr, order.data(), nullptr);
+        sp = split_queue(h, off.data(), h_pairs, B, nullptr, order.data(), nullptr);
         if ((rc = h->s_order.reserve(sizeof(int32_t) * (size_t)B))) return rc;
         CU(cudaMemcpyAsync(h->s_order.p, order.data(), sizeof(int32_t) * (size_t)B, cudaMemcpyHostToDevice, st));
-        rc = launch_split(h, xy, offsets, n_scans, sp, (const int32_t *)h->s_pairs.p,
-                          h_init ? (const double *)h->s_init.p : nullptr, B, p,
-                          (double *)h->s_T.p, (double *)h->s_err.p, (int32_t *)h->s_passes.p,
-                          (double *)h->s_hist.p, (int32_t *)h->s_corr.p, st, nullptr, nullptr, nullptr,
-                          (const int32_t *)h->s_order.p, nullptr);
-    } else
-    rc = launch(h, xy, offsets, n_scans, longest,
-                p->pair_mode == 0 ? (const int32_t *)h->s_pairs.p : nullptr,
-                h_init ? (const double *)h->s_init.p : nullptr, B, p,
-                (double *)h->s_T.p, (double *)h->s_err.p, (int32_t *)h->s_passes.p,
-                (double *)h->s_hist.p, (int32_t *)h->s_corr.p, st);
-    if (rc) return rc;
+        b.order = (const int32_t *)h->s_order.p; b.split = &sp;
+    }
+    if ((rc = launch(h, b))) return rc;
     CU(cudaMemcpyAsync(h_T, h->s_T.p, nbI, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(h_err, h->s_err.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(h_passes, h->s_passes.p, sizeof(int32_t) * (size_t)B, cudaMemcpyDeviceToHost, st));
@@ -916,17 +938,8 @@ int icpb_run_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, i
                   const icpb_params *p, double *h_T, double *h_err, int32_t *h_passes,
                   double *h_hist, int32_t *h_corr)
 {
-    if (!h) return fail(ICPB_EINVAL, "handle is null%s");
-    int rc = check_params(p, B);
-    if (rc) return rc;
-    if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
-    if (B == 0) return 0;
-    if (!h_T || !h_err || !h_passes) return fail(ICPB_EINVAL, "output pointer is null%s");
-    if (p->pair_mode == 0 && !h_pairs) return fail(ICPB_EINVAL, "pairs is null with pair_mode 0%s");
-    if (p->hist_cap > 0 && !h_hist) return fail(ICPB_EINVAL, "hist_cap > 0 but hist is null%s");
-    if (p->corr_stride > 0 && !h_corr) return fail(ICPB_EINVAL, "corr_stride > 0 but corr is null%s");
-    if (p->corr_stride > 0 && p->corr_stride < h->longest)
-        return fail(ICPB_EINVAL, "corr_stride is smaller than the longest scan%s");
+    int rc = run_check(h, p, B, true, h_pairs, h_T, h_err, h_passes, h_hist, h_corr);
+    if (rc || B == 0) return rc;
     if (p->pair_mode == 0) {
         for (int64_t b = 0; b < 2 * B; ++b)
             if (h_pairs[b] < 0 || h_pairs[b] >= h->n_scans) return fail(ICPB_EINVAL, "pair index out of range%s");
@@ -1095,6 +1108,7 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     std::vector<int64_t> job_first, job_last;
     std::vector<int32_t> job_piece, jobs_of_piece;
     std::vector<std::atomic<int32_t>> piece_done(src.scan_xy ? (size_t)nseg : 0);
+    PackGuard packers;
     const double *up_xy = src.xy;
     if (src.scan_xy) {
         int nthr = h->tune_pack_threads > 0 ? h->tune_pack_threads : host_threads_available();
@@ -1117,38 +1131,23 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
         job.scan_xy = src.scan_xy; job.offsets = h_offsets; job.dst = (double *)h->stage_xy.p;
         job.job_first = job_first.data(); job.job_last = job_last.data(); job.job_piece = job_piece.data();
         job.n_jobs = (int64_t)job_first.size(); job.done = piece_done.data();
+        packers.job = &job; packers.pool = h->pool;
         if (h->pool) h->pool->start(&job);
         up_xy = (const double *)h->stage_xy.p;
     }
-    // once the pool runs, every exit path must stop it first (the job lives on this stack frame)
-    auto pack_finish = [&]() {
-        if (!src.scan_xy) return;
-        job.next.store(job.n_jobs, std::memory_order_relaxed);   // hand out no more jobs
-        if (h->pool) h->pool->finish();
-    };
-#define CUP(call)                                                                         \
-    do {                                                                                  \
-        cudaError_t e_ = (call);                                                          \
-        if (e_ != cudaSuccess) {                                                          \
-            snprintf(g_err, sizeof g_err, "%s failed: %s", #call, cudaGetErrorString(e_)); \
-            pack_finish();                                                                \
-            return align_abort(h, (int)e_);                                               \
-        }                                                                                 \
-    } while (0)
-
     // The packers (list input) are already at work on the pinned staging; the caller's pairs and initial
     // guesses are checked now, before any state of the handle changes: a rejected call leaves the old
     // table usable.
     {
         int32_t lo = 0, hi = 0;                               // branch-free range check
         for (int64_t b = 0; b < 2 * B; ++b) { lo = h_pairs[b] < lo ? h_pairs[b] : lo; hi = h_pairs[b] > hi ? h_pairs[b] : hi; }
-        if (lo < 0 || hi >= n_scans) { pack_finish(); return fail(ICPB_EINVAL, "pair index out of range%s"); }
+        if (lo < 0 || hi >= n_scans) return fail(ICPB_EINVAL, "pair index out of range%s");
     }
     if (h_init && B > 0) {                                    // before any state of the handle changes
         for (int64_t b = 0; b < B && init_ld == 9; ++b) {
             const double *m = h_init + 9 * b;
             if (!(m[6] == 0.0 && m[7] == 0.0 && m[8] == 1.0))
-            { pack_finish(); return fail(ICPB_EINVAL, "transform bottom row must be [0, 0, 1] (an SE(2) matrix)%s"); }
+                return fail(ICPB_EINVAL, "transform bottom row must be [0, 0, 1] (an SE(2) matrix)%s");
         }
         uint64_t bad = 0;                                     // all-ones exponent = inf or NaN; integer test, vectorises
         for (int64_t k = 0; k < (int64_t)init_ld * B; ++k) {
@@ -1156,13 +1155,14 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
             memcpy(&u, h_init + k, sizeof u);
             bad |= (uint64_t)((u & 0x7ff0000000000000ULL) == 0x7ff0000000000000ULL);
         }
-        if (bad) { pack_finish(); return fail(ICPB_EINVAL, "transform holds non-finite values%s"); }
+        if (bad) return fail(ICPB_EINVAL, "transform holds non-finite values%s");
     }
     // ---- from here on the handle's table is being replaced: a failure leaves it without one ----
     h->prep_for = nullptr; h->xy = nullptr; h->offsets = nullptr; h->n_scans = 0; h->longest = 0;
     cudaStream_t cp = h->stream, cp2 = h->cstream[1], cs = h->cstream[0];
     if (B == 0) {                                             // upload only
-        if (src.scan_xy) { pack_run(&job); pack_finish(); }
+        if (src.scan_xy) pack_run(&job);
+        packers.finish();                                     // before job.bad is read
         if (src.scan_xy && job.bad.load()) return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates%s"));
         CUA(cudaMemcpyAsync(h->own_xy.p, up_xy, nb_xy, cudaMemcpyHostToDevice, cp));
         CUA(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, cp));
@@ -1189,12 +1189,12 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
         s_prev = seg_end[k];
         return e;
     };
-    CUP(cudaMemsetAsync(h->arrived_dev, 0, sizeof(int32_t), cp));
-    CUP(cudaEventRecord(h->seg_ev[1], cp));                   // the counter is zero before the kernel may start
+    CUA(cudaMemsetAsync(h->arrived_dev, 0, sizeof(int32_t), cp));
+    CUA(cudaEventRecord(h->seg_ev[1], cp));                   // the counter is zero before the kernel may start
     int n_sent = 0;
     if (!src.scan_xy) {
         const int n_early = nseg < 4 ? nseg : 4;
-        for (; n_sent < n_early; ++n_sent) CUP(enqueue_piece(n_sent));
+        for (; n_sent < n_early; ++n_sent) CUA(enqueue_piece(n_sent));
     }
     // Queue order: pairs grouped by the segment that completes them; the pairs, initial guesses and
     // results themselves stay in the caller's order.  A batch that already comes in arrival order
@@ -1226,7 +1226,7 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
         }
     }
     // a table whose longest scan does not fit shared memory: the queue is split by scan length, each part
-    // keeping its arrival order (launch_split)
+    // keeping its arrival order
     Split sp;
     const bool split = needs_split(h, longest, B, p);
     if (split) {
@@ -1245,23 +1245,23 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     }
     const double t_prep = trace ? now_us() : 0.0;
     // the small per-pair block goes up on a second copy stream, beside the pieces already in flight
-    CUP(cudaMemsetAsync(d_passes + B, 0, sizeof(int32_t), cp2));
-    CUP(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, cp2));
+    CUA(cudaMemsetAsync(d_passes + B, 0, sizeof(int32_t), cp2));
+    CUA(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, cp2));
     const size_t nb_idx = (in_order ? 3 : 4) * nb4;           // pairs, seg (, order)
-    if (h_init) CUP(cudaMemcpyAsync(d_init, pinit, nbI + nb_idx, cudaMemcpyHostToDevice, cp2));
-    else        CUP(cudaMemcpyAsync(d_pairs, ppairs, nb_idx, cudaMemcpyHostToDevice, cp2));
-    CUP(cudaEventRecord(h->seg_ev[0], cp2));
+    if (h_init) CUA(cudaMemcpyAsync(d_init, pinit, nbI + nb_idx, cudaMemcpyHostToDevice, cp2));
+    else        CUA(cudaMemcpyAsync(d_pairs, ppairs, nb_idx, cudaMemcpyHostToDevice, cp2));
+    CUA(cudaEventRecord(h->seg_ev[0], cp2));
     // ONE launch over all pairs, in arrival order; its CTAs wait on the segment counter
-    CUP(cudaStreamWaitEvent(cs, h->seg_ev[0], 0));
-    CUP(cudaStreamWaitEvent(cs, h->seg_ev[1], 0));
-    if (split)
-        rc = launch_split(h, d_xy, d_off, n_scans, sp, d_pairs, h_init ? d_init : nullptr, B, p, d_T, d_err, d_passes,
-                          nullptr, nullptr, cs, d_seg, h->arrived_dev, ep, d_order, d_passes + B);
-    else
-    rc = launch(h, d_xy, d_off, n_scans, longest, d_pairs, h_init ? d_init : nullptr, B, p,
-                d_T, d_err, d_passes, nullptr, nullptr, cs, B, d_seg, h->arrived_dev, ep,
-                in_order ? nullptr : d_order, d_passes + B);
-    if (rc) { pack_finish(); return align_abort(h, rc); }
+    CUA(cudaStreamWaitEvent(cs, h->seg_ev[0], 0));
+    CUA(cudaStreamWaitEvent(cs, h->seg_ev[1], 0));
+    Batch bt;
+    bt.xy = d_xy; bt.offsets = d_off; bt.n_scans = n_scans; bt.longest = longest;
+    bt.pairs = d_pairs; bt.init = h_init ? d_init : nullptr; bt.B = B; bt.p = p;
+    bt.T = d_T; bt.err = d_err; bt.passes = d_passes;
+    bt.stream = cs; bt.ep = ep; bt.order = in_order ? nullptr : d_order;
+    bt.seg_of_pair = d_seg; bt.arrived = h->arrived_dev; bt.upload_timeout = d_passes + B;
+    bt.split = split ? &sp : nullptr;
+    if ((rc = launch(h, bt))) return align_abort(h, rc);
     bool bad_scans = false;
     double t_ready[kMaxSegments] = {0}, t_enqd[kMaxSegments] = {0};   // trace: piece k packed / enqueued (host clock)
     cudaEvent_t tev[kMaxSegments + 1] = {nullptr};            // trace: when piece k had landed (device clock)
@@ -1284,10 +1284,10 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
             if (job.bad.load(std::memory_order_relaxed)) { bad_scans = true; break; }
         }
         if (trace) { t_ready[k] = now_us() - t_entry; cudaEventCreate(&tev0[k]); cudaEventRecord(tev0[k], cp); }
-        CUP(enqueue_piece(k));
+        CUA(enqueue_piece(k));
         if (trace) { t_enqd[k] = now_us() - t_entry; cudaEventCreate(&tev[k]); cudaEventRecord(tev[k], cp); }
     }
-    pack_finish();
+    packers.finish();                                         // every piece is packed, or a bad scan ended it
     if (bad_scans) {
         // the kernel is waiting for pieces that will not come: raise its give-up flag, drain, report
         CUA(cudaMemcpyAsync(d_passes + B, h->seg_vals_pinned + 1, sizeof(int32_t), cudaMemcpyHostToDevice, cp));
@@ -1307,13 +1307,10 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     if (tP[B] != 0) {
         // a CTA gave up waiting for its scans (see the kernel): by now the whole table is resident,
         // so run the batch again without the streaming protocol
-        if (split)
-            rc = launch_split(h, d_xy, d_off, n_scans, sp, d_pairs, h_init ? d_init : nullptr, B, p, d_T, d_err,
-                              d_passes, nullptr, nullptr, cp, nullptr, nullptr, ep, d_order, nullptr);
-        else
-        rc = launch(h, d_xy, d_off, n_scans, longest, d_pairs, h_init ? d_init : nullptr, B, p,
-                    d_T, d_err, d_passes, nullptr, nullptr, cp, 0, nullptr, nullptr, ep);
-        if (rc) return align_abort(h, rc);
+        Batch again = bt;
+        again.seg_of_pair = nullptr; again.arrived = nullptr; again.upload_timeout = nullptr;
+        again.stream = cp;
+        if ((rc = launch(h, again))) return align_abort(h, rc);
         if (!acc) CUA(cudaMemcpyAsync(tT, d_T, nb_down, cudaMemcpyDeviceToHost, cp));
         else      CUA(cudaMemcpyAsync(acc_cnt, h->s_hist.p, sizeof(int64_t), cudaMemcpyDeviceToHost, cp));
         CUA(cudaStreamSynchronize(cp));
@@ -1373,7 +1370,6 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
         cudaEventDestroy(tev[kMaxSegments]);
     }
     return 0;
-#undef CUP
 }
 
 int align_check(icpb_handle h, int64_t n_scans, const int32_t *h_pairs, int32_t init_ld, int64_t B,
@@ -1385,11 +1381,34 @@ int align_check(icpb_handle h, int64_t n_scans, const int32_t *h_pairs, int32_t 
         return fail(ICPB_EINVAL, "icpb_align_host: init_ld / T_ld must be 6 (2x3 rows) or 9 (3x3)%s");
     int rc = check_params(p, B);
     if (rc) return rc;
-    if ((rc = check_epilogue(ep, p))) return rc;
+    if ((rc = check_epilogue(ep))) return rc;
     if (p->pair_mode != 0 || p->hist_cap > 0 || p->corr_stride > 0)
         return fail(ICPB_EINVAL, "icpb_align_host: explicit pairs, no history/correspondences (use upload + run)%s");
     if (B >= (int64_t(1) << 31)) return fail(ICPB_EINVAL, "icpb_align_host: at most 2^31 - 1 pairs per call%s");
     if (B > 0 && (!h_pairs || !h_T || !h_err || !h_passes)) return fail(ICPB_EINVAL, "null pointer%s");
+    return 0;
+}
+
+// The scan table of an icpb_align_host* call, packed (xy + off) or as a list of arrays (scan_xy +
+// scan_len; its offsets are computed into `offsets`, which src then points to).
+int table_src(const double *xy, const int64_t *off, const double *const *scan_xy, const int64_t *scan_len,
+              int64_t n_scans, std::vector<int64_t> &offsets, TableSrc *src, int64_t *longest)
+{
+    if (xy && off) {
+        src->xy = xy; src->offsets = off;
+        return validate_offsets(off, n_scans, longest);
+    }
+    if (!scan_xy || !scan_len) return fail(ICPB_EINVAL, "icpb_align_host: no scans (xy + offsets or a list of arrays)%s");
+    offsets.resize((size_t)n_scans + 1);
+    offsets[0] = 0;
+    *longest = 0;
+    for (int64_t s = 0; s < n_scans; ++s) {
+        if (!scan_xy[s] || scan_len[s] <= 0)
+            return fail(ICPB_EINVAL, "empty scan in the list (the reference's argmin raises on it)%s");
+        offsets[(size_t)s + 1] = offsets[(size_t)s] + scan_len[s];
+        if (scan_len[s] > *longest) *longest = scan_len[s];
+    }
+    src->scan_xy = scan_xy; src->offsets = offsets.data();
     return 0;
 }
 
@@ -1400,13 +1419,12 @@ int icpb_align_host_ex(icpb_handle h, const double *h_xy, const int64_t *h_offse
                        const icpb_params *p, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes,
                        const icpb_epilogue *ep)
 {
-    if (!h_xy || !h_offsets) return fail(ICPB_EINVAL, "icpb_align_host: bad argument%s");
     int rc = align_check(h, n_scans, h_pairs, init_ld, B, p, h_T, T_ld, h_err, h_passes, ep);
     if (rc) return rc;
-    int64_t longest = 0;
-    if ((rc = validate_offsets(h_offsets, n_scans, &longest))) return rc;
     TableSrc src;
-    src.xy = h_xy; src.offsets = h_offsets;
+    std::vector<int64_t> offsets;
+    int64_t longest = 0;
+    if ((rc = table_src(h_xy, h_offsets, nullptr, nullptr, n_scans, offsets, &src, &longest))) return rc;
     return align_impl(h, src, n_scans, longest, h_pairs, h_init, init_ld, B, p, h_T, T_ld, h_err, h_passes, ep);
 }
 
@@ -1415,20 +1433,12 @@ int icpb_align_host_scans(icpb_handle h, const double *const *scan_xy, const int
                           const icpb_params *p, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes,
                           const icpb_epilogue *ep)
 {
-    if (!scan_xy || !scan_len) return fail(ICPB_EINVAL, "icpb_align_host_scans: bad argument%s");
     int rc = align_check(h, n_scans, h_pairs, init_ld, B, p, h_T, T_ld, h_err, h_passes, ep);
     if (rc) return rc;
-    std::vector<int64_t> offsets((size_t)n_scans + 1);
-    offsets[0] = 0;
-    int64_t longest = 0;
-    for (int64_t s = 0; s < n_scans; ++s) {
-        if (!scan_xy[s] || scan_len[s] <= 0)
-            return fail(ICPB_EINVAL, "empty scan in the list (the reference's argmin raises on it)%s");
-        offsets[(size_t)s + 1] = offsets[(size_t)s] + scan_len[s];
-        if (scan_len[s] > longest) longest = scan_len[s];
-    }
     TableSrc src;
-    src.scan_xy = scan_xy; src.offsets = offsets.data();
+    std::vector<int64_t> offsets;
+    int64_t longest = 0;
+    if ((rc = table_src(nullptr, nullptr, scan_xy, scan_len, n_scans, offsets, &src, &longest))) return rc;
     return align_impl(h, src, n_scans, longest, h_pairs, h_init, init_ld, B, p, h_T, T_ld, h_err, h_passes, ep);
 }
 
@@ -1438,35 +1448,16 @@ int icpb_align_host_accept(icpb_handle h, const double *h_xy, const int64_t *h_o
                            const icpb_params *p, double accept_thresh, int64_t capacity, int64_t *n_accepted,
                            int64_t *h_rows, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes)
 {
-    if (!h || n_scans <= 0 || B <= 0 || !h_pairs) return fail(ICPB_EINVAL, "icpb_align_host_accept: bad argument%s");
-    if (!((h_xy && h_offsets) || (scan_xy && scan_len))) return fail(ICPB_EINVAL, "icpb_align_host_accept: no scans%s");
-    if ((init_ld != 6 && init_ld != 9) || (T_ld != 6 && T_ld != 9))
-        return fail(ICPB_EINVAL, "icpb_align_host_accept: init_ld / T_ld must be 6 or 9%s");
-    if (capacity < 1 || !n_accepted || !h_rows || !h_T || !h_err || !h_passes || isnan(accept_thresh))
-        return fail(ICPB_EINVAL, "icpb_align_host_accept: bad output arguments%s");
-    int rc = check_params(p, B);
+    int rc = align_check(h, n_scans, h_pairs, init_ld, B, p, h_T, T_ld, h_err, h_passes, nullptr);
     if (rc) return rc;
-    if (p->pair_mode != 0 || p->hist_cap > 0 || p->corr_stride > 0)
-        return fail(ICPB_EINVAL, "icpb_align_host_accept: explicit pairs, no history/correspondences%s");
-    if (B >= (int64_t(1) << 31)) return fail(ICPB_EINVAL, "icpb_align_host_accept: at most 2^31 - 1 pairs per call%s");
-    AcceptHost acc = {accept_thresh, capacity, n_accepted, h_rows, h_T, T_ld, h_err, h_passes};
+    if (B == 0) return fail(ICPB_EINVAL, "icpb_align_host_accept: bad argument%s");
+    if (capacity < 1 || !n_accepted || !h_rows || isnan(accept_thresh))
+        return fail(ICPB_EINVAL, "icpb_align_host_accept: bad output arguments%s");
     TableSrc src;
     std::vector<int64_t> offsets;
     int64_t longest = 0;
-    if (h_xy) {
-        if ((rc = validate_offsets(h_offsets, n_scans, &longest))) return rc;
-        src.xy = h_xy; src.offsets = h_offsets;
-    } else {
-        offsets.resize((size_t)n_scans + 1);
-        offsets[0] = 0;
-        for (int64_t sc = 0; sc < n_scans; ++sc) {
-            if (!scan_xy[sc] || scan_len[sc] <= 0)
-                return fail(ICPB_EINVAL, "empty scan in the list (the reference's argmin raises on it)%s");
-            offsets[(size_t)sc + 1] = offsets[(size_t)sc] + scan_len[sc];
-            if (scan_len[sc] > longest) longest = scan_len[sc];
-        }
-        src.scan_xy = scan_xy; src.offsets = offsets.data();
-    }
+    if ((rc = table_src(h_xy, h_offsets, scan_xy, scan_len, n_scans, offsets, &src, &longest))) return rc;
+    AcceptHost acc = {accept_thresh, capacity, n_accepted, h_rows, h_T, T_ld, h_err, h_passes};
     return align_impl(h, src, n_scans, longest, h_pairs, h_init, init_ld, B, p, nullptr, T_ld, nullptr, nullptr,
                       nullptr, &acc);
 }
@@ -1838,9 +1829,8 @@ int icpb_get_kernel_info(icpb_handle h, int64_t B, icpb_kernel_info *out)
     LaunchCfg cfg;
     int rc = make_cfg(h, h->longest, B > 0 ? B : (int64_t)1 << 40, &cfg, nullptr, h->tune_large == 1);
     if (rc) return rc;
-    const kernel_fn fn = cfg.big ? big_kernel(nullptr) : pick_kernel(nullptr);
     cudaFuncAttributes fa;
-    CU(cudaFuncGetAttributes(&fa, fn));
+    CU(cudaFuncGetAttributes(&fa, align_kernel(cfg.big, false, false)));
     int64_t grid = (int64_t)cfg.ctas_per_sm * h->sm_count;
     if (B > 0 && grid > B) grid = B;
     out->threads_per_cta = cfg.threads; out->ctas_per_sm = cfg.ctas_per_sm; out->sm_count = h->sm_count;

@@ -301,6 +301,35 @@ def test_mixed_table_align_accept(eng, mixed_case):
         np.testing.assert_array_equal(acc.iters, full.iters[keep])
 
 
+def test_mixed_table_rerun_after_missing_counter(gicp, eng, mixed_case, mixed_ref):
+    """The streaming rerun of a split batch: when the arrival counter never moves, the CTAs of both
+    launches give up after ~0.5 s and the library reruns both parts on the resident table, with the
+    results of a call that did not have to."""
+    _, mixed, _, _, all_pairs, all_init, short_rows = mixed_case
+    n0 = eng.launch_count
+    ref = eng.align(gicp.ScanTable(mixed), all_pairs, all_init, epsilon=0.05)
+    assert eng.launch_count - n0 == 2                       # one launch per part
+    thresh = float(np.median(ref.error))
+    rows_ref, acc_ref = eng.align_accept(mixed, all_pairs, thresh, all_init, epsilon=0.05)
+    eng.set_tuning("drop_counter", 1)
+    try:
+        n0 = eng.launch_count
+        got = eng.align(gicp.ScanTable(mixed), all_pairs, all_init, epsilon=0.05)
+        assert eng.launch_count - n0 == 4                   # both parts, then both again
+        rows, acc = eng.align_accept(mixed, all_pairs, thresh, all_init, epsilon=0.05)
+    finally:
+        eng.set_tuning("drop_counter", 0)
+    _check_mixed(got, mixed_ref, short_rows)
+    np.testing.assert_array_equal(got.T, ref.T)
+    np.testing.assert_array_equal(got.error, ref.error)
+    np.testing.assert_array_equal(got.iters, ref.iters)
+    assert 0 < len(rows_ref) < len(all_pairs)
+    np.testing.assert_array_equal(rows, rows_ref)
+    np.testing.assert_array_equal(acc.T, acc_ref.T)
+    np.testing.assert_array_equal(acc.error, acc_ref.error)
+    np.testing.assert_array_equal(acc.iters, acc_ref.iters)
+
+
 @pytest.mark.parametrize("n_peers", [1, 5])
 def test_mixed_table_fused_gather(eng, mixed_case, mixed_ref, n_peers):
     import torch
