@@ -170,10 +170,11 @@ struct PackJob {
     int64_t n_jobs;
     std::atomic<int64_t> next{0};
     std::atomic<int32_t> *done;         // per piece
-    std::atomic<uint64_t> bad{0};       // non-finite coordinate seen
+    std::atomic<uint64_t> bad{0};       // a coordinate beyond ICPB_MAX_COORD (or NaN) seen
 };
 
-// One scan into the pinned staging table with NON-TEMPORAL stores, checking for inf / NaN on the way.
+// One scan into the pinned staging table with NON-TEMPORAL stores, checking on the way that every
+// coordinate is within ICPB_MAX_COORD (!(|v| <= bound): NaN fails too).
 // Ordinary stores leave the freshly written lines dirty in the writing core's private cache; the
 // copy engine's reads then have to snoop them out of cores that have already gone idle, and the
 // last pieces of the table -- the ones still cache resident when the packing ends -- crawl at
@@ -184,34 +185,28 @@ static inline uint64_t copy_scan(double *dst, const double *src, int64_t n_doubl
 {
     uint64_t bad = 0;
 #if defined(__x86_64__)
-    const __m128i expo = _mm_set_epi32(0x7ff00000, 0, 0x7ff00000, 0);       // exponent bits of both doubles
-    __m128i acc = _mm_setzero_si128();
+    const __m128d sign = _mm_set1_pd(-0.0), lim = _mm_set1_pd(ICPB_MAX_COORD);
+    // not (|v| <= lim): the unordered compare is true for NaN
+    auto out = [&](__m128d v) { return _mm_cmpnle_pd(_mm_andnot_pd(sign, v), lim); };
+    __m128d acc = _mm_setzero_pd();
     int64_t k = 0;
     for (; k + 8 <= n_doubles; k += 8) {                                    // one 64-byte line per trip
         const __m128d a = _mm_loadu_pd(src + k), b = _mm_loadu_pd(src + k + 2);
         const __m128d c = _mm_loadu_pd(src + k + 4), d = _mm_loadu_pd(src + k + 6);
         _mm_stream_pd(dst + k, a); _mm_stream_pd(dst + k + 2, b);
         _mm_stream_pd(dst + k + 4, c); _mm_stream_pd(dst + k + 6, d);
-        // all-ones exponent = inf or NaN: compare the high words, ignore the low ones
-        const __m128i ea = _mm_cmpeq_epi32(_mm_and_si128(_mm_castpd_si128(a), expo), expo);
-        const __m128i eb = _mm_cmpeq_epi32(_mm_and_si128(_mm_castpd_si128(b), expo), expo);
-        const __m128i ec = _mm_cmpeq_epi32(_mm_and_si128(_mm_castpd_si128(c), expo), expo);
-        const __m128i ed = _mm_cmpeq_epi32(_mm_and_si128(_mm_castpd_si128(d), expo), expo);
-        acc = _mm_or_si128(acc, _mm_or_si128(_mm_or_si128(ea, eb), _mm_or_si128(ec, ed)));
+        acc = _mm_or_pd(acc, _mm_or_pd(_mm_or_pd(out(a), out(b)), _mm_or_pd(out(c), out(d))));
     }
     for (; k + 2 <= n_doubles; k += 2) {
         const __m128d a = _mm_loadu_pd(src + k);
         _mm_stream_pd(dst + k, a);
-        acc = _mm_or_si128(acc, _mm_cmpeq_epi32(_mm_and_si128(_mm_castpd_si128(a), expo), expo));
+        acc = _mm_or_pd(acc, out(a));
     }
-    // the low words compare equal trivially (0 == 0): keep the high words only
-    const __m128i hi = _mm_and_si128(acc, _mm_set_epi32(-1, 0, -1, 0));
-    bad = (uint64_t)(_mm_movemask_epi8(hi) != 0);
+    bad = (uint64_t)(_mm_movemask_pd(acc) != 0);
 #else
     memcpy(dst, src, sizeof(double) * (size_t)n_doubles);
-    const uint64_t *u = (const uint64_t *)dst;
     for (int64_t k = 0; k < n_doubles; ++k)
-        bad |= (uint64_t)((u[k] & 0x7ff0000000000000ULL) == 0x7ff0000000000000ULL);
+        bad |= (uint64_t)!(fabs(dst[k]) <= ICPB_MAX_COORD);
 #endif
     return bad;
 }
@@ -1149,13 +1144,14 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
             if (!(m[6] == 0.0 && m[7] == 0.0 && m[8] == 1.0))
                 return fail(ICPB_EINVAL, "transform bottom row must be [0, 0, 1] (an SE(2) matrix)%s");
         }
-        uint64_t bad = 0;                                     // all-ones exponent = inf or NaN; integer test, vectorises
-        for (int64_t k = 0; k < (int64_t)init_ld * B; ++k) {
-            uint64_t u;
-            memcpy(&u, h_init + k, sizeof u);
-            bad |= (uint64_t)((u & 0x7ff0000000000000ULL) == 0x7ff0000000000000ULL);
+        bool bad = false;                                     // !(|v| <= bound): NaN fails too
+        for (int64_t b = 0; b < B; ++b) {
+            const double *m = h_init + (int64_t)init_ld * b;
+            bad |= !(fabs(m[0]) <= ICPB_MAX_GUESS_LINEAR) | !(fabs(m[1]) <= ICPB_MAX_GUESS_LINEAR) |
+                   !(fabs(m[3]) <= ICPB_MAX_GUESS_LINEAR) | !(fabs(m[4]) <= ICPB_MAX_GUESS_LINEAR) |
+                   !(fabs(m[2]) <= ICPB_MAX_GUESS_SHIFT) | !(fabs(m[5]) <= ICPB_MAX_GUESS_SHIFT);
         }
-        if (bad) return fail(ICPB_EINVAL, "transform holds non-finite values%s");
+        if (bad) return fail(ICPB_EINVAL, "transform holds non-finite values or values beyond the bounds of icpb.h%s");
     }
     // ---- from here on the handle's table is being replaced: a failure leaves it without one ----
     h->prep_for = nullptr; h->xy = nullptr; h->offsets = nullptr; h->n_scans = 0; h->longest = 0;
@@ -1163,7 +1159,7 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     if (B == 0) {                                             // upload only
         if (src.scan_xy) pack_run(&job);
         packers.finish();                                     // before job.bad is read
-        if (src.scan_xy && job.bad.load()) return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates%s"));
+        if (src.scan_xy && job.bad.load()) return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates or coordinates beyond ICPB_MAX_COORD%s"));
         CUA(cudaMemcpyAsync(h->own_xy.p, up_xy, nb_xy, cudaMemcpyHostToDevice, cp));
         CUA(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, cp));
         CUA(cudaStreamSynchronize(cp));
@@ -1291,7 +1287,7 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     if (bad_scans) {
         // the kernel is waiting for pieces that will not come: raise its give-up flag, drain, report
         CUA(cudaMemcpyAsync(d_passes + B, h->seg_vals_pinned + 1, sizeof(int32_t), cudaMemcpyHostToDevice, cp));
-        return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates%s"));
+        return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates or coordinates beyond ICPB_MAX_COORD%s"));
     }
     CUA(cudaEventRecord(h->done_ev[0], cs));
     CUA(cudaStreamWaitEvent(cp, h->done_ev[0], 0));

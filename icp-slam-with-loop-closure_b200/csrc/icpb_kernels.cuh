@@ -28,7 +28,8 @@
 namespace icpb {
 
 constexpr int   kChunk    = 16;        // targets per bookkeeping chunk
-constexpr float kPadCoord = 1.0e15f;   // coordinates of padding targets (distance ~2e30, never a candidate)
+constexpr float kPadCoord = 1.0e15f;   // coordinates of padding targets (distance ~2e30, never a candidate
+                                       // for inputs within ICPB_MAX_COORD: DESIGN.md section 4)
 constexpr int   kMaxWarps = 32;
 constexpr int   kNumSums  = 8;        // 7 fp64 sums per reduction tile (+1 pad): see kS* below
 // columns of a tile's partial sums (a = moved source point - c, b = matched target - g):
@@ -410,16 +411,26 @@ __device__ __forceinline__ void dist32x4_minus(float px, float py, float nthr, c
     }
 }
 
-// Largest singular value of the linear part of T (a bound on how much T stretches a distance), as
-// a float with a safety factor.  1 for the rigid transforms ICP composes; the caller's initial
-// guess may be any affine map with bottom row [0 0 1].
+// Largest singular value of the linear part [a b; c d] of T (a bound on how much T stretches a
+// distance), with a safety factor.  1 for the rigid transforms ICP composes; the caller's initial
+// guess may be any affine map with bottom row [0 0 1] within the bounds of include/icpb.h (the passes
+// keep its singular values: they only compose rotations onto it).
+// sigma_max = (hypot(a + d, c - b) + hypot(a - d, c + b)) / 2 adds two non-negative terms, so unlike
+// sqrt((f2 + sqrt(f2^2 - 4 det^2)) / 2) it does not cancel (in fp32 that form underestimates a
+// near-conformal map such as R diag(1 + 5e-4, 1) R' by 2.5e-4 relative, more than the chunk test's
+// slack).  In fp32 each sum or difference is off by at most 3u sigma_max (u = 2^-24; every entry is
+// <= sigma_max), each root by at most 8u sigma_max, so the estimate is >= (1 - 5e-7) sigma_max and the
+// factor 1.00002 still leaves the 1e-5 that the fp32 roundings of the radius in the caller need.
+// Below ~1e-18 the fp32 squares underflow; there 2 max|entry| (>= the Frobenius norm >= sigma_max)
+// is the bound, and below fp32's range the 1e-30 floor is.  One lane, once per pass.
 __device__ __forceinline__ double stretch_of(const double *T)
 {
     const float a = (float)T[0], b = (float)T[1], c = (float)T[3], d = (float)T[4];
-    const float f2 = a * a + b * b + c * c + d * d;
-    const float det = a * d - b * c;
-    const float disc = fmaxf(f2 * f2 - 4.0f * det * det, 0.0f);
-    return (double)(sqrtf(0.5f * (f2 + sqrtf(disc))) * 1.00002f + 1e-30f);
+    const float p = a + d, q = c - b, r = a - d, t = c + b;
+    float s = 0.5f * (sqrtf(p * p + q * q) + sqrtf(r * r + t * t));
+    const float m = fmaxf(fmaxf(fabsf(a), fabsf(b)), fmaxf(fabsf(c), fabsf(d)));
+    if (m < 1e-18f) s = fmaxf(s, 2.0f * m);
+    return (double)(s * 1.00002f + 1e-30f);
 }
 
 // PRUNE = false: exhaustive sweep over every chunk (the reference's brute force; used for the

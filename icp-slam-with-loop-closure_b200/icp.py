@@ -31,6 +31,17 @@ __all__ = ["icp", "icp_iteration", "icp_batch", "get_correspondences", "get_clos
            "ScanTable", "ScanList", "IcpEngine", "BatchResult", "engine", "make_epilogue"]
 
 
+# Input magnitudes the kernel is exact for (include/icpb.h: ICPB_MAX_COORD, ICPB_MAX_GUESS_LINEAR,
+# ICPB_MAX_GUESS_SHIFT).  `not (abs(v) <= bound)` is also true for NaN.
+MAX_COORD = 1e10
+MAX_GUESS_LINEAR = 1e3
+MAX_GUESS_SHIFT = 1e12
+
+
+def _coords_ok(xy) -> bool:
+    return bool((np.abs(xy) <= MAX_COORD).all())
+
+
 # --------------------------------------------------------------------------- scan table
 class ScanTable:
     """The reference's ``lidar_points`` (a list of (m_i, 2) float64 arrays,
@@ -57,8 +68,8 @@ class ScanTable:
             if self.offsets.ndim != 1 or len(self.offsets) < 2 or self.offsets[0] != 0 \
                     or self.offsets[-1] != len(self.xy) or np.any(np.diff(self.offsets) <= 0):
                 raise ValueError("offsets must start at 0, end at len(xy) and be strictly increasing")
-        if not np.isfinite(self.xy).all():
-            raise ValueError("scan table holds non-finite coordinates")
+        if not _coords_ok(self.xy):
+            raise ValueError(f"scan table holds non-finite coordinates or coordinates beyond +-{MAX_COORD:g}")
 
     @classmethod
     def from_lengths(cls, lengths) -> "ScanTable":
@@ -110,8 +121,9 @@ def _to6(T) -> np.ndarray:
         raise ValueError(f"transform has shape {T.shape}; expected (..., 3, 3)")
     if not (np.all(T[..., 2, 0] == 0) and np.all(T[..., 2, 1] == 0) and np.all(T[..., 2, 2] == 1)):
         raise ValueError("transform bottom row must be [0, 0, 1] (an SE(2) matrix)")
-    if not np.isfinite(T).all():
-        raise ValueError("transform holds non-finite values")
+    if not (np.all(np.abs(T[..., :2, :2]) <= MAX_GUESS_LINEAR) and np.all(np.abs(T[..., :2, 2]) <= MAX_GUESS_SHIFT)):
+        raise ValueError(f"transform holds non-finite values or values beyond the bounds of include/icpb.h "
+                         f"(|linear part| <= {MAX_GUESS_LINEAR:g}, |translation| <= {MAX_GUESS_SHIFT:g})")
     return np.ascontiguousarray(T[..., :2, :].reshape(T.shape[:-2] + (6,)))
 
 
@@ -527,8 +539,8 @@ def _cloud_xy(pc, name: str) -> np.ndarray:
     if not np.all(pc[:, 2] == 1.0):
         raise ValueError(f"{name}: the homogeneous column must be all ones")
     xy = np.ascontiguousarray(pc[:, :2])
-    if not np.isfinite(xy).all():
-        raise ValueError(f"{name} holds non-finite coordinates")
+    if not _coords_ok(xy):
+        raise ValueError(f"{name} holds non-finite coordinates or coordinates beyond +-{MAX_COORD:g}")
     return xy
 
 

@@ -36,6 +36,24 @@ extern "C" {
                                  scans that do not fit shared memory run on the large-scan variant */
 #define ICPB_ENOSCANS 10003   /* run called before a scan table was set                       */
 
+/* Input magnitudes.  The alignment kernel pads target arrays with points at (1e15, 1e15) and filters
+ * in fp32; within these bounds every moved source point stays below 6e13 in every pass, so a real
+ * target is always far nearer than any padding point (squared distances <= 7e27 against >= 1.7e30)
+ * and no fp32 square overflows (DESIGN.md section 4 has the arithmetic).  The results are exact for
+ * every input within them:
+ *   - scan coordinates:                      |x|, |y| <= ICPB_MAX_COORD;
+ *   - the linear part of an initial guess:   |r00|, |r01|, |r10|, |r11| <= ICPB_MAX_GUESS_LINEAR
+ *     (any affine map: shear, reflection, rank-deficient and zero linear parts included);
+ *   - the translation of an initial guess:   |tx|, |ty| <= ICPB_MAX_GUESS_SHIFT.
+ * A coordinate or guess outside them (NaN and inf included) is rejected with ICPB_EINVAL where the
+ * library reads the values on the host: scans by icpb_align_host_scans (and the list form of
+ * icpb_align_host_accept) while packing, guesses by the icpb_align_host* calls before anything runs.
+ * The Python layer checks every entry point.  Entry points that take device buffers, and the packed
+ * tables of the host calls, take the caller's word for it. */
+#define ICPB_MAX_COORD        1e10
+#define ICPB_MAX_GUESS_LINEAR 1e3
+#define ICPB_MAX_GUESS_SHIFT  1e12
+
 /* icpb_params.flags: sweep every target for every source point (the reference's brute force,
  * src/icp.py:10-19) instead of skipping target chunks that provably cannot hold a nearest
  * neighbour.  Results are identical either way; the flag exists to measure the FP32-pipe
@@ -185,7 +203,8 @@ int icpb_plan_upload(const int64_t *h_offsets, int64_t n_scans, int32_t pieces_w
 /* The same with the transforms in the caller's own layout: init_ld / T_ld = 9 reads and writes the
  * reference's full 3x3 row-major matrices (what scripts/main.py:244 passes and src/icp.py:97
  * returns; the bottom row is checked to be [0, 0, 1] on the way in and written on the way out),
- * 6 the packed top two rows.  Non-finite initial guesses are rejected (ICPB_EINVAL). */
+ * 6 the packed top two rows.  Initial guesses beyond the bounds above (non-finite ones included) are
+ * rejected (ICPB_EINVAL). */
 int icpb_align_host_ld(icpb_handle h, const double *h_xy, const int64_t *h_offsets, int64_t n_scans,
                        const int32_t *h_pairs, const double *h_init, int32_t init_ld, int64_t B,
                        const icpb_params *p, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes);
@@ -200,8 +219,8 @@ int icpb_align_host_ex(icpb_handle h, const double *h_xy, const int64_t *h_offse
 /* The same with the scans exactly as the reference holds them: `lidar_points`, a list of n_scans
  * separate (m_i, 2) float64 C-ordered arrays in ordinary pageable memory (src/dataloader.py:110-112,
  * the arguments of scripts/main.py:242-243).  scan_xy[s] points at scan s, scan_len[s] = m_i.  A few
- * host threads copy the scans into a pinned staging table piece by piece (checking for non-finite
- * coordinates on the way: ICPB_EINVAL) while earlier pieces are already on their way to the device and
+ * host threads copy the scans into a pinned staging table piece by piece (checking that every
+ * coordinate is within ICPB_MAX_COORD on the way: ICPB_EINVAL) while earlier pieces are already on their way to the device and
  * the kernel is aligning the pairs whose scans have landed. */
 int icpb_align_host_scans(icpb_handle h, const double *const *scan_xy, const int64_t *scan_len, int64_t n_scans,
                           const int32_t *h_pairs, const double *h_init, int32_t init_ld, int64_t B,
