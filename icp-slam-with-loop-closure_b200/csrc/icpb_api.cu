@@ -1540,14 +1540,32 @@ static int upload_poses(icpb_handle h, const double *h_xy, const double *h_trave
     return 0;
 }
 
+// The input contract of the candidate kernels (include/icpb.h, ICPB_MAX_POSE_COORD): poses within the
+// bound (so no squared distance overflows), `travelled` finite and non-decreasing (upper_bound's binary
+// search), a min_dist_along_path that is not NaN (np.searchsorted and upper_bound disagree on NaN).
+static int proximity_check(const double *h_xy, const double *h_travelled, int64_t n, double min_dist_along_path,
+                           const char *who)
+{
+    if (min_dist_along_path != min_dist_along_path) return fail(ICPB_EINVAL, "%s: min_dist_along_path is NaN", who);
+    bool bad = false;
+    for (int64_t k = 0; k < 2 * n; ++k) bad |= !(fabs(h_xy[k]) <= ICPB_MAX_POSE_COORD);
+    if (bad) return fail(ICPB_EINVAL, "%s: pose coordinates are non-finite or beyond ICPB_MAX_POSE_COORD", who);
+    for (int64_t i = 0; i < n; ++i)
+        bad |= !isfinite(h_travelled[i]) || (i > 0 && h_travelled[i] < h_travelled[i - 1]);
+    if (bad) return fail(ICPB_EINVAL, "%s: travelled must be finite and non-decreasing", who);
+    return 0;
+}
+
 int icpb_proximity_closest(icpb_handle h, const double *h_xy, const double *h_travelled, int64_t n,
                            double min_dist_along_path, double max_dist, int32_t *h_closest, double *h_dist)
 {
     if (!h || !h_xy || !h_travelled || n <= 0 || n > 0x3fffffff || !h_closest || !h_dist)
         return fail(ICPB_EINVAL, "icpb_proximity_closest: bad argument%s");
+    int rc = proximity_check(h_xy, h_travelled, n, min_dist_along_path, "icpb_proximity_closest");
+    if (rc) return rc;
     ON_DEVICE(h);
     double *d_xy, *d_trav;
-    int rc = upload_poses(h, h_xy, h_travelled, n, &d_xy, &d_trav);
+    rc = upload_poses(h, h_xy, h_travelled, n, &d_xy, &d_trav);
     if (rc) return rc;
     if ((rc = h->s_passes.reserve(sizeof(int32_t) * (size_t)n))) return rc;
     if ((rc = h->s_err.reserve(sizeof(double) * (size_t)n))) return rc;
@@ -1569,9 +1587,11 @@ int icpb_proximity_pairs(icpb_handle h, const double *h_xy, const double *h_trav
     if (!h || !h_xy || !h_travelled || n <= 0 || n > 0x3fffffff || !n_pairs || capacity < 0 ||
         (capacity > 0 && !h_pairs))
         return fail(ICPB_EINVAL, "icpb_proximity_pairs: bad argument%s");
+    int rc = proximity_check(h_xy, h_travelled, n, min_dist_along_path, "icpb_proximity_pairs");
+    if (rc) return rc;
     ON_DEVICE(h);
     double *d_xy, *d_trav;
-    int rc = upload_poses(h, h_xy, h_travelled, n, &d_xy, &d_trav);
+    rc = upload_poses(h, h_xy, h_travelled, n, &d_xy, &d_trav);
     if (rc) return rc;
     if ((rc = h->s_T.reserve(sizeof(int64_t) * 2 * (size_t)n))) return rc;
     int64_t *d_count = (int64_t *)h->s_T.p, *d_off = d_count + n;
@@ -1713,9 +1733,28 @@ namespace {
 
 int grid_check(icpb_handle h, const double *h_poses, int64_t n, double cell_width, const char *who)
 {
-    if (!h || !h_poses || n <= 0 || !(cell_width > 0.0)) return fail(ICPB_EINVAL, "%s: bad argument", who);
+    if (!h || !h_poses || n <= 0 || !(cell_width > 0.0 && isfinite(cell_width)))
+        return fail(ICPB_EINVAL, "%s: bad argument", who);
     if (!h->xy) return fail(ICPB_ENOSCANS, "%s: no scan table set", who);
     if (n > h->n_scans) return fail(ICPB_EINVAL, "%s: more poses than scans in the table", who);
+    bool bad = false;
+    for (int64_t k = 0; k < 3 * n; ++k) bad |= !isfinite(h_poses[k]);
+    if (bad) return fail(ICPB_EINVAL, "%s: non-finite pose", who);
+    return 0;
+}
+
+// ICPB_MAX_GRID_CELL (include/icpb.h): every cell coordinate the walk can see -- the pose's and the beam
+// end's, |global| <= |pose| + sqrt(2) * ICPB_MAX_COORD -- is bounded from the host's data alone.
+int grid_cell_check(const double *h_poses, int64_t n, double min_x, double min_y, double cell_width)
+{
+    if (!isfinite(min_x) || !isfinite(min_y))
+        return fail(ICPB_EINVAL, "icpb_occupancy_grid_update: non-finite grid origin%s");
+    double p = 0.0;
+    for (int64_t i = 0; i < n; ++i) p = fmax(p, fmax(fabs(h_poses[3 * i]), fabs(h_poses[3 * i + 1])));
+    const double reach = (p + fmax(fabs(min_x), fabs(min_y)) + M_SQRT2 * ICPB_MAX_COORD) / cell_width;
+    if (!(reach <= ICPB_MAX_GRID_CELL))
+        return fail(ICPB_EINVAL, "icpb_occupancy_grid_update: cell coordinates could exceed ICPB_MAX_GRID_CELL "
+                                 "(poses or origin too far for this cell width)%s");
     return 0;
 }
 
@@ -1747,6 +1786,8 @@ int icpb_occupancy_grid_bounds(icpb_handle h, const double *h_poses, int64_t n, 
     int rc = grid_check(h, h_poses, n, cell_width, "icpb_occupancy_grid_bounds");
     if (rc) return rc;
     if (!min_x_out || !min_y_out || !height || !width) return fail(ICPB_EINVAL, "icpb_occupancy_grid_bounds: null output%s");
+    if (!isfinite(min_width) || !isfinite(min_height))
+        return fail(ICPB_EINVAL, "icpb_occupancy_grid_bounds: non-finite minimum size%s");
     ON_DEVICE(h);
     if ((rc = h->s_grid.reserve(sizeof(double) * 4 * (size_t)n + 4 * sizeof(unsigned long long)))) return rc;
     unsigned long long *d_mm = (unsigned long long *)h->s_grid.p;
@@ -1769,9 +1810,12 @@ int icpb_occupancy_grid_bounds(icpb_handle h, const double *h_poses, int64_t n, 
     double width_dist = max_x - min_x, height_dist = max_y - min_y;
     if (width_dist < min_width) { const double off = (min_width - width_dist) / 2; min_x -= off; width_dist = min_width; }
     if (height_dist < min_height) { const double off = (min_height - height_dist) / 2; min_y -= off; height_dist = min_height; }
+    const double w_cells = ceil(width_dist / cell_width), h_cells = ceil(height_dist / cell_width);
+    if (!(w_cells * h_cells <= (double)ICPB_MAX_GRID_CELLS))                 // NaN and inf too
+        return fail(ICPB_EINVAL, "icpb_occupancy_grid_bounds: the grid would exceed ICPB_MAX_GRID_CELLS cells%s");
     *min_x_out = min_x; *min_y_out = min_y;
-    *width = (int64_t)ceil(width_dist / cell_width);
-    *height = (int64_t)ceil(height_dist / cell_width);
+    *width = (int64_t)w_cells;
+    *height = (int64_t)h_cells;
     return 0;
 }
 
@@ -1782,11 +1826,12 @@ int icpb_occupancy_grid_update(icpb_handle h, const double *h_poses, int64_t n, 
     int rc = grid_check(h, h_poses, n, cell_width, "icpb_occupancy_grid_update");
     if (rc) return rc;
     if (!h_grid || height <= 0 || width <= 0 || height > 0x7fffffff || width > 0x7fffffff ||
-        height * width > ((int64_t)1 << 30))
+        height * width > ICPB_MAX_GRID_CELLS)
         return fail(ICPB_EINVAL, "icpb_occupancy_grid_update: bad grid%s");
     // the per-cell closed form needs a miss to leave a cell negative and a hit to leave it positive
     if (k_hit < 1 || k_hit > 127 || k_miss < 1 || k_miss > 127)
         return fail(ICPB_EINVAL, "icpb_occupancy_grid_update: kHitOdds and kMissOdds must be integers in 1..127%s");
+    if ((rc = grid_cell_check(h_poses, n, min_x, min_y, cell_width))) return rc;
     ON_DEVICE(h);
     // the beam order keys are 32 bit: 2 * (beam index + 1) + 1 must fit (2^31 - 2 beams)
     int64_t n_points = 0;

@@ -54,6 +54,27 @@ extern "C" {
 #define ICPB_MAX_GUESS_LINEAR 1e3
 #define ICPB_MAX_GUESS_SHIFT  1e12
 
+/* Occupancy grid (icpb_occupancy_grid_*).  The Bresenham walk runs in 64-bit integers on cell
+ * coordinates; with every |cell coordinate| <= ICPB_MAX_GRID_CELL = 2^60 a beam spans
+ * M = max(|dx|, |dy|) <= 2^61 cells, the walk's error term stays within 1.5 M and `2 * error` within
+ * 3 * 2^61 < 2^63, so the walk visits exactly the reference's cells (DESIGN.md section 4).  The update
+ * checks this on the host before anything runs, from the poses and the grid origin alone (a global
+ * beam end lies within sqrt(2) * ICPB_MAX_COORD of its pose):
+ *     (max |pose x|, |pose y| + max(|min_x|, |min_y|) + sqrt(2) * ICPB_MAX_COORD) / cell_width <= 2^60
+ * With coordinates of 1e10 m this rejects only cell widths below about 1.2e-8 m.  Non-finite poses,
+ * min_x, min_y, min_width, min_height and cell widths are rejected by both calls, and so is a grid of
+ * more than ICPB_MAX_GRID_CELLS cells: icpb_occupancy_grid_bounds reports it before a caller
+ * allocates one. */
+#define ICPB_MAX_GRID_CELL  1152921504606846976.0   /* 2^60 */
+#define ICPB_MAX_GRID_CELLS 1073741824LL            /* 2^30: height * width */
+
+/* Loop-closure candidates (icpb_proximity_*).  Pose coordinates |x|, |y| <= ICPB_MAX_POSE_COORD keep
+ * every squared distance below 8e24, far from overflow, so every row with a candidate range finds its
+ * nearest pose.  Both calls reject with ICPB_EINVAL: a pose outside the bound (NaN and inf included),
+ * a `travelled` array that is not finite and non-decreasing (the row start is a binary search in it),
+ * and a NaN min_dist_along_path. */
+#define ICPB_MAX_POSE_COORD 1e12
+
 /* icpb_params.flags: sweep every target for every source point (the reference's brute force,
  * src/icp.py:10-19) instead of skipping target chunks that provably cannot hold a nearest
  * neighbour.  Results are identical either way; the flag exists to measure the FP32-pipe
@@ -261,7 +282,8 @@ int icpb_fit_pairs_host(icpb_handle h, const double *h_a_xy, const double *h_b_x
  * cumulative sum of consecutive distances, first entry 0).  For every pose i, start =
  * searchsorted(travelled, travelled[i] + min_dist_along_path, "right") (:18); h_closest[i] is
  * start + argmin(dist[i, start:]) (:21) if that distance is <= max_dist (:22), else -1 (also
- * when start is past the end, where the reference stops, :19-20).
+ * when start is past the end, where the reference stops, :19-20).  Inputs are checked against
+ * ICPB_MAX_POSE_COORD and the rules beside it before anything runs.
  */
 int icpb_proximity_closest(icpb_handle h, const double *h_xy, const double *h_travelled, int64_t n,
                            double min_dist_along_path, double max_dist, int32_t *h_closest, double *h_dist);
@@ -320,6 +342,8 @@ int icpb_pose_graph_sgd(icpb_handle h, double *h_poses, int64_t n, const int32_t
  *   (height x width int8, row 0 at min_y, C order), in place.  Bit-identical to the reference's
  *   sequential loops, including its int8 wrap-around at :109 and :128 (see csrc/icpb_grid.cuh).
  *   kHitOdds and kMissOdds must be integers in 1..127.
+ * Both calls check their inputs against ICPB_MAX_GRID_CELL / ICPB_MAX_GRID_CELLS (above) and return
+ * ICPB_EINVAL before anything runs; a rejected update leaves h_grid untouched.
  */
 int icpb_occupancy_grid_bounds(icpb_handle h, const double *h_poses, int64_t n, double cell_width,
                                double min_width, double min_height, double *min_x, double *min_y,

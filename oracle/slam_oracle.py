@@ -110,3 +110,22 @@ def proximity_candidates_ref(poses, min_dist_along_path=2, max_dist=1):
             out.append((i, j))
     out.reverse()
     return np.asarray(out, dtype=np.int64).reshape(-1, 2)
+
+
+def proximity_pairs_ref(poses, min_dist_along_path=2, max_dist=1):
+    """Every pair the rows of src/loop_closure_detection.py:12-25 consider, kept if within max_dist:
+    (source = j, target = i) int32 rows ordered by i then j, with cdist's rounding
+    sqrt((dx*dx) + (dy*dy)) -- np.hypot rounds differently in about one entry in six."""
+    xy = np.asarray(poses, dtype=np.float64)[:, :2]
+    n = len(xy)
+    step = np.sqrt((xy[1:, 0] - xy[:-1, 0]) ** 2 + (xy[1:, 1] - xy[:-1, 1]) ** 2)
+    travelled = np.concatenate(([0.0], np.cumsum(step)))
+    out = []
+    for i in range(n):
+        j0 = int(np.searchsorted(travelled, travelled[i] + min_dist_along_path, side="right"))
+        if j0 >= n:
+            break
+        dx, dy = xy[j0:, 0] - xy[i, 0], xy[j0:, 1] - xy[i, 1]
+        js = j0 + np.nonzero(np.sqrt(dx * dx + dy * dy) <= max_dist)[0]
+        out.append(np.stack((js, np.full_like(js, i)), axis=1))
+    return np.concatenate(out).astype(np.int32) if out else np.zeros((0, 2), np.int32)

@@ -71,7 +71,8 @@ def test_image_match_call_site():
 
 def test_candidate_generation_on_gpu():
     """icpb_proximity_closest / icpb_proximity_pairs against the numpy restatement of
-    src/loop_closure_detection.py:12-25 and against synth.proximity_pairs, on a 5,000-pose loop."""
+    src/loop_closure_detection.py:12-25 and against its every-pair form (slam_oracle.proximity_pairs_ref,
+    cdist's rounding), on a 5,000-pose loop."""
     from icp_slam_b200 import callers, synth
     from oracle import slam_oracle
     z, _ = load()
@@ -83,7 +84,7 @@ def test_candidate_generation_on_gpu():
         np.testing.assert_array_equal(callers.proximity_candidates(poses, **kw),
                                       slam_oracle.proximity_candidates_ref(poses, **kw))
     got = callers.proximity_pairs(poses)
-    want = synth.proximity_pairs(poses)
+    want = slam_oracle.proximity_pairs_ref(poses)
     np.testing.assert_array_equal(got, want)
     assert len(got) > 100000
 

@@ -56,3 +56,53 @@ def test_chain_composition_matches_reference():
     for i in range(1, n):
         poses[i] = synth.mat_to_pose(synth.pose_to_mat(poses[i - 1]) @ T[i - 1])
     np.testing.assert_allclose(poses, z["corrected"], atol=1e-9)
+
+
+def _detect_proximity_cdist(poses, min_dist_along_path=2, max_dist=1):
+    """src/loop_closure_detection.py:12-25 written out with scipy's cdist, as the reference does:
+    (candidates in its processing order, every pair within the radius as (j, i) rows)."""
+    from scipy.spatial.distance import cdist
+    positions = np.asarray(poses, dtype=np.float64)[:, :2]
+    steps = np.sqrt((positions[1:, 0] - positions[:-1, 0]) ** 2 + (positions[1:, 1] - positions[:-1, 1]) ** 2)
+    dist_traveled = np.concatenate(([0.0], np.cumsum(steps)))
+    dists = cdist(positions, positions)
+    matches, pairs = [], []
+    for i in range(len(positions)):
+        start = np.searchsorted(dist_traveled, dist_traveled[i] + min_dist_along_path, side="right")
+        if start >= len(positions):
+            break
+        j = start + np.argmin(dists[i, start:])
+        if dists[i, j] <= max_dist:
+            matches.append((i, j))
+        pairs += [(jj, i) for jj in range(start, len(positions)) if dists[i, jj] <= max_dist]
+    matches.reverse()
+    return (np.asarray(matches, dtype=np.int64).reshape(-1, 2), np.asarray(pairs, dtype=np.int32).reshape(-1, 2))
+
+
+def boundary_poses(rng, n=300, scale=3.0):
+    """A wandering path that stops (runs of identical poses: travelled has plateaus, distances tie)
+    and revisits 3-4-5 offsets of earlier poses, so distances sit exactly on radius 5."""
+    p = np.cumsum(rng.normal(0, scale / 10, (n, 2)), axis=0)
+    p[40:60] = p[40]
+    p[100:104] = p[3] + (3.0, 4.0)
+    p[150] = p[3] + (-4.0, 3.0)
+    p = np.round(p * 64) / 64                                 # exact binary fractions: exact ties
+    return np.c_[p, rng.uniform(-np.pi, np.pi, n)]
+
+
+def test_proximity_refs_equal_a_literal_cdist_implementation():
+    from icp_slam_b200 import synth
+    from oracle import slam_oracle
+    rng = np.random.default_rng(8)
+    cases = [(rng.normal(0, 3, (400, 3)), 2, 1), (boundary_poses(rng), 2, 5.0), (boundary_poses(rng), 0.0, 5.0),
+             (boundary_poses(rng), -1.0, 0.0), (boundary_poses(rng), np.inf, 5.0), (boundary_poses(rng), 3, np.inf),
+             (synth.loop_trajectory(600, step=0.05), 2, 1), (rng.normal(0, 3, (1, 3)), 0, 1)]
+    for poses, mdp, md in cases:
+        cand, pairs = _detect_proximity_cdist(poses, mdp, md)
+        np.testing.assert_array_equal(slam_oracle.proximity_candidates_ref(poses, mdp, md), cand)
+        np.testing.assert_array_equal(slam_oracle.proximity_pairs_ref(poses, mdp, md), pairs)
+    # on the boundary family the radius is met exactly, and hypot would round some pairs differently
+    poses = boundary_poses(np.random.default_rng(9))
+    _, pairs = _detect_proximity_cdist(poses, 2, 5.0)
+    d = np.sqrt(((poses[pairs[:, 0], :2] - poses[pairs[:, 1], :2]) ** 2).sum(1))
+    assert (d == 5.0).sum() >= 5
