@@ -13,7 +13,6 @@
 #include <thread>
 #include <mutex>
 #include <condition_variable>
-#include <time.h>
 #include <sched.h>
 #if defined(__x86_64__)
 #include <emmintrin.h>
@@ -93,14 +92,6 @@ struct DevBuf {
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
 
-// host clock in microseconds (ICPB_TRACE timings of the host entry points)
-static double now_us()
-{
-    timespec ts;
-    clock_gettime(CLOCK_MONOTONIC, &ts);
-    return ts.tv_sec * 1e6 + ts.tv_nsec * 1e-3;
-}
-
 struct PinnedBuf {
     void *p = nullptr;
     size_t cap = 0;
@@ -167,7 +158,7 @@ struct PackJob {
     double *dst;                        // pinned staging
     const int64_t *job_first, *job_last;  // scans [first, last) of job j
     const int32_t *job_piece;           // upload piece of job j
-    int64_t n_jobs;
+    int64_t n_jobs = 0;
     std::atomic<int64_t> next{0};
     std::atomic<int32_t> *done;         // per piece
     std::atomic<uint64_t> bad{0};       // a coordinate beyond ICPB_MAX_COORD (or NaN) seen
@@ -211,22 +202,18 @@ static inline uint64_t copy_scan(double *dst, const double *src, int64_t n_doubl
     return bad;
 }
 
-static void pack_run(PackJob *job)
+static void pack_one(PackJob *job, int64_t j)
 {
-    for (;;) {
-        const int64_t j = job->next.fetch_add(1, std::memory_order_relaxed);
-        if (j >= job->n_jobs) break;
-        uint64_t bad = 0;
-        for (int64_t s = job->job_first[j]; s < job->job_last[j]; ++s) {
-            const int64_t o = job->offsets[s], m = job->offsets[s + 1] - o;
-            bad |= copy_scan(job->dst + 2 * o, job->scan_xy[s], 2 * m);
-        }
-#if defined(__x86_64__)
-        _mm_sfence();                                   // the streamed lines are in memory before the piece is announced
-#endif
-        if (bad) job->bad.fetch_or(1, std::memory_order_relaxed);
-        job->done[job->job_piece[j]].fetch_add(1, std::memory_order_release);
+    uint64_t bad = 0;
+    for (int64_t s = job->job_first[j]; s < job->job_last[j]; ++s) {
+        const int64_t o = job->offsets[s], m = job->offsets[s + 1] - o;
+        bad |= copy_scan(job->dst + 2 * o, job->scan_xy[s], 2 * m);
     }
+#if defined(__x86_64__)
+    _mm_sfence();                                       // the streamed lines are in memory before the piece is announced
+#endif
+    if (bad) job->bad.fetch_or(1, std::memory_order_relaxed);
+    job->done[job->job_piece[j]].fetch_add(1, std::memory_order_release);
 }
 
 struct PackPool {
@@ -252,7 +239,7 @@ struct PackPool {
                         seen = generation;
                         j = job;
                     }
-                    pack_run(j);
+                    for (int64_t i; (i = j->next.fetch_add(1, std::memory_order_relaxed)) < j->n_jobs;) pack_one(j, i);
                     {
                         std::lock_guard<std::mutex> lk(mu);
                         --running;
@@ -284,21 +271,6 @@ struct PackPool {
         cv.notify_all();
         for (auto &w : workers) w.join();
     }
-};
-
-// The workers of a PackPool write through a PackJob on the dispatching call's stack frame: this guard,
-// declared after the job and what it points to, stops them on every way out of that call.
-struct PackGuard {
-    PackJob *job = nullptr;                             // set while workers may be running it
-    PackPool *pool = nullptr;
-    void finish()                                       // hand out no more jobs, wait for the workers
-    {
-        if (!job) return;
-        job->next.store(job->n_jobs, std::memory_order_relaxed);
-        if (pool) pool->finish();
-        job = nullptr;
-    }
-    ~PackGuard() { finish(); }
 };
 
 }  // namespace
@@ -342,10 +314,29 @@ struct icpb_ctx {
     PackPool *pool = nullptr;                       // host threads that pack scans into stage_xy
     // tuning / test hooks (icpb_set_tuning); 0 or -1 = the library's own choice
     int tune_threads = 0, tune_cluster = -1, tune_segments = 0, tune_pack_threads = 0, tune_large = -1;
-    bool tune_flag_copy = false, tune_drop_counter = false, tune_trace = false;
+    bool tune_drop_counter = false;
 };
 
 namespace {
+
+// The handle's scan table; a new table has no staging images yet (ensure_prep).
+void set_table(icpb_ctx *h, const double *xy, const int64_t *off, int64_t n_scans, int64_t longest)
+{
+    h->prep_for = nullptr; h->xy = xy; h->offsets = off; h->n_scans = n_scans; h->longest = longest;
+}
+
+void drop_table(icpb_ctx *h) { set_table(h, nullptr, nullptr, 0, 0); }
+
+// A whole table from host memory into the handle's own buffers (reserved by the caller), which then hold
+// the handle's table.
+int upload_table(icpb_ctx *h, const double *xy, const int64_t *off, int64_t n_scans, int64_t longest)
+{
+    CU(cudaMemcpyAsync(h->own_xy.p, xy, sizeof(double) * 2 * (size_t)off[n_scans], cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->own_off.p, off, sizeof(int64_t) * (size_t)(n_scans + 1), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    set_table(h, (const double *)h->own_xy.p, (const int64_t *)h->own_off.p, n_scans, longest);
+    return 0;
+}
 
 // Launch geometry for a batch whose longest scan has `longest` points.  When the layout does not fit
 // one CTA's shared memory (or `big` asks for it) the launch uses the large-scan variant.
@@ -466,6 +457,15 @@ int run_check(const icpb_ctx *h, const icpb_params *p, int64_t B, bool empty_ok,
     if (p->corr_stride > 0 && !corr) return fail(ICPB_EINVAL, "corr_stride > 0 without a correspondence buffer%s");
     if (p->corr_stride > 0 && p->corr_stride < h->longest)
         return fail(ICPB_EINVAL, "corr_stride is smaller than the longest scan%s");
+    return 0;
+}
+
+// Every scan id of B explicit pairs names a scan of the table.
+int check_pairs(const int32_t *pairs, int64_t B, int64_t n_scans)
+{
+    int32_t lo = 0, hi = 0;                                   // branch-free range check
+    for (int64_t b = 0; b < 2 * B; ++b) { lo = pairs[b] < lo ? pairs[b] : lo; hi = pairs[b] > hi ? pairs[b] : hi; }
+    if (lo < 0 || hi >= n_scans) return fail(ICPB_EINVAL, "pair index out of range%s");
     return 0;
 }
 
@@ -763,9 +763,7 @@ int icpb_set_tuning(icpb_handle h, const char *key, int64_t value)
         if (h->pool && (int)h->pool->workers.size() != v - 1) { delete h->pool; h->pool = nullptr; }
         h->tune_pack_threads = v;
     }
-    else if (!strcmp(key, "flag_copy")) h->tune_flag_copy = v != 0;
     else if (!strcmp(key, "drop_counter")) h->tune_drop_counter = v != 0;
-    else if (!strcmp(key, "trace")) h->tune_trace = v != 0;
     else return fail(ICPB_EINVAL, "icpb_set_tuning: unknown key %s", key);
     return 0;
 }
@@ -813,18 +811,9 @@ int icpb_upload_scans(icpb_handle h, const double *h_xy, const int64_t *h_offset
     int rc = validate_offsets(h_offsets, n_scans, &longest);
     if (rc) return rc;
     ON_DEVICE(h);
-    const size_t nb_xy = sizeof(double) * 2 * (size_t)h_offsets[n_scans];
-    const size_t nb_off = sizeof(int64_t) * (size_t)(n_scans + 1);
-    if ((rc = h->own_xy.reserve(nb_xy))) return rc;
-    if ((rc = h->own_off.reserve(nb_off))) return rc;
-    CU(cudaMemcpyAsync(h->own_xy.p, h_xy, nb_xy, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    h->prep_for = nullptr; h->xy = (const double *)h->own_xy.p;
-    h->offsets = (const int64_t *)h->own_off.p;
-    h->n_scans = n_scans;
-    h->longest = longest;
-    return 0;
+    if ((rc = h->own_xy.reserve(sizeof(double) * 2 * (size_t)h_offsets[n_scans]))) return rc;
+    if ((rc = h->own_off.reserve(sizeof(int64_t) * (size_t)(n_scans + 1)))) return rc;
+    return upload_table(h, h_xy, h_offsets, n_scans, longest);
 }
 
 int icpb_set_scans_device(icpb_handle h, const double *d_xy, const int64_t *d_offsets,
@@ -832,7 +821,7 @@ int icpb_set_scans_device(icpb_handle h, const double *d_xy, const int64_t *d_of
 {
     if (!h || !d_xy || !d_offsets || n_scans <= 0 || longest_scan <= 0)
         return fail(ICPB_EINVAL, "icpb_set_scans_device: bad argument%s");
-    h->prep_for = nullptr; h->xy = d_xy; h->offsets = d_offsets; h->n_scans = n_scans; h->longest = longest_scan;
+    set_table(h, d_xy, d_offsets, n_scans, longest_scan);
     return 0;
 }
 
@@ -935,10 +924,7 @@ int icpb_run_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, i
 {
     int rc = run_check(h, p, B, true, h_pairs, h_T, h_err, h_passes, h_hist, h_corr);
     if (rc || B == 0) return rc;
-    if (p->pair_mode == 0) {
-        for (int64_t b = 0; b < 2 * B; ++b)
-            if (h_pairs[b] < 0 || h_pairs[b] >= h->n_scans) return fail(ICPB_EINVAL, "pair index out of range%s");
-    }
+    if (p->pair_mode == 0 && (rc = check_pairs(h_pairs, B, h->n_scans))) return rc;
     ON_DEVICE(h);
     return run_host_common(h, h->xy, h->offsets, h->n_scans, h->longest, h_pairs, h_init, B, p,
                            h_T, h_err, h_passes, h_hist, h_corr);
@@ -1018,7 +1004,7 @@ int align_abort(icpb_ctx *h, int rc)
     cudaStreamSynchronize(h->stream); cudaStreamSynchronize(h->cstream[0]); cudaStreamSynchronize(h->cstream[1]);
     cudaGetLastError();
     memcpy(g_err, keep, sizeof keep);
-    h->prep_for = nullptr; h->xy = nullptr; h->offsets = nullptr; h->n_scans = 0; h->longest = 0;
+    drop_table(h);
     return rc;
 }
 #define CUA(call)                                                                         \
@@ -1052,13 +1038,219 @@ struct AcceptHost {
     int32_t *passes;
 };
 
+// The caller's pairs and initial guesses (init_ld 6: 2x3 rows, 9: 3x3 matrices).  icpb_align_host* checks
+// them before any state of the handle changes: a rejected call leaves the old table usable.
+int check_align_inputs(const int32_t *pairs, const double *init, int32_t init_ld, int64_t B, int64_t n_scans)
+{
+    int rc = check_pairs(pairs, B, n_scans);
+    if (rc || !init || B == 0) return rc;
+    for (int64_t b = 0; b < B && init_ld == 9; ++b) {
+        const double *m = init + 9 * b;
+        if (!(m[6] == 0.0 && m[7] == 0.0 && m[8] == 1.0))
+            return fail(ICPB_EINVAL, "transform bottom row must be [0, 0, 1] (an SE(2) matrix)%s");
+    }
+    bool bad = false;                                         // !(|v| <= bound): NaN fails too
+    for (int64_t b = 0; b < B; ++b) {
+        const double *m = init + (int64_t)init_ld * b;
+        bad |= !(fabs(m[0]) <= ICPB_MAX_GUESS_LINEAR) | !(fabs(m[1]) <= ICPB_MAX_GUESS_LINEAR) |
+               !(fabs(m[3]) <= ICPB_MAX_GUESS_LINEAR) | !(fabs(m[4]) <= ICPB_MAX_GUESS_LINEAR) |
+               !(fabs(m[2]) <= ICPB_MAX_GUESS_SHIFT) | !(fabs(m[5]) <= ICPB_MAX_GUESS_SHIFT);
+    }
+    if (bad) return fail(ICPB_EINVAL, "transform holds non-finite values or values beyond the bounds of icpb.h%s");
+    return 0;
+}
+
+// The list form of the scan table: host threads (the handle's PackPool and the calling thread) pack the
+// caller's arrays into the pinned staging table, every upload piece split into one run of scans per thread.
+// The workers write through this object, which lives on the calling frame: the destructor stops them on
+// every way out of the call.
+struct ListPacker {
+    PackJob job;
+    std::vector<int64_t> job_first, job_last;
+    std::vector<int32_t> job_piece;
+    int32_t jobs_of_piece[kMaxSegments];
+    std::atomic<int32_t> piece_done[kMaxSegments];
+    PackPool *pool = nullptr;                           // set while its workers may be running `job`
+
+    void start(icpb_ctx *h, const double *const *scan_xy, const int64_t *offsets, double *dst,
+               const int64_t *seg_end, int nseg)
+    {
+        const int nthr = h->tune_pack_threads > 0 ? std::min(h->tune_pack_threads, 32)
+                                                  : std::min(host_threads_available(), 8);   // default: at most 8
+        if (!h->pool && nthr > 1) h->pool = new (std::nothrow) PackPool(nthr - 1);
+        int64_t s0 = 0;
+        for (int k = 0; k < nseg; ++k) {
+            const int64_t s1 = seg_end[k], n = s1 - s0;
+            const int parts = (int)(n < nthr ? n : nthr);
+            for (int q = 0; q < parts; ++q) {
+                job_first.push_back(s0 + n * q / parts); job_last.push_back(s0 + n * (q + 1) / parts);
+                job_piece.push_back(k);
+            }
+            jobs_of_piece[k] = parts;
+            piece_done[k].store(0, std::memory_order_relaxed);
+            s0 = s1;
+        }
+        job.scan_xy = scan_xy; job.offsets = offsets; job.dst = dst;
+        job.job_first = job_first.data(); job.job_last = job_last.data(); job.job_piece = job_piece.data();
+        job.n_jobs = (int64_t)job_first.size(); job.done = piece_done;
+        pool = h->pool;
+        if (pool) pool->start(&job);
+    }
+    // Returns once piece k is packed; this thread packs too while it waits.  true: a bad coordinate was seen.
+    bool wait_piece(int k)
+    {
+        while (piece_done[k].load(std::memory_order_acquire) < jobs_of_piece[k]) {
+            const int64_t j = job.next.fetch_add(1, std::memory_order_relaxed);
+            if (j < job.n_jobs) pack_one(&job, j);
+        }
+        return job.bad.load(std::memory_order_relaxed) != 0;
+    }
+    // Hands out no more jobs and waits for the workers.  true: a bad coordinate was seen.
+    bool finish()
+    {
+        job.next.store(job.n_jobs, std::memory_order_relaxed);
+        if (pool) pool->finish();
+        pool = nullptr;
+        return job.bad.load() != 0;
+    }
+    ~ListPacker() { finish(); }
+};
+
+// Piece k of the streaming upload (scans [seg_end[k-1], seg_end[k]) of xy), then the arrival counter's new
+// value k + 1, in stream order: the counter changes after the piece it announces has landed.
+cudaError_t enqueue_piece(icpb_ctx *h, const double *xy, const int64_t *off, const int64_t *seg_end, int k)
+{
+    const int64_t o0 = off[k ? seg_end[k - 1] : 0], o1 = off[seg_end[k]];
+    cudaError_t e = cudaSuccess;
+    if (o1 > o0)
+        e = cudaMemcpyAsync((double *)h->own_xy.p + 2 * o0, xy + 2 * o0, sizeof(double) * 2 * (size_t)(o1 - o0),
+                            cudaMemcpyHostToDevice, h->stream);
+    // (drop_counter, tests only: the kernel must time out and the batch be rerun.)  Without
+    // cuStreamWriteValue32, or when it fails, the counter is copied.
+    if (e == cudaSuccess && !h->tune_drop_counter &&
+        (!h->write32 || h->write32(h->stream, (unsigned long long)(uintptr_t)h->arrived_dev, (unsigned)(k + 1), 0) != 0))
+        e = cudaMemcpyAsync(h->arrived_dev, h->seg_vals_pinned + (k + 1), sizeof(int32_t), cudaMemcpyHostToDevice,
+                            h->stream);
+    return e;
+}
+
+// Queue order of a streamed batch: pairs grouped by the piece that completes them (the later of their two
+// scans); the pairs, guesses and results themselves stay in the caller's order.  pseg[q]: the piece of the
+// pair at queue position q, porder[q]: that pair, unless the batch already comes in arrival order (the
+// odometry chain does).  A table whose longest scan does not fit shared memory splits the queue by scan
+// length, each part keeping its arrival order.  scratch: B words.
+struct QueueOrder {
+    bool in_order = true;                               // queue position = pair id
+    bool split = false;                                 // porder holds the split queue, sp its parts
+    Split sp;
+};
+
+QueueOrder order_queue(icpb_ctx *h, const int64_t *off, int64_t n_scans, int64_t longest, const int64_t *seg_end,
+                       int nseg, const int32_t *pairs, int64_t B, const icpb_params *p, int32_t *scratch,
+                       int32_t *porder, int32_t *pseg)
+{
+    QueueOrder qo;
+    std::vector<int32_t> seg_of_scan((size_t)n_scans);
+    for (int64_t sc = 0, k = 0; sc < n_scans; ++sc) { while (sc >= seg_end[k]) ++k; seg_of_scan[sc] = (int32_t)k; }
+    int32_t *seg_of_pair = scratch;
+    int32_t prev = 0, sorted = 1;
+    for (int64_t b = 0; b < B; ++b) {
+        const int32_t i = pairs[2 * b], j = pairs[2 * b + 1];
+        const int32_t sg = seg_of_scan[i > j ? i : j];
+        seg_of_pair[b] = sg;
+        sorted &= (int32_t)(sg >= prev);
+        prev = sg;
+    }
+    qo.in_order = sorted != 0;
+    if (qo.in_order) {
+        memcpy(pseg, seg_of_pair, sizeof(int32_t) * (size_t)B);
+    } else {                                                  // stable counting sort
+        int64_t start[kMaxSegments + 1] = {0};
+        for (int64_t b = 0; b < B; ++b) ++start[seg_of_pair[b] + 1];
+        for (int k = 0; k < nseg; ++k) start[k + 1] += start[k];
+        for (int64_t b = 0; b < B; ++b) {
+            const int64_t q = start[seg_of_pair[b]]++;
+            porder[q] = (int32_t)b; pseg[q] = seg_of_pair[b];
+        }
+    }
+    qo.split = needs_split(h, longest, B, p);
+    if (qo.split) {
+        const std::vector<int32_t> queue(porder, porder + (qo.in_order ? 0 : B));
+        qo.sp = split_queue(h, off, pairs, B, qo.in_order ? nullptr : queue.data(), porder, pseg);
+        qo.in_order = false;
+    }
+    return qo;
+}
+
+// n transforms of 6 doubles (the top two rows) into rows of ld doubles: 6 (2x3) or 9 (3x3, bottom row [0, 0, 1]).
+void put_transforms(double *dst, int32_t ld, const double *t6, int64_t n)
+{
+    if (ld == 6) { memcpy(dst, t6, sizeof(double) * 6 * (size_t)n); return; }
+    for (int64_t b = 0; b < n; ++b) {
+        double *m = dst + 9 * b;
+        memcpy(m, t6 + 6 * b, 6 * sizeof(double));
+        m[6] = 0.0; m[7] = 0.0; m[8] = 1.0;
+    }
+}
+
+// The inverse of put_transforms: the top two rows of n transforms of ld (6 or 9) doubles, as 6 doubles each.
+void get_transforms(double *t6, const double *src, int32_t ld, int64_t n)
+{
+    if (ld == 6) { memcpy(t6, src, sizeof(double) * 6 * (size_t)n); return; }
+    for (int64_t b = 0; b < n; ++b) memcpy(t6 + 6 * b, src + 9 * b, 6 * sizeof(double));
+}
+
+// icpb_align_host_accept's results: the n records the kernel appended as pairs finished (n < 0: more pairs
+// passed than the capacity, and -n of them), fetched and put in ascending pair order.
+int deliver_accepted(icpb_ctx *h, const AcceptHost *acc, int64_t n, cudaStream_t st)
+{
+    *acc->n_out = n < 0 ? -n : n;
+    if (n < 0) return fail(ICPB_EINVAL, "icpb_align_host_accept: more pairs accepted than the capacity given%s");
+    std::vector<double> rec(8 * (size_t)n);
+    if (n > 0) {
+        CU(cudaMemcpyAsync(rec.data(), (double *)h->s_hist.p + 2, sizeof(double) * 8 * (size_t)n,
+                           cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+    }
+    std::vector<int64_t> idx((size_t)n);
+    for (int64_t k = 0; k < n; ++k) idx[(size_t)k] = k;
+    auto tag_of = [&](int64_t k) { int64_t t; memcpy(&t, &rec[8 * (size_t)k + 7], sizeof t); return t; };
+    std::sort(idx.begin(), idx.end(), [&](int64_t x, int64_t y) { return (tag_of(x) >> 16) < (tag_of(y) >> 16); });
+    for (int64_t q = 0; q < n; ++q) {
+        const double *r = &rec[8 * (size_t)idx[(size_t)q]];
+        const int64_t tag = tag_of(idx[(size_t)q]);
+        acc->rows[q] = tag >> 16;
+        acc->passes[q] = (int32_t)(tag & 0xffff);
+        acc->err[q] = r[6];
+        put_transforms(acc->T + (size_t)acc->T_ld * q, acc->T_ld, r, 1);
+    }
+    return 0;
+}
+
+// Every pair's results, from the pinned download area [T | err | passes] into the caller's arrays.
+void deliver_all(const double *down, int64_t B, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes)
+{
+    put_transforms(h_T, T_ld, down, B);
+    memcpy(h_err, down + 6 * B, sizeof(double) * (size_t)B);
+    memcpy(h_passes, down + 7 * B, sizeof(int32_t) * (size_t)B);
+}
+
+// A call without pairs: the table goes up whole (planned as one piece), and the handle owns it once it has landed.
+int upload_only(icpb_ctx *h, const TableSrc &src, ListPacker &packer, const double *up_xy, int64_t n_scans,
+                int64_t longest)
+{
+    if (src.scan_xy) packer.wait_piece(0);
+    if (packer.finish())                                      // before the table goes up
+        return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates or coordinates beyond ICPB_MAX_COORD%s"));
+    const int rc = upload_table(h, up_xy, src.offsets, n_scans, longest);
+    return rc ? align_abort(h, rc) : 0;
+}
+
 int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t longest,
                const int32_t *h_pairs, const double *h_init, int32_t init_ld, int64_t B,
                const icpb_params *p, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes,
                const icpb_epilogue *ep, const AcceptHost *acc = nullptr)
 {
-    const bool trace = h->tune_trace;
-    const double t_entry = trace ? now_us() : 0.0;
     const int64_t *h_offsets = src.offsets;
     int rc;
     ON_DEVICE(h);
@@ -1089,161 +1281,37 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     }
     double *pinit = (double *)h->stage.p;
     int32_t *ppairs = (int32_t *)(pinit + 6 * B), *pseg = ppairs + 2 * B, *porder = pseg + B;
-    double *tT = (double *)((char *)h->stage.p + nb_up), *tE = tT + 6 * B;
-    int32_t *tP = (int32_t *)(tE + B);
+    double *tT = (double *)((char *)h->stage.p + nb_up);
+    int32_t *tP = (int32_t *)(tT + 7 * B);
     double *d_init = (double *)h->s_init.p;
     int32_t *d_pairs = (int32_t *)(d_init + 6 * B), *d_seg = d_pairs + 2 * B, *d_order = d_seg + B;
     double *d_T = (double *)h->s_T.p, *d_err = d_T + 6 * B;
     int32_t *d_passes = (int32_t *)(d_err + B);
-    const double *d_xy = (const double *)h->own_xy.p;
-    const int64_t *d_off = (const int64_t *)h->own_off.p;
 
-    // ---- list form: host threads pack the scans into pinned staging, piece by piece ----
-    PackJob job;
-    std::vector<int64_t> job_first, job_last;
-    std::vector<int32_t> job_piece, jobs_of_piece;
-    std::vector<std::atomic<int32_t>> piece_done(src.scan_xy ? (size_t)nseg : 0);
-    PackGuard packers;
-    const double *up_xy = src.xy;
-    if (src.scan_xy) {
-        int nthr = h->tune_pack_threads > 0 ? h->tune_pack_threads : host_threads_available();
-        if (nthr > 32) nthr = 32;
-        if (h->tune_pack_threads <= 0 && nthr > 8) nthr = 8;      // default: at most 8
-        if (nthr < 1) nthr = 1;
-        if (!h->pool && nthr > 1) h->pool = new (std::nothrow) PackPool(nthr - 1);
-        jobs_of_piece.assign((size_t)nseg, 0);
-        for (int k = 0, s0 = 0; k < nseg; ++k) {              // every piece split into nthr runs of scans
-            const int64_t s1 = seg_end[k], n = s1 - s0;
-            const int parts = (int)(n < nthr ? n : nthr);
-            for (int q = 0; q < parts; ++q) {
-                job_first.push_back(s0 + n * q / parts); job_last.push_back(s0 + n * (q + 1) / parts);
-                job_piece.push_back(k);
-            }
-            jobs_of_piece[(size_t)k] = parts;
-            piece_done[(size_t)k].store(0, std::memory_order_relaxed);
-            s0 = (int)s1;
-        }
-        job.scan_xy = src.scan_xy; job.offsets = h_offsets; job.dst = (double *)h->stage_xy.p;
-        job.job_first = job_first.data(); job.job_last = job_last.data(); job.job_piece = job_piece.data();
-        job.n_jobs = (int64_t)job_first.size(); job.done = piece_done.data();
-        packers.job = &job; packers.pool = h->pool;
-        if (h->pool) h->pool->start(&job);
-        up_xy = (const double *)h->stage_xy.p;
-    }
-    // The packers (list input) are already at work on the pinned staging; the caller's pairs and initial
-    // guesses are checked now, before any state of the handle changes: a rejected call leaves the old
-    // table usable.
-    {
-        int32_t lo = 0, hi = 0;                               // branch-free range check
-        for (int64_t b = 0; b < 2 * B; ++b) { lo = h_pairs[b] < lo ? h_pairs[b] : lo; hi = h_pairs[b] > hi ? h_pairs[b] : hi; }
-        if (lo < 0 || hi >= n_scans) return fail(ICPB_EINVAL, "pair index out of range%s");
-    }
-    if (h_init && B > 0) {                                    // before any state of the handle changes
-        for (int64_t b = 0; b < B && init_ld == 9; ++b) {
-            const double *m = h_init + 9 * b;
-            if (!(m[6] == 0.0 && m[7] == 0.0 && m[8] == 1.0))
-                return fail(ICPB_EINVAL, "transform bottom row must be [0, 0, 1] (an SE(2) matrix)%s");
-        }
-        bool bad = false;                                     // !(|v| <= bound): NaN fails too
-        for (int64_t b = 0; b < B; ++b) {
-            const double *m = h_init + (int64_t)init_ld * b;
-            bad |= !(fabs(m[0]) <= ICPB_MAX_GUESS_LINEAR) | !(fabs(m[1]) <= ICPB_MAX_GUESS_LINEAR) |
-                   !(fabs(m[3]) <= ICPB_MAX_GUESS_LINEAR) | !(fabs(m[4]) <= ICPB_MAX_GUESS_LINEAR) |
-                   !(fabs(m[2]) <= ICPB_MAX_GUESS_SHIFT) | !(fabs(m[5]) <= ICPB_MAX_GUESS_SHIFT);
-        }
-        if (bad) return fail(ICPB_EINVAL, "transform holds non-finite values or values beyond the bounds of icpb.h%s");
-    }
+    // The packers (list input) start now, so they work while the caller's pairs and initial guesses are checked
+    ListPacker packer;
+    const double *up_xy = src.scan_xy ? (const double *)h->stage_xy.p : src.xy;
+    if (src.scan_xy) packer.start(h, src.scan_xy, h_offsets, (double *)h->stage_xy.p, seg_end, nseg);
+    if ((rc = check_align_inputs(h_pairs, h_init, init_ld, B, n_scans))) return rc;
     // ---- from here on the handle's table is being replaced: a failure leaves it without one ----
-    h->prep_for = nullptr; h->xy = nullptr; h->offsets = nullptr; h->n_scans = 0; h->longest = 0;
+    drop_table(h);
+    if (B == 0) return upload_only(h, src, packer, up_xy, n_scans, longest);
     cudaStream_t cp = h->stream, cp2 = h->cstream[1], cs = h->cstream[0];
-    if (B == 0) {                                             // upload only
-        if (src.scan_xy) pack_run(&job);
-        packers.finish();                                     // before job.bad is read
-        if (src.scan_xy && job.bad.load()) return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates or coordinates beyond ICPB_MAX_COORD%s"));
-        CUA(cudaMemcpyAsync(h->own_xy.p, up_xy, nb_xy, cudaMemcpyHostToDevice, cp));
-        CUA(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, cp));
-        CUA(cudaStreamSynchronize(cp));
-        h->prep_for = nullptr; h->xy = d_xy; h->offsets = d_off; h->n_scans = n_scans; h->longest = longest;
-        return 0;
-    }
     // The first pieces start NOW, before the per-pair staging below: the copy engine works while the
     // host sorts and packs (everything has been validated above; nothing below can fail on user input).
-    int64_t s_prev = 0;
-    auto enqueue_piece = [&](int k) -> cudaError_t {
-        const int64_t o0 = h_offsets[s_prev], o1 = h_offsets[seg_end[k]];
-        cudaError_t e = cudaSuccess;
-        if (o1 > o0)
-            e = cudaMemcpyAsync((double *)h->own_xy.p + 2 * o0, up_xy + 2 * o0, sizeof(double) * 2 * (size_t)(o1 - o0),
-                                cudaMemcpyHostToDevice, cp);
-        // stream order: the counter changes after the segment it announces has landed
-        if (e != cudaSuccess || h->tune_drop_counter) {
-            // (drop_counter, tests only: the kernel must time out and the batch be rerun)
-        } else if (h->tune_flag_copy || !h->write32 ||
-                   h->write32(cp, (unsigned long long)(uintptr_t)h->arrived_dev, (unsigned)(k + 1), 0) != 0) {
-            e = cudaMemcpyAsync(h->arrived_dev, h->seg_vals_pinned + (k + 1), sizeof(int32_t), cudaMemcpyHostToDevice, cp);
-        }
-        s_prev = seg_end[k];
-        return e;
-    };
     CUA(cudaMemsetAsync(h->arrived_dev, 0, sizeof(int32_t), cp));
     CUA(cudaEventRecord(h->seg_ev[1], cp));                   // the counter is zero before the kernel may start
     int n_sent = 0;
-    if (!src.scan_xy) {
-        const int n_early = nseg < 4 ? nseg : 4;
-        for (; n_sent < n_early; ++n_sent) CUA(enqueue_piece(n_sent));
-    }
-    // Queue order: pairs grouped by the segment that completes them; the pairs, initial guesses and
-    // results themselves stay in the caller's order.  A batch that already comes in arrival order
-    // (the odometry chain does) needs no permutation at all.
-    bool in_order = true;
-    {
-        std::vector<int32_t> seg_of_scan((size_t)n_scans);
-        for (int64_t sc = 0, k = 0; sc < n_scans; ++sc) { while (sc >= seg_end[k]) ++k; seg_of_scan[sc] = (int32_t)k; }
-        int32_t *seg_of_pair = tP;                            // scratch: the download area is free until the end
-        int32_t prev = 0, sorted = 1;
-        for (int64_t b = 0; b < B; ++b) {
-            const int32_t i = h_pairs[2 * b], j = h_pairs[2 * b + 1];
-            const int32_t sg = seg_of_scan[i > j ? i : j];
-            seg_of_pair[b] = sg;
-            sorted &= (int32_t)(sg >= prev);
-            prev = sg;
-        }
-        in_order = sorted != 0;
-        if (in_order) {
-            memcpy(pseg, seg_of_pair, nb4);
-        } else {                                              // stable counting sort
-            int64_t start[kMaxSegments + 1] = {0};
-            for (int64_t b = 0; b < B; ++b) ++start[seg_of_pair[b] + 1];
-            for (int k = 0; k < nseg; ++k) start[k + 1] += start[k];
-            for (int64_t b = 0; b < B; ++b) {
-                const int64_t q = start[seg_of_pair[b]]++;
-                porder[q] = (int32_t)b; pseg[q] = seg_of_pair[b];
-            }
-        }
-    }
-    // a table whose longest scan does not fit shared memory: the queue is split by scan length, each part
-    // keeping its arrival order
-    Split sp;
-    const bool split = needs_split(h, longest, B, p);
-    if (split) {
-        std::vector<int32_t> queue(in_order ? 0 : (size_t)B);
-        if (!in_order) memcpy(queue.data(), porder, nb4);
-        sp = split_queue(h, h_offsets, h_pairs, B, in_order ? nullptr : queue.data(), porder, pseg);
-        in_order = false;
-    }
+    if (!src.scan_xy)
+        for (; n_sent < (nseg < 4 ? nseg : 4); ++n_sent) CUA(enqueue_piece(h, up_xy, h_offsets, seg_end, n_sent));
+    const QueueOrder qo = order_queue(h, h_offsets, n_scans, longest, seg_end, nseg, h_pairs, B, p,
+                                      tP /* the download area is free until the end */, porder, pseg);
     memcpy(ppairs, h_pairs, 2 * nb4);
-    if (h_init) {
-        if (init_ld == 6) {
-            memcpy(pinit, h_init, nbI);
-        } else {
-            for (int64_t b = 0; b < B; ++b) memcpy(pinit + 6 * b, h_init + 9 * b, 6 * sizeof(double));
-        }
-    }
-    const double t_prep = trace ? now_us() : 0.0;
+    if (h_init) get_transforms(pinit, h_init, init_ld, B);
     // the small per-pair block goes up on a second copy stream, beside the pieces already in flight
     CUA(cudaMemsetAsync(d_passes + B, 0, sizeof(int32_t), cp2));
     CUA(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, cp2));
-    const size_t nb_idx = (in_order ? 3 : 4) * nb4;           // pairs, seg (, order)
+    const size_t nb_idx = (qo.in_order ? 3 : 4) * nb4;        // pairs, seg (, order)
     if (h_init) CUA(cudaMemcpyAsync(d_init, pinit, nbI + nb_idx, cudaMemcpyHostToDevice, cp2));
     else        CUA(cudaMemcpyAsync(d_pairs, ppairs, nb_idx, cudaMemcpyHostToDevice, cp2));
     CUA(cudaEventRecord(h->seg_ev[0], cp2));
@@ -1251,40 +1319,18 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     CUA(cudaStreamWaitEvent(cs, h->seg_ev[0], 0));
     CUA(cudaStreamWaitEvent(cs, h->seg_ev[1], 0));
     Batch bt;
-    bt.xy = d_xy; bt.offsets = d_off; bt.n_scans = n_scans; bt.longest = longest;
-    bt.pairs = d_pairs; bt.init = h_init ? d_init : nullptr; bt.B = B; bt.p = p;
+    bt.xy = (const double *)h->own_xy.p; bt.offsets = (const int64_t *)h->own_off.p; bt.n_scans = n_scans;
+    bt.longest = longest; bt.pairs = d_pairs; bt.init = h_init ? d_init : nullptr; bt.B = B; bt.p = p;
     bt.T = d_T; bt.err = d_err; bt.passes = d_passes;
-    bt.stream = cs; bt.ep = ep; bt.order = in_order ? nullptr : d_order;
+    bt.stream = cs; bt.ep = ep; bt.order = qo.in_order ? nullptr : d_order;
     bt.seg_of_pair = d_seg; bt.arrived = h->arrived_dev; bt.upload_timeout = d_passes + B;
-    bt.split = split ? &sp : nullptr;
+    bt.split = qo.split ? &qo.sp : nullptr;
     if ((rc = launch(h, bt))) return align_abort(h, rc);
-    bool bad_scans = false;
-    double t_ready[kMaxSegments] = {0}, t_enqd[kMaxSegments] = {0};   // trace: piece k packed / enqueued (host clock)
-    cudaEvent_t tev[kMaxSegments + 1] = {nullptr};            // trace: when piece k had landed (device clock)
-    cudaEvent_t tev0[kMaxSegments] = {nullptr};               // trace: when piece k's copy could start
-    if (trace) { cudaEventCreate(&tev[kMaxSegments]); cudaEventRecord(tev[kMaxSegments], cp); }
     for (int k = n_sent; k < nseg; ++k) {
-        if (src.scan_xy) {
-            // this thread packs too while a piece is incomplete (pack_run returns when no job is left)
-            while (piece_done[(size_t)k].load(std::memory_order_acquire) < jobs_of_piece[(size_t)k]) {
-                const int64_t j = job.next.fetch_add(1, std::memory_order_relaxed);
-                if (j < job.n_jobs) {
-                    PackJob one;                              // run exactly job j on this thread
-                    one.scan_xy = job.scan_xy; one.offsets = job.offsets; one.dst = job.dst;
-                    one.job_first = job.job_first + j; one.job_last = job.job_last + j; one.job_piece = job.job_piece + j;
-                    one.n_jobs = 1; one.done = job.done;
-                    pack_run(&one);
-                    if (one.bad.load()) job.bad.fetch_or(1, std::memory_order_relaxed);
-                }
-            }
-            if (job.bad.load(std::memory_order_relaxed)) { bad_scans = true; break; }
-        }
-        if (trace) { t_ready[k] = now_us() - t_entry; cudaEventCreate(&tev0[k]); cudaEventRecord(tev0[k], cp); }
-        CUA(enqueue_piece(k));
-        if (trace) { t_enqd[k] = now_us() - t_entry; cudaEventCreate(&tev[k]); cudaEventRecord(tev[k], cp); }
+        if (src.scan_xy && packer.wait_piece(k)) break;       // a bad scan: no further piece goes up
+        CUA(enqueue_piece(h, up_xy, h_offsets, seg_end, k));
     }
-    packers.finish();                                         // every piece is packed, or a bad scan ended it
-    if (bad_scans) {
+    if (packer.finish()) {
         // the kernel is waiting for pieces that will not come: raise its give-up flag, drain, report
         CUA(cudaMemcpyAsync(d_passes + B, h->seg_vals_pinned + 1, sizeof(int32_t), cudaMemcpyHostToDevice, cp));
         return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates or coordinates beyond ICPB_MAX_COORD%s"));
@@ -1298,7 +1344,6 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
         CUA(cudaMemcpyAsync(tP + B, d_passes + B, sizeof(int32_t), cudaMemcpyDeviceToHost, cp));
         CUA(cudaMemcpyAsync(acc_cnt, h->s_hist.p, sizeof(int64_t), cudaMemcpyDeviceToHost, cp));
     }
-    const double t_enq = trace ? now_us() : 0.0;
     CUA(cudaStreamSynchronize(cp));
     if (tP[B] != 0) {
         // a CTA gave up waiting for its scans (see the kernel): by now the whole table is resident,
@@ -1312,59 +1357,9 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
         CUA(cudaStreamSynchronize(cp));
     }
     // only now does the handle own the new table
-    h->prep_for = nullptr; h->xy = d_xy; h->offsets = d_off; h->n_scans = n_scans; h->longest = longest;
-    const double t_sync = trace ? now_us() : 0.0;
-    if (acc) {
-        // the accepted records only: fetch, order by pair id (the kernel appended them as they finished)
-        const int64_t n = *acc_cnt;
-        *acc->n_out = n < 0 ? -n : n;
-        if (n < 0) return fail(ICPB_EINVAL, "icpb_align_host_accept: more pairs accepted than the capacity given%s");
-        std::vector<double> rec(8 * (size_t)n);
-        if (n > 0) {
-            CU(cudaMemcpyAsync(rec.data(), (double *)h->s_hist.p + 2, sizeof(double) * 8 * (size_t)n,
-                               cudaMemcpyDeviceToHost, cp));
-            CU(cudaStreamSynchronize(cp));
-        }
-        std::vector<int64_t> idx((size_t)n);
-        for (int64_t k = 0; k < n; ++k) idx[(size_t)k] = k;
-        auto tag_of = [&](int64_t k) { int64_t t; memcpy(&t, &rec[8 * (size_t)k + 7], sizeof t); return t; };
-        std::sort(idx.begin(), idx.end(), [&](int64_t x, int64_t y) { return (tag_of(x) >> 16) < (tag_of(y) >> 16); });
-        for (int64_t q = 0; q < n; ++q) {
-            const double *r = &rec[8 * (size_t)idx[(size_t)q]];
-            const int64_t tag = tag_of(idx[(size_t)q]);
-            acc->rows[q] = tag >> 16;
-            acc->passes[q] = (int32_t)(tag & 0xffff);
-            acc->err[q] = r[6];
-            double *m = acc->T + (size_t)acc->T_ld * q;
-            memcpy(m, r, 6 * sizeof(double));
-            if (acc->T_ld == 9) { m[6] = 0.0; m[7] = 0.0; m[8] = 1.0; }
-        }
-        return 0;
-    }
-    if (T_ld == 6) {
-        memcpy(h_T, tT, nbI);
-    } else {
-        for (int64_t b = 0; b < B; ++b) {
-            double *m = h_T + 9 * b;
-            memcpy(m, tT + 6 * b, 6 * sizeof(double));
-            m[6] = 0.0; m[7] = 0.0; m[8] = 1.0;
-        }
-    }
-    memcpy(h_err, tE, nbE);
-    memcpy(h_passes, tP, nb4);
-    if (trace) {
-        fprintf(stderr, "[icpb_align_host] prep %.0f us, enqueue %.0f us, wait %.0f us, scatter %.0f us (%d segments)\n",
-                t_prep - t_entry, t_enq - t_prep, t_sync - t_enq, now_us() - t_sync, nseg);
-        fprintf(stderr, "  piece: packed at / enqueued at (host us) / landed at (us after the copy stream's first event):");
-        for (int k = 0; k < nseg; ++k) {
-            float ms = 0.f, ms0 = 0.f;
-            if (tev[k]) { cudaEventElapsedTime(&ms, tev[kMaxSegments], tev[k]); cudaEventDestroy(tev[k]); }
-            if (tev0[k]) { cudaEventElapsedTime(&ms0, tev[kMaxSegments], tev0[k]); cudaEventDestroy(tev0[k]); }
-            fprintf(stderr, " %d:%.0f/%.0f/%.0f-%.0f", k, t_ready[k], t_enqd[k], ms0 * 1e3, ms * 1e3);
-        }
-        fprintf(stderr, "\n");
-        cudaEventDestroy(tev[kMaxSegments]);
-    }
+    set_table(h, bt.xy, bt.offsets, n_scans, longest);
+    if (acc) return deliver_accepted(h, acc, *acc_cnt, cp);
+    deliver_all(tT, B, h_T, T_ld, h_err, h_passes);
     return 0;
 }
 

@@ -363,8 +363,7 @@ int icpb_get_kernel_info(icpb_handle h, int64_t B, icpb_kernel_info *out);
 /* Tuning and test hooks, per handle (nothing is read from the environment).  Keys: "threads" (CTA
  * width cap, multiple of 32), "cluster" (force a cluster size: 0/1 never, 2/4/8), "segments" (upload
  * pieces), "pack_threads" (host threads of icpb_align_host_scans, default min(8, cpus)),
- * "flag_copy" (arrival counter by 4-byte copies), "drop_counter" (tests: never
- * advance the arrival counter), "trace" (host timings on stderr), "large" (1: every pair on the
+ * "drop_counter" (tests: never advance the arrival counter), "large" (1: every pair on the
  * large-scan variant, arrays in device scratch instead of shared memory -- same results; 0 / -1: only
  * pairs whose scans do not fit shared memory).  0 / -1 restore the default.
  *

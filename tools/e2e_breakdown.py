@@ -19,7 +19,6 @@ for nthr in (4, 8, 12, 16):
     e.set_tuning("pack_threads", nthr)
     print("align (list, %d pack thr)  %.3f ms" % (nthr, tm(lambda: e.align(scans, pairs, init, epsilon=0.05))))
 e.set_tuning("pack_threads", 0)
-e.set_tuning("trace", 1); e.align(scans, pairs, init, epsilon=0.05); e.set_tuning("trace", 0)
 print("ScanList(scans)           %.3f ms" % tm(lambda: gicp.ScanList(scans)))
 e.set_scans(tp)
 print("run only (resident scans) %.3f ms" % tm(lambda: e.run(pairs, init, epsilon=0.05)))

@@ -1,7 +1,6 @@
 #!/usr/bin/env python
-"""Host-to-host time of IcpEngine.align on the headline workload for the three input forms (list of
-pageable arrays, prebuilt ScanList, pinned table), and one traced call: when every upload piece was
-packed, enqueued and had landed (developer probe; DESIGN.md section 5)."""
+"""Host-to-host time of IcpEngine.align on the headline workload for the three input forms: a list of
+pageable arrays, a prebuilt ScanList and a pinned table (developer probe; DESIGN.md section 5)."""
 import sys, time, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -19,4 +18,3 @@ print("align(ScanList prebuilt) %.3f ms" % tm(lambda: e.align(sl, pairs, init, e
 t = gicp.ScanTable(scans); xy = torch.from_numpy(t.xy).pin_memory()
 tp = gicp.ScanTable(xy=xy.numpy(), offsets=t.offsets)
 print("align(pinned table) %.3f ms" % tm(lambda: e.align(tp, pairs, init, epsilon=0.05)))
-e.set_tuning("trace", 1); e.align(scans, pairs, init, epsilon=0.05); e.set_tuning("trace", 0)
