@@ -23,7 +23,7 @@ EXPORTS = ["icpb_default_params", "icpb_abi_version", "icpb_create", "icpb_destr
            "icpb_run_device_gather", "icpb_pose_graph_sgd", "icpb_occupancy_grid_bounds",
            "icpb_occupancy_grid_update", "icpb_run_device_ex", "icpb_align_host_ex", "icpb_align_host_scans",
            "icpb_set_tuning", "icpb_scan_count", "icpb_align_host_accept",
-           "icpb_compose_chain_device", "icpb_compose_chain_gpu"]
+           "icpb_compose_chain_device", "icpb_compose_chain_gpu", "icpb_run_multistart_host"]
 
 
 class IcpbParams(ctypes.Structure):
@@ -63,6 +63,7 @@ def sources():
                                               os.path.join(c, "icpb_sgd.cuh"),
                                               os.path.join(c, "icpb_grid.cuh"),
                                               os.path.join(c, "icpb_compose.cuh"),
+                                              os.path.join(c, "icpb_multistart.cuh"),
                                               os.path.join(_ROOT, "include", "icpb.h")]
 
 
@@ -174,6 +175,8 @@ def lib() -> ctypes.CDLL:
                                          ctypes.POINTER(IcpbParams), ctypes.c_double, i64,
                                          ctypes.POINTER(ctypes.c_int64), vp, dp, ctypes.c_int32, dp, i32p]
     L.icpb_run_host.argtypes = [vp, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p, dp, i32p]
+    L.icpb_run_multistart_host.argtypes = [vp, i32p, dp, i64, dp, ctypes.c_int32, ctypes.POINTER(IcpbParams),
+                                           dp, dp, i32p, i32p, dp, i32p]
     L.icpb_align_host.argtypes = [vp, dp, vp, i64, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p]
     L.icpb_align_host_ld.argtypes = [vp, dp, vp, i64, i32p, dp, ctypes.c_int32, i64, ctypes.POINTER(IcpbParams),
                                      dp, ctypes.c_int32, dp, i32p]

@@ -148,8 +148,17 @@ def proximity_pairs(poses, min_dist_along_path=2, max_dist=1, device=None) -> np
     return pairs
 
 
+def _multistart_accept(lidar_points, pairs, starts, thresh, epsilon, max_iters, device):
+    """Every candidate aligned from the identity with every start (so its guesses are the starts
+    themselves), the best start kept, and the pairs whose best error is below ``thresh``: (rows,
+    MultiStartResult of those rows).  The threshold runs on the host over B results, not B * K."""
+    res = _icp.icp_multistart(lidar_points, pairs, starts, None, epsilon=epsilon, max_iters=max_iters, device=device)
+    rows = np.nonzero(res.error < thresh)[0]
+    return rows, _icp.MultiStartResult(res.T[rows], res.error[rows], res.iters[rows], start=res.start[rows])
+
+
 def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist=1, err_thresh=110,
-                            max_iters=100, epsilon=0.05, device=None):
+                            max_iters=100, epsilon=0.05, device=None, starts=None):
     """Loop-closure constraints the reference's ``detect_proximity`` would add, in its order.
 
     ICP is a pure function of its inputs, so every candidate is aligned in one batch
@@ -157,16 +166,24 @@ def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist
     loop -- skip a candidate if either endpoint was already used by an *accepted* one, accept if
     error < err_thresh -- is replayed on the results (:27-39).  Returns a list of
     (i, j, T 3x3) ready for ``pose_graph.add_constraint(i, j, T)``, and the BatchResult of the candidates
-    that passed the threshold."""
+    that passed the threshold.
+
+    ``starts`` ((K, 3, 3), e.g. ``icp.heading_starts(8)``): for revisits whose relative heading is
+    unknown, every candidate is aligned from each start with ``icp_multistart`` and its best start is
+    the one tested against the threshold; the BatchResult is then a MultiStartResult (``start`` says
+    which start won)."""
     cand = proximity_candidates(poses, min_dist_along_path, max_dist, device)
     if len(cand) == 0:
         return [], None
     pairs = np.stack((cand[:, 1], cand[:, 0]), axis=1).astype(np.int32)
-    # the `error < err_thresh` test runs in the kernel epilogue: only the candidates that pass it come
-    # back (a candidate that fails it never marks its endpoints as used, so the greedy loop over the
-    # passing ones, in the reference's order, accepts exactly what the reference accepts)
-    rows, res = _icp.engine(device).align_accept(lidar_points, pairs, err_thresh, None, epsilon=epsilon,
-                                                 max_iters=max_iters)
+    if starts is not None:
+        rows, res = _multistart_accept(lidar_points, pairs, starts, err_thresh, epsilon, max_iters, device)
+    else:
+        # the `error < err_thresh` test runs in the kernel epilogue: only the candidates that pass it come
+        # back (a candidate that fails it never marks its endpoints as used, so the greedy loop over the
+        # passing ones, in the reference's order, accepts exactly what the reference accepts)
+        rows, res = _icp.engine(device).align_accept(lidar_points, pairs, err_thresh, None, epsilon=epsilon,
+                                                     max_iters=max_iters)
     used = set()
     out = []
     for (i, j), T in zip(cand[rows], res.T):
@@ -180,19 +197,24 @@ def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist
 
 
 def image_match_loop_closures(good_matches, lidar_points, image_rate=1, icp_err_thresh=30, max_iters=100,
-                              epsilon=0.05, device=None):
+                              epsilon=0.05, device=None, starts=None):
     """ICP block of the reference's ``detect_images_direct_similarity``
     (src/loop_closure_detection.py:134-159): for every image match (i, j) align scan
     ``i*image_rate`` (source) onto scan ``j*image_rate`` (target) from the identity -- note the
     argument order is the opposite of ``detect_proximity``'s, a reference quirk kept as is -- and
     keep the pairs with error < icp_err_thresh.  Returns [(i*rate, j*rate, T)] in match order, and
-    the BatchResult of the accepted pairs.  The ORB/matcher front end that produces ``good_matches`` is out of scope."""
+    the BatchResult of the accepted pairs.  The ORB/matcher front end that produces ``good_matches`` is out of scope.
+    ``starts``: a multi-start sweep per match, as in ``proximity_loop_closures`` (an image match between
+    scans taken facing different directions)."""
     gm = np.asarray(good_matches, dtype=np.int64).reshape(-1, 2)
     if len(gm) == 0:
         return [], None
     pairs = (gm * image_rate).astype(np.int32)               # (source = i*rate, target = j*rate)
-    rows, res = _icp.engine(device).align_accept(lidar_points, pairs, icp_err_thresh, None, epsilon=epsilon,
-                                                 max_iters=max_iters)          # filter on the device
+    if starts is not None:
+        rows, res = _multistart_accept(lidar_points, pairs, starts, icp_err_thresh, epsilon, max_iters, device)
+    else:
+        rows, res = _icp.engine(device).align_accept(lidar_points, pairs, icp_err_thresh, None, epsilon=epsilon,
+                                                     max_iters=max_iters)      # filter on the device
     out = [(int(pairs[r, 0]), int(pairs[r, 1]), T) for r, T in zip(rows, res.T)]
     return out, res
 

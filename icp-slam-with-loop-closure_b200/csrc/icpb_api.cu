@@ -24,6 +24,7 @@
 #include "icpb_sgd.cuh"
 #include "icpb_grid.cuh"
 #include "icpb_compose.cuh"
+#include "icpb_multistart.cuh"
 
 namespace {
 
@@ -306,6 +307,7 @@ struct icpb_ctx {
     DevBuf s_accept;                                // acceptance epilogue: [appended, CTAs left] counters
     DevBuf s_big;                                   // large-scan variant: one scratch region per CTA
     DevBuf s_order;                                 // queue order of a batch split by scan length
+    DevBuf s_ms;                                    // multi-start: a slice's pairs, guesses, order, results; the starts
     // per-scan staging images of the resident table (KernelArgs::prep_in), built on first use
     DevBuf prep;
     const double *prep_for = nullptr;               // the table (h->xy) the images were built from
@@ -781,7 +783,7 @@ int icpb_destroy(icpb_handle h)
     if (h->arrived_dev) cudaFree(h->arrived_dev);
     if (h->seg_vals_pinned) cudaFreeHost(h->seg_vals_pinned);
     h->s_seg.release(); h->stage.release(); h->s_sgd.release(); h->s_grid.release();
-    h->s_accept.release(); h->stage_xy.release(); h->prep.release(); h->s_big.release(); h->s_order.release();
+    h->s_accept.release(); h->stage_xy.release(); h->prep.release(); h->s_big.release(); h->s_order.release(); h->s_ms.release();
     h->own_xy.release(); h->own_off.release();
     h->s_pairs.release(); h->s_init.release(); h->s_T.release(); h->s_err.release();
     h->s_passes.release(); h->s_hist.release(); h->s_corr.release();
@@ -928,6 +930,160 @@ int icpb_run_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, i
     ON_DEVICE(h);
     return run_host_common(h, h->xy, h->offsets, h->n_scans, h->longest, h_pairs, h_init, B, p,
                            h_T, h_err, h_passes, h_hist, h_corr);
+}
+
+}  // extern "C"
+
+namespace {
+
+// Problems of one multi-start launch: a slice holds floor(kMaxMultistart / K) pairs with all K of their
+// starts, so the int32 queue order of a split slice stays in range and its scratch (116 bytes per
+// problem: pair, guess, transform, error, passes) within ~490 MB.
+constexpr int64_t kMaxMultistart = int64_t(1) << 22;
+
+// Every composed guess G = init[b] . S[k] (the formula of icpb.h, identity for a null init) is within the
+// guess bounds, tested as !(|v| <= bound) like check_align_inputs; evaluated in one pass, not stored.
+// Contraction is off so that a product is never fused into the sum that follows it.
+#if defined(__GNUC__) && !defined(__clang__)
+__attribute__((optimize("fp-contract=off")))
+#endif
+int check_composed(const double *init, int64_t B, const double *S, int32_t K)
+{
+    static const double kI[6] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0};
+    bool bad = false;
+    for (int64_t b = 0; b < B; ++b) {
+        const double *I = init ? init + 6 * b : kI;
+        for (int32_t k = 0; k < K; ++k) {
+            const double *s = S + 6 * (int64_t)k;
+            for (int r = 0; r < 2; ++r) {
+                const double a = I[3 * r], c = I[3 * r + 1], t = I[3 * r + 2];
+                const double p0 = a * s[0], q0 = c * s[3], p1 = a * s[1], q1 = c * s[4];
+                const double p2 = a * s[2], q2 = c * s[5];
+                const double g0 = p0 + q0, g1 = p1 + q1, g2 = (p2 + q2) + t;
+                bad |= !(fabs(g0) <= ICPB_MAX_GUESS_LINEAR) | !(fabs(g1) <= ICPB_MAX_GUESS_LINEAR) |
+                       !(fabs(g2) <= ICPB_MAX_GUESS_SHIFT);
+            }
+        }
+    }
+    if (bad) return fail(ICPB_EINVAL, "a composed guess init . start holds non-finite values or values beyond the bounds of icpb.h%s");
+    return 0;
+}
+
+// Device-side arrays of one multi-start call, carved out of one buffer (256-byte aligned).
+struct MsArrays {
+    int32_t *pairs = nullptr, *pair_order = nullptr, *passes = nullptr, *start = nullptr;
+    double *init = nullptr, *starts = nullptr, *T = nullptr, *err = nullptr;
+};
+
+int run_multistart(icpb_ctx *h, const int32_t *h_pairs, const double *h_init, int64_t B, const double *h_starts,
+                   int32_t K, const icpb_params *p_in, double *h_T, double *h_err, int32_t *h_passes, int32_t *h_start,
+                   double *h_err_all, int32_t *h_passes_all)
+{
+    int rc;
+    cudaStream_t st = h->stream;
+    const int64_t per = kMaxMultistart / K;                           // pairs per slice
+    const int64_t n_max = B < per ? B : per, q_max = n_max * K;
+    // per-pair arrays of a slice and the K starts
+    size_t used = 0;
+    auto carve = [&](size_t bytes) { const size_t o = used; used += (bytes + 255) & ~size_t(255); return o; };
+    const size_t o_pairs = carve(8 * (size_t)n_max), o_init = carve(h_init ? 48 * (size_t)n_max : 0);
+    const size_t o_order = carve(4 * (size_t)n_max), o_starts = carve(48 * (size_t)K);
+    const size_t o_T = carve(48 * (size_t)n_max), o_err = carve(8 * (size_t)n_max);
+    const size_t o_passes = carve(4 * (size_t)n_max), o_start = carve(4 * (size_t)n_max);
+    if ((rc = h->s_ms.reserve(used))) return rc;
+    unsigned char *base = (unsigned char *)h->s_ms.p;
+    MsArrays d;
+    d.pairs = (int32_t *)(base + o_pairs); d.init = h_init ? (double *)(base + o_init) : nullptr;
+    d.pair_order = (int32_t *)(base + o_order); d.starts = (double *)(base + o_starts);
+    d.T = (double *)(base + o_T); d.err = (double *)(base + o_err);
+    d.passes = (int32_t *)(base + o_passes); d.start = (int32_t *)(base + o_start);
+    // the expanded problems of a slice, in the host entry point's scratch
+    if ((rc = h->s_pairs.reserve(8 * (size_t)q_max)) || (rc = h->s_init.reserve(48 * (size_t)q_max)) ||
+        (rc = h->s_T.reserve(48 * (size_t)q_max)) || (rc = h->s_err.reserve(8 * (size_t)q_max)) ||
+        (rc = h->s_passes.reserve(4 * (size_t)q_max)))
+        return rc;
+    int32_t *epairs = (int32_t *)h->s_pairs.p, *epasses = (int32_t *)h->s_passes.p;
+    double *eG = (double *)h->s_init.p, *eT = (double *)h->s_T.p, *eerr = (double *)h->s_err.p;
+    CU(cudaMemcpyAsync(d.starts, h_starts, 48 * (size_t)K, cudaMemcpyHostToDevice, st));
+    icpb_params p = *p_in;
+    p.k_first = 0; p.k_stride = 0;
+    std::vector<int64_t> off;                                         // the table's offsets, for a split
+    std::vector<int32_t> pair_order;
+    for (int64_t p0 = 0; p0 < B; p0 += per) {
+        const int64_t n = B - p0 < per ? B - p0 : per, nq = n * K;
+        p.k_block = nq;
+        CU(cudaMemcpyAsync(d.pairs, h_pairs + 2 * p0, 8 * (size_t)n, cudaMemcpyHostToDevice, st));
+        if (h_init) CU(cudaMemcpyAsync(d.init, h_init + 6 * p0, 48 * (size_t)n, cudaMemcpyHostToDevice, st));
+        Split sp;
+        const bool split = needs_split(h, h->longest, nq, &p);
+        if (split) {
+            if (off.empty()) {
+                off.resize((size_t)h->n_scans + 1);
+                CU(cudaMemcpyAsync(off.data(), h->offsets, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, st));
+                CU(cudaStreamSynchronize(st));
+            }
+            // the slice's pairs in queue order; the expansion turns every pair into its K problems
+            pair_order.resize((size_t)n);
+            const Split ps = split_queue(h, off.data(), h_pairs + 2 * p0, n, nullptr, pair_order.data(), nullptr);
+            sp.ns = ps.ns * K; sp.Ls = ps.Ls; sp.Ll = ps.Ll;
+            if ((rc = h->s_order.reserve(4 * (size_t)q_max))) return rc;
+            CU(cudaMemcpyAsync(d.pair_order, pair_order.data(), 4 * (size_t)n, cudaMemcpyHostToDevice, st));
+        }
+        int64_t blocks = (nq + icpb::kMultistartThreads - 1) / icpb::kMultistartThreads;
+        if (blocks > 16 * (int64_t)h->sm_count) blocks = 16 * (int64_t)h->sm_count;
+        icpb::multistart_expand_kernel<<<(unsigned)blocks, icpb::kMultistartThreads, 0, st>>>(
+            d.pairs, d.init, d.starts, K, n, split ? d.pair_order : nullptr, epairs, eG,
+            split ? (int32_t *)h->s_order.p : nullptr);
+        CU(cudaGetLastError());
+        Batch b;
+        b.xy = h->xy; b.offsets = h->offsets; b.n_scans = h->n_scans; b.longest = h->longest;
+        b.pairs = epairs; b.init = eG; b.B = nq; b.p = &p;
+        b.T = eT; b.err = eerr; b.passes = epasses; b.stream = st;
+        if (split) { b.order = (const int32_t *)h->s_order.p; b.split = &sp; }
+        if ((rc = launch(h, b))) return rc;
+        blocks = (n + icpb::kMultistartThreads - 1) / icpb::kMultistartThreads;
+        if (blocks > 16 * (int64_t)h->sm_count) blocks = 16 * (int64_t)h->sm_count;
+        icpb::multistart_select_kernel<<<(unsigned)blocks, icpb::kMultistartThreads, 0, st>>>(
+            eT, eerr, epasses, K, n, d.T, d.err, d.passes, d.start);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(h_T + 6 * p0, d.T, 48 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_err + p0, d.err, 8 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_passes + p0, d.passes, 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_start + p0, d.start, 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        // problem p_local * K + k is row p, column k of the (B, K) arrays
+        if (h_err_all) CU(cudaMemcpyAsync(h_err_all + p0 * K, eerr, 8 * (size_t)nq, cudaMemcpyDeviceToHost, st));
+        if (h_passes_all) CU(cudaMemcpyAsync(h_passes_all + p0 * K, epasses, 4 * (size_t)nq, cudaMemcpyDeviceToHost, st));
+        // the next slice overwrites the scratch: its copies are enqueued behind these on the same stream
+    }
+    CU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int icpb_run_multistart_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, int64_t B,
+                             const double *h_starts, int32_t K, const icpb_params *p,
+                             double *h_T, double *h_err, int32_t *h_passes, int32_t *h_start,
+                             double *h_err_all, int32_t *h_passes_all)
+{
+    if (!h) return fail(ICPB_EINVAL, "handle is null%s");
+    if (!p) return fail(ICPB_EINVAL, "params is null%s");
+    if (p->hist_cap > 0 || p->corr_stride > 0)
+        return fail(ICPB_EINVAL, "multi-start runs record no history or correspondences: rerun icpb_run_host on "
+                                 "the winning guesses for them%s");
+    if (p->pair_mode != 0) return fail(ICPB_EINVAL, "multi-start runs take explicit pairs (pair_mode 0)%s");
+    if (K < 1 || K > kMaxMultistart) return fail(ICPB_EINVAL, "the number of starts must be in 1 .. 2^22%s");
+    if (!h_starts) return fail(ICPB_EINVAL, "starts is null%s");
+    int rc = run_check(h, p, B, true, h_pairs, h_T, h_err, h_passes, nullptr, nullptr);
+    if (rc || B == 0) return rc;
+    if (!h_start) return fail(ICPB_EINVAL, "output pointer is null%s");
+    if ((rc = check_pairs(h_pairs, B, h->n_scans))) return rc;
+    if ((rc = check_composed(h_init, B, h_starts, K))) return rc;
+    ON_DEVICE(h);
+    return run_multistart(h, h_pairs, h_init, B, h_starts, K, p, h_T, h_err, h_passes, h_start,
+                          h_err_all, h_passes_all);
 }
 
 /* Upload + align with the upload hidden behind the kernels: the scan table goes up in segments on

@@ -11,7 +11,8 @@ Same names, argument meaning and return contracts as the reference module:
 
 plus the batched entry point ``icp_batch`` that replaces the reference's joblib fan-outs
 (scripts/main.py:240-247, src/loop_closure_detection.py:134-142,
-src/pose_graph_optimization.py:60-68) with one kernel launch.
+src/pose_graph_optimization.py:60-68) with one kernel launch, and ``icp_multistart``, which aligns
+every pair from K start transforms and keeps the best one (``heading_starts``, ``compose_starts``).
 
 There is no CPU fallback: without libicpb.so and a B200 every call raises.
 """
@@ -25,10 +26,11 @@ import numpy as np
 
 from . import _lib
 from ._lib import IcpbError  # noqa: F401  (re-exported)
+from .synth import pose_to_mat
 
-__all__ = ["icp", "icp_iteration", "icp_batch", "get_correspondences", "get_closest_point",
-           "get_transform", "get_error",
-           "ScanTable", "ScanList", "IcpEngine", "BatchResult", "engine", "make_epilogue"]
+__all__ = ["icp", "icp_iteration", "icp_batch", "icp_multistart", "heading_starts", "compose_starts",
+           "get_correspondences", "get_closest_point", "get_transform", "get_error",
+           "ScanTable", "ScanList", "IcpEngine", "BatchResult", "MultiStartResult", "engine", "make_epilogue"]
 
 
 # Input magnitudes the kernel is exact for (include/icpb.h: ICPB_MAX_COORD, ICPB_MAX_GUESS_LINEAR,
@@ -115,6 +117,15 @@ class BatchResult:
         return len(self.error)
 
 
+@dataclass
+class MultiStartResult(BatchResult):
+    """Per-pair results of ``icp_multistart``: the winning start's ``T``, ``error`` and ``iters``, and
+    which start won.  With ``return_all=True`` also every start's error and pass count."""
+    start: np.ndarray | None = None            # (B,) int32: the smallest k with the smallest error
+    error_all: np.ndarray | None = None        # (B, K) float64
+    iters_all: np.ndarray | None = None        # (B, K) int32
+
+
 def _to6(T) -> np.ndarray:
     T = np.asarray(T, dtype=np.float64)
     if T.shape[-2:] != (3, 3):
@@ -136,6 +147,51 @@ def _to33(T6: np.ndarray) -> np.ndarray:
 
 def _ptr(a):
     return None if a is None else ctypes.c_void_p(a.ctypes.data)
+
+
+def _rows6(T, n, name) -> np.ndarray:
+    """(n, 3, 3) SE(2)-shaped matrices (n None: any number) -> (n, 6) top rows, with the shape, the
+    bottom rows and finiteness checked; the bounds are the library's to check (on the composed guesses)."""
+    T = np.asarray(T, dtype=np.float64)
+    if T.ndim != 3 or T.shape[1:] != (3, 3) or (n is not None and len(T) != n):
+        raise ValueError(f"{name} has shape {T.shape}; expected ({'K' if n is None else n}, 3, 3)")
+    if not (np.all(T[..., 2, 0] == 0) and np.all(T[..., 2, 1] == 0) and np.all(T[..., 2, 2] == 1)):
+        raise ValueError(f"{name}: bottom row must be [0, 0, 1] (an SE(2) matrix)")
+    if not np.isfinite(T).all():
+        raise ValueError(f"{name} holds non-finite values")
+    return np.ascontiguousarray(T[..., :2, :].reshape(T.shape[:-2] + (6,)))
+
+
+def heading_starts(k: int) -> np.ndarray:
+    """(k, 3, 3) rotations by theta_i = -pi + 2 pi i / k, i = 0 .. k-1 (``pose_to_mat((0, 0, theta_i))``):
+    a sweep of k headings for ``icp_multistart``, the guesses of bench.py's highres workload."""
+    k = int(k)
+    if k < 1:
+        raise ValueError("heading_starts needs k >= 1")
+    th = -np.pi + 2 * np.pi * np.arange(k) / k
+    return np.stack([pose_to_mat((0.0, 0.0, t)) for t in th])
+
+
+def compose_starts(init, starts) -> np.ndarray:
+    """(B, K, 3, 3): the guesses ``icp_multistart`` aligns from, G[p, k] = init[p] @ starts[k], with the
+    formula of include/icpb.h -- every product and sum rounded on its own, left to right, so the result
+    has the library's bits: ``icp_batch(scans, np.repeat(pairs, K, axis=0), G.reshape(-1, 3, 3))``
+    reproduces every problem of a multi-start run.  ``init`` is (B, 3, 3), or None for one identity
+    guess (B = 1)."""
+    S = np.asarray(starts, dtype=np.float64)
+    if S.ndim != 3 or S.shape[1:] != (3, 3):
+        raise ValueError(f"starts has shape {S.shape}; expected (K, 3, 3)")
+    I = np.eye(3)[None] if init is None else np.asarray(init, dtype=np.float64)
+    if I.ndim != 3 or I.shape[1:] != (3, 3):
+        raise ValueError(f"init has shape {I.shape}; expected (B, 3, 3)")
+    G = np.zeros((len(I), len(S), 3, 3))
+    for r in range(2):
+        a, c, t = I[:, None, r, 0], I[:, None, r, 1], I[:, None, r, 2]
+        G[:, :, r, 0] = a * S[None, :, 0, 0] + c * S[None, :, 1, 0]
+        G[:, :, r, 1] = a * S[None, :, 0, 1] + c * S[None, :, 1, 1]
+        G[:, :, r, 2] = (a * S[None, :, 0, 2] + c * S[None, :, 1, 2]) + t
+    G[:, :, 2, 2] = 1.0
+    return G
 
 
 class ScanList:
@@ -311,6 +367,35 @@ class IcpEngine:
             pad = np.arange(cap)[None, :] >= passes[:, None]
             history[pad] = np.eye(3)
         return BatchResult(_to33(T6), err, passes, history, corr)
+
+    # -- multi-start run on the resident table ---------------------------------------------------
+    def run_multistart(self, pairs, starts, init_transforms=None, epsilon=0.01, max_iters=100,
+                       stopping_thresh=0.0001, rotation_only=False, return_all=False,
+                       exhaustive: bool = False) -> MultiStartResult:
+        """Every pair aligned from ``init[p] @ starts[k]`` for every start k (icpb_run_multistart_host);
+        returns the winner per pair (the smallest k with the smallest error).  The library checks the
+        composed guesses against its bounds (ValueError)."""
+        if self.table is None:
+            raise ValueError("no scan table set")
+        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive)
+        pairs_a = np.ascontiguousarray(pairs, dtype=np.int32)
+        if pairs_a.size == 0:
+            pairs_a = pairs_a.reshape(0, 2)
+        if pairs_a.ndim != 2 or pairs_a.shape[1] != 2:
+            raise ValueError(f"pairs has shape {pairs_a.shape}; expected (B, 2) of (source, target) scan ids")
+        B = len(pairs_a)
+        S6 = _rows6(starts, None, "starts")
+        K = len(S6)
+        init6 = None if init_transforms is None else _rows6(init_transforms, B, "init_transforms")
+        T6, err = np.empty((B, 6)), np.empty(B)
+        passes, start = np.empty(B, dtype=np.int32), np.empty(B, dtype=np.int32)
+        err_all = np.empty((B, K)) if return_all else None
+        passes_all = np.empty((B, K), dtype=np.int32) if return_all else None
+        _lib.check(self._L.icpb_run_multistart_host(self._h, _ptr(pairs_a), _ptr(init6), B, _ptr(S6), K,
+                                                    ctypes.byref(p), _ptr(T6), _ptr(err), _ptr(passes),
+                                                    _ptr(start), _ptr(err_all), _ptr(passes_all)),
+                   "icpb_run_multistart_host")
+        return MultiStartResult(_to33(T6), err, passes, start=start, error_all=err_all, iters_all=passes_all)
 
     # -- upload + run in one call, upload overlapped with the kernels ---------------------------
     def align(self, scans, pairs, init_transforms=None, epsilon=0.01, max_iters=100, stopping_thresh=0.0001,
@@ -636,3 +721,19 @@ def icp_batch(scans, pairs, init_transforms=None, epsilon=0.01, max_iters=100, s
     e.set_scans(scans)
     return e.run(pairs, init_transforms, epsilon, max_iters, stopping_thresh, rotation_only,
                  return_history, return_correspondences)
+
+
+def icp_multistart(scans, pairs, starts, init_transforms=None, epsilon=0.01, max_iters=100, stopping_thresh=0.0001,
+                   rotation_only=False, return_all=False, device: int | None = None) -> MultiStartResult:
+    """Multi-start ``icp_batch``: pair p is aligned from ``init_transforms[p] @ starts[k]`` for every
+    start k ((K, 3, 3), e.g. ``heading_starts(32)``; identity guesses when ``init_transforms`` is None)
+    and the start with the smallest error wins (``np.argmin``'s rule: the first on ties).  Every start is
+    exactly the ``icp()`` call ``icp_batch`` makes for the guess ``compose_starts(init, starts)[p, k]``;
+    the expansion and the selection run on the device, so only B results cross PCIe.  ``return_all``
+    adds every start's error and pass count, (B, K).  ``scans`` is uploaded unless it is the ScanTable
+    already resident on the device."""
+    e = engine(device)
+    if not (isinstance(scans, ScanTable) and e.table is scans):
+        e.set_scans(scans)
+    return e.run_multistart(pairs, starts, init_transforms, epsilon, max_iters, stopping_thresh, rotation_only,
+                            return_all)

@@ -204,6 +204,41 @@ int icpb_run_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, i
                   const icpb_params *p, double *h_T, double *h_err, int32_t *h_passes,
                   double *h_hist, int32_t *h_corr);
 
+/*
+ * Multi-start alignment on the resident scan table: every pair is aligned from K shared start transforms
+ * and the start with the smallest error is returned -- the standard remedy for loop closures whose
+ * relative heading is unknown (a corridor driven the other way, an image match between scans taken
+ * facing different directions), where a single guess converges to the wrong minimum.
+ *   h_pairs   B x 2 int32 (source, target) scan ids, as icpb_run_host
+ *   h_init    B x 6 float64 per-pair guesses init[p], or NULL for the identity
+ *   h_starts  K x 6 float64 start transforms S[k] (2x3 rows like every guess), 1 <= K <= 2^22
+ * Problem (p, k) is exactly icp(scan[src_p], scan[dst_p], G[p,k], epsilon, max_iters, stopping_thresh,
+ * rotation_only) with G = init[p] . S[k]: the start acts in the source frame first, so a heading start
+ * turns the source scan about its own sensor origin and keeps the translation of init.  G is evaluated
+ * in float64, every product and sum rounded to nearest on its own (no FMA contraction), left to right:
+ *     G00 = I00*S00 + I01*S10     G01 = I00*S01 + I01*S11     G02 = (I00*S02 + I01*S12) + I02
+ *     G10 = I10*S00 + I11*S10     G11 = I10*S01 + I11*S11     G12 = (I10*S02 + I11*S12) + I12
+ * (numpy's element-wise * and + give the same bits), so every problem gives the bits icpb_run_host gives
+ * for the expanded pair list (pair p repeated K times, guesses G[p, 0..K-1]).  rotation_only zeroes the
+ * translation of G, as icp() does with its guess.
+ * Outputs per pair: the winning start's h_T (B x 6), h_err and h_passes, and h_start[p] = the smallest k
+ * with the smallest error (strict < over ascending k: np.argmin's rule, errors being finite within the
+ * bounds above).  Optional (NULL = not wanted): h_err_all (B x K float64) and h_passes_all (B x K int32),
+ * the results of every start, for callers that judge how ambiguous a match is.
+ * Rejected with ICPB_EINVAL before anything runs (the table stays usable): K outside 1 .. 2^22, null
+ * starts, a pair index out of range, hist_cap or corr_stride > 0 (for the winner's history rerun
+ * icpb_run_host on the winning guesses: each problem is deterministic, so the results are the same),
+ * pair_mode != 0, and any composed guess G outside the guess bounds (!(|v| <= bound), NaN included) --
+ * guesses and starts can each be within them while their product is not.
+ * The pairs run in slices of floor(2^22 / K) pairs, one alignment launch per slice (two when the table
+ * holds scans beyond shared memory and the slice is split by scan length), and a pair's K starts are
+ * next to each other in the queue.  Synchronous, like icpb_run_host.
+ */
+int icpb_run_multistart_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, int64_t B,
+                             const double *h_starts, int32_t K, const icpb_params *p,
+                             double *h_T, double *h_err, int32_t *h_passes, int32_t *h_start,
+                             double *h_err_all, int32_t *h_passes_all);
+
 /* icpb_upload_scans + icpb_run_host in one call with the upload overlapped with the kernels: the
  * scan table is copied in segments and every pair is launched as soon as both of its scans have
  * arrived.  Explicit pairs only, no history / correspondences.  This is what the Python
