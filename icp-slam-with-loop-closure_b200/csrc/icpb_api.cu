@@ -74,6 +74,7 @@ struct DeviceGuard {
 #endif
 constexpr int kPointsPerThread = ICPB_R;
 constexpr int kQueueRing = 64;
+constexpr int kQueueWords = kQueueRing + 3;       // the ring, the work counter, the two acceptance counters
 
 
 struct DevBuf {
@@ -109,6 +110,15 @@ struct PinnedBuf {
     }
     void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
 };
+
+// The layout of one synchronous call's arrays in the handle's scratch arena (icpb_ctx::arena): every
+// carve() names one array and returns its 256-byte-aligned offset; `used`, the total, is reserved once at
+// the top of the call, and at() turns an offset into the array.  Nothing carved outlives its call.
+struct Carve {
+    size_t used = 0;
+    size_t operator()(size_t bytes) { const size_t o = used; used += (bytes + 255) & ~size_t(255); return o; }
+};
+template <class T> T *at(const DevBuf &b, size_t o) { return (T *)((unsigned char *)b.p + o); }
 
 constexpr int kMaxSegments = 64;        // pieces of the streaming scan-table upload (icpb_align_host)
 
@@ -284,30 +294,34 @@ struct icpb_ctx {
     const double *xy = nullptr;
     const int64_t *offsets = nullptr;
     int64_t n_scans = 0, longest = 0;
-    DevBuf own_xy, own_off;
+    std::vector<int64_t> host_off;                  // the table's offsets on the host (table_host_offsets)
     // queue counters
-    unsigned long long *queue = nullptr;      // kQueueRing counters, then one work counter
+    unsigned long long *queue = nullptr;      // kQueueWords: kQueueRing counters, the work counter, then the
+                                              // acceptance epilogue's [appended, CTAs left] counters
     unsigned long long *executed = nullptr;   // non-null while work counting is enabled
     int64_t launches = 0;
-    // scratch for host-pointer entry points
-    DevBuf s_pairs, s_init, s_T, s_err, s_passes, s_hist, s_corr, s_pair_xy, s_pair_off;
+    // The scratch arrays of every entry point that synchronises before it returns, carved per call (Carve).
+    // Memory that outlives a call stays out of it:
+    //   own_xy, own_off  the resident table;
+    //   prep             the table's staging images, kept until the table changes;
+    //   s_big            launch()'s per-CTA scratch of the large-scan variant, also used by the asynchronous
+    //                    icpb_run_device*, whose kernels may still run when the next call starts (launches
+    //                    on different streams share it, as they share the acceptance counters);
+    //   stage, stage_xy  pinned: reallocating pinned memory is slow, and their sizes vary independently
+    //                    (the batch size and the table size).
+    DevBuf arena;
+    DevBuf own_xy, own_off;
     cudaStream_t stream = nullptr;
     cudaStream_t cstream[2] = {nullptr, nullptr};   // compute streams of the pipelined host entry point
-    cudaEvent_t seg_ev[16] = {};                    // "scan segment k has arrived"
-    cudaEvent_t done_ev[2] = {};
+    // align_impl: the arrival counter is zero / the pairs block is up / the kernel is done
+    cudaEvent_t counter_zeroed = nullptr, inputs_up = nullptr, kernel_done = nullptr;
     int32_t *arrived_dev = nullptr;                 // streaming upload: segments delivered so far
     // cuStreamWriteValue32 (driver API, looked up at run time): a stream-ordered 4-byte store, cheaper
     // than a 4-byte DMA for the "segment k has arrived" counter; nullptr -> the counter is copied
     int (*write32)(cudaStream_t, unsigned long long, unsigned int, unsigned int) = nullptr;
     int32_t *seg_vals_pinned = nullptr;             // 0..kMaxSegments in pinned host memory (sources of the flag copies)
-    DevBuf s_seg;
-    PinnedBuf stage;                                // pinned staging of the small per-call arrays
-    DevBuf s_sgd;                                   // pose-graph SGD: poses, edges, transforms, scratch
-    DevBuf s_grid;                                  // occupancy grid: poses, per-cell words, the grid
-    DevBuf s_accept;                                // acceptance epilogue: [appended, CTAs left] counters
+    PinnedBuf stage;                                // pinned staging of align_impl's per-pair blocks
     DevBuf s_big;                                   // large-scan variant: one scratch region per CTA
-    DevBuf s_order;                                 // queue order of a batch split by scan length
-    DevBuf s_ms;                                    // multi-start: a slice's pairs, guesses, order, results; the starts
     // per-scan staging images of the resident table (KernelArgs::prep_in), built on first use
     DevBuf prep;
     const double *prep_for = nullptr;               // the table (h->xy) the images were built from
@@ -321,13 +335,39 @@ struct icpb_ctx {
 
 namespace {
 
-// The handle's scan table; a new table has no staging images yet (ensure_prep).
-void set_table(icpb_ctx *h, const double *xy, const int64_t *off, int64_t n_scans, int64_t longest)
+// A pair fits the shared-memory kernel when the layout of its longer scan fits at the widest CTA a
+// launch may pick (8 warps), so that it fits whatever width the launch settles on.
+bool fits_smem(const icpb_ctx *h, int64_t n)
 {
-    h->prep_for = nullptr; h->xy = xy; h->offsets = off; h->n_scans = n_scans; h->longest = longest;
+    const icpb::SmemLayout L = icpb::smem_layout(n, 8);
+    return L.bytes != 0x7fffffff && L.bytes <= h->smem_limit;
 }
 
-void drop_table(icpb_ctx *h) { set_table(h, nullptr, nullptr, 0, 0); }
+// The handle's scan table; a new table has no staging images yet (ensure_prep).  off_host: the offsets
+// on the host, kept when a batch on the table may be split by scan length (null for a borrowed table).
+void set_table(icpb_ctx *h, const double *xy, const int64_t *off, int64_t n_scans, int64_t longest,
+               const int64_t *off_host)
+{
+    h->prep_for = nullptr; h->xy = xy; h->offsets = off; h->n_scans = n_scans; h->longest = longest;
+    h->host_off.clear();
+    if (off_host && !fits_smem(h, longest)) h->host_off.assign(off_host, off_host + n_scans + 1);
+}
+
+void drop_table(icpb_ctx *h) { set_table(h, nullptr, nullptr, 0, 0, nullptr); }
+
+// The table's offsets on the host, for split_queue: kept by set_table for a table from host memory,
+// fetched on first need for a borrowed one and kept until the next set_table.
+int table_host_offsets(icpb_ctx *h, const int64_t **out)
+{
+    if (h->host_off.empty()) {
+        std::vector<int64_t> off((size_t)h->n_scans + 1);
+        CU(cudaMemcpyAsync(off.data(), h->offsets, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaStreamSynchronize(h->stream));
+        h->host_off.swap(off);
+    }
+    *out = h->host_off.data();
+    return 0;
+}
 
 // A whole table from host memory into the handle's own buffers (reserved by the caller), which then hold
 // the handle's table.
@@ -336,7 +376,7 @@ int upload_table(icpb_ctx *h, const double *xy, const int64_t *off, int64_t n_sc
     CU(cudaMemcpyAsync(h->own_xy.p, xy, sizeof(double) * 2 * (size_t)off[n_scans], cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(h->own_off.p, off, sizeof(int64_t) * (size_t)(n_scans + 1), cudaMemcpyHostToDevice, h->stream));
     CU(cudaStreamSynchronize(h->stream));
-    set_table(h, (const double *)h->own_xy.p, (const int64_t *)h->own_off.p, n_scans, longest);
+    set_table(h, (const double *)h->own_xy.p, (const int64_t *)h->own_off.p, n_scans, longest, off);
     return 0;
 }
 
@@ -404,14 +444,6 @@ int make_cfg(icpb_ctx *h, int64_t longest, int64_t B, LaunchCfg *c, const icpb_p
     if (per_sm < 1) return fail(ICPB_EINVAL, "kernel does not fit on an SM%s");
     c->ctas_per_sm = per_sm;
     return 0;
-}
-
-// A pair fits the shared-memory kernel when the layout of its longer scan fits at the widest CTA a
-// launch may pick (8 warps), so that it fits whatever width the launch settles on.
-bool fits_smem(const icpb_ctx *h, int64_t n)
-{
-    const icpb::SmemLayout L = icpb::smem_layout(n, 8);
-    return L.bytes != 0x7fffffff && L.bytes <= h->smem_limit;
 }
 
 int check_params(const icpb_params *p, int64_t B)
@@ -553,14 +585,12 @@ int launch(icpb_ctx *h, const Batch &b)
             a.rec_row0 = ep->row0; a.rec_stride = ep->row_stride;
             if (ep->row_block > 0) a.rec_block = ep->row_block;
             if (ep->d_accept_rec || ep->d_accept_peer_ptrs) {
-                int rc2;
-                if ((rc2 = h->s_accept.reserve(2 * sizeof(unsigned long long)))) return rc2;
                 a.accept_thresh = ep->accept_thresh; a.accept_cap = ep->accept_cap; a.accept_rank = ep->rank;
                 a.accept_rec = ep->d_accept_peer_ptrs ? nullptr : ep->d_accept_rec;
                 a.accept_peers = (double *const *)ep->d_accept_peer_ptrs;
                 a.accept_count_peers = (long long *const *)ep->d_accept_count_peer_ptrs;
                 a.accept_count_out = (long long *)ep->d_accept_count;
-                a.accept_ctr = (unsigned long long *)h->s_accept.p;
+                a.accept_ctr = h->queue + kQueueRing + 1;
                 // [0] rows appended: zeroed by the first launch of a batch only; [1] CTAs that have left: per launch
                 const bool cont = q0 > 0;
                 CU(cudaMemsetAsync(a.accept_ctr + (cont ? 1 : 0), 0, (cont ? 1 : 2) * sizeof(unsigned long long), b.stream));
@@ -713,12 +743,12 @@ int icpb_create(int device, icpb_handle *out)
     if (!h) return fail(ICPB_EINVAL, "out of host memory%s");
     h->device = device;
     h->sm_count = prop.multiProcessorCount;
-    cudaError_t e = cudaMalloc(&h->queue, sizeof(unsigned long long) * (kQueueRing + 1));
-    if (e == cudaSuccess) e = cudaMemset(h->queue, 0, sizeof(unsigned long long) * (kQueueRing + 1));
+    cudaError_t e = cudaMalloc(&h->queue, sizeof(unsigned long long) * kQueueWords);
+    if (e == cudaSuccess) e = cudaMemset(h->queue, 0, sizeof(unsigned long long) * kQueueWords);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
     for (int k = 0; k < 2 && e == cudaSuccess; ++k) e = cudaStreamCreateWithFlags(&h->cstream[k], cudaStreamNonBlocking);
-    for (int k = 0; k < 16 && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&h->seg_ev[k], cudaEventDisableTiming);
-    for (int k = 0; k < 2 && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&h->done_ev[k], cudaEventDisableTiming);
+    for (cudaEvent_t *ev : {&h->counter_zeroed, &h->inputs_up, &h->kernel_done})
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
     // dynamic shared memory up to the device's opt-in maximum minus each kernel's static part, set
     // once: the attribute belongs to the function, not to a handle.  The large-scan variants keep only
     // a few KB in shared memory but ask for the same maximum; the limit a layout must fit comes from
@@ -778,16 +808,11 @@ int icpb_destroy(icpb_handle h)
     h->pool = nullptr;
     if (h->stream) { cudaStreamSynchronize(h->stream); cudaStreamDestroy(h->stream); }
     for (int k = 0; k < 2; ++k) if (h->cstream[k]) { cudaStreamSynchronize(h->cstream[k]); cudaStreamDestroy(h->cstream[k]); }
-    for (int k = 0; k < 16; ++k) if (h->seg_ev[k]) cudaEventDestroy(h->seg_ev[k]);
-    for (int k = 0; k < 2; ++k) if (h->done_ev[k]) cudaEventDestroy(h->done_ev[k]);
+    for (cudaEvent_t ev : {h->counter_zeroed, h->inputs_up, h->kernel_done}) if (ev) cudaEventDestroy(ev);
     if (h->arrived_dev) cudaFree(h->arrived_dev);
     if (h->seg_vals_pinned) cudaFreeHost(h->seg_vals_pinned);
-    h->s_seg.release(); h->stage.release(); h->s_sgd.release(); h->s_grid.release();
-    h->s_accept.release(); h->stage_xy.release(); h->prep.release(); h->s_big.release(); h->s_order.release(); h->s_ms.release();
-    h->own_xy.release(); h->own_off.release();
-    h->s_pairs.release(); h->s_init.release(); h->s_T.release(); h->s_err.release();
-    h->s_passes.release(); h->s_hist.release(); h->s_corr.release();
-    h->s_pair_xy.release(); h->s_pair_off.release();
+    h->arena.release(); h->own_xy.release(); h->own_off.release(); h->prep.release(); h->s_big.release();
+    h->stage.release(); h->stage_xy.release();
     if (h->queue) cudaFree(h->queue);
     delete h;
     return 0;
@@ -813,6 +838,7 @@ int icpb_upload_scans(icpb_handle h, const double *h_xy, const int64_t *h_offset
     int rc = validate_offsets(h_offsets, n_scans, &longest);
     if (rc) return rc;
     ON_DEVICE(h);
+    drop_table(h);                                  // reserving may free the old table's memory
     if ((rc = h->own_xy.reserve(sizeof(double) * 2 * (size_t)h_offsets[n_scans]))) return rc;
     if ((rc = h->own_off.reserve(sizeof(int64_t) * (size_t)(n_scans + 1)))) return rc;
     return upload_table(h, h_xy, h_offsets, n_scans, longest);
@@ -823,7 +849,7 @@ int icpb_set_scans_device(icpb_handle h, const double *d_xy, const int64_t *d_of
 {
     if (!h || !d_xy || !d_offsets || n_scans <= 0 || longest_scan <= 0)
         return fail(ICPB_EINVAL, "icpb_set_scans_device: bad argument%s");
-    set_table(h, d_xy, d_offsets, n_scans, longest_scan);
+    set_table(h, d_xy, d_offsets, n_scans, longest_scan, nullptr);
     return 0;
 }
 
@@ -870,7 +896,10 @@ int icpb_run_device_gather(icpb_handle h, const int32_t *d_pairs, const double *
     return icpb_run_device_ex(h, d_pairs, d_init, B, p, d_T, d_err, d_passes, &ep, stream);
 }
 
-static int run_host_common(icpb_handle h, const double *xy, const int64_t *offsets, int64_t n_scans,
+// A batch from host buffers on the handle's table (cloud null; host offsets from table_host_offsets if the
+// batch is split), or on a table of two clouds that go up with the call (icpb_icp_pair_host: cloud[0],
+// cloud[1] at the host offsets off).
+static int run_host_common(icpb_handle h, const double *const *cloud, const int64_t *off, int64_t n_scans,
                            int64_t longest, const int32_t *h_pairs, const double *h_init, int64_t B,
                            const icpb_params *p, double *h_T, double *h_err, int32_t *h_passes,
                            double *h_hist, int32_t *h_corr)
@@ -880,42 +909,49 @@ static int run_host_common(icpb_handle h, const double *xy, const int64_t *offse
     const size_t nbP = sizeof(int32_t) * 2 * (size_t)B, nbI = sizeof(double) * 6 * (size_t)B;
     const size_t nbH = sizeof(double) * 6 * (size_t)B * (size_t)p->hist_cap;
     const size_t nbC = sizeof(int32_t) * (size_t)B * (size_t)p->corr_stride;
-    if (p->pair_mode == 0) {
-        if ((rc = h->s_pairs.reserve(nbP))) return rc;
-        CU(cudaMemcpyAsync(h->s_pairs.p, h_pairs, nbP, cudaMemcpyHostToDevice, st));
-    }
-    if (h_init) {
-        if ((rc = h->s_init.reserve(nbI))) return rc;
-        CU(cudaMemcpyAsync(h->s_init.p, h_init, nbI, cudaMemcpyHostToDevice, st));
-    }
-    if ((rc = h->s_T.reserve(nbI))) return rc;
-    if ((rc = h->s_err.reserve(sizeof(double) * (size_t)B))) return rc;
-    if ((rc = h->s_passes.reserve(sizeof(int32_t) * (size_t)B))) return rc;
-    if (nbH) { if ((rc = h->s_hist.reserve(nbH))) return rc; CU(cudaMemsetAsync(h->s_hist.p, 0, nbH, st)); }
-    if (nbC) { if ((rc = h->s_corr.reserve(nbC))) return rc; CU(cudaMemsetAsync(h->s_corr.p, 0xff, nbC, st)); }
+    const bool split = needs_split(h, longest, B, p);
+    Carve c;
+    const size_t o_xy = c(cloud ? sizeof(double) * 2 * (size_t)off[n_scans] : 0);
+    const size_t o_off = c(cloud ? sizeof(int64_t) * (size_t)(n_scans + 1) : 0);
+    const size_t o_pairs = c(p->pair_mode == 0 ? nbP : 0), o_init = c(h_init ? nbI : 0);
+    const size_t o_T = c(nbI), o_err = c(sizeof(double) * (size_t)B), o_passes = c(sizeof(int32_t) * (size_t)B);
+    const size_t o_hist = c(nbH), o_corr = c(nbC), o_order = c(split ? sizeof(int32_t) * (size_t)B : 0);
+    if ((rc = h->arena.reserve(c.used))) return rc;
     Batch b;
-    b.xy = xy; b.offsets = offsets; b.n_scans = n_scans; b.longest = longest;
-    b.pairs = p->pair_mode == 0 ? (const int32_t *)h->s_pairs.p : nullptr;
-    b.init = h_init ? (const double *)h->s_init.p : nullptr; b.B = B; b.p = p;
-    b.T = (double *)h->s_T.p; b.err = (double *)h->s_err.p; b.passes = (int32_t *)h->s_passes.p;
-    b.hist = (double *)h->s_hist.p; b.corr = (int32_t *)h->s_corr.p; b.stream = st;
+    b.xy = h->xy; b.offsets = h->offsets; b.n_scans = n_scans; b.longest = longest;
+    if (cloud) {
+        double *xy = at<double>(h->arena, o_xy);
+        int64_t *d_off = at<int64_t>(h->arena, o_off);
+        CU(cudaMemcpyAsync(xy, cloud[0], sizeof(double) * 2 * (size_t)off[1], cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(xy + 2 * off[1], cloud[1], sizeof(double) * 2 * (size_t)(off[2] - off[1]),
+                           cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_off, off, sizeof(int64_t) * (size_t)(n_scans + 1), cudaMemcpyHostToDevice, st));
+        b.xy = xy; b.offsets = d_off;
+    }
+    int32_t *d_pairs = at<int32_t>(h->arena, o_pairs);
+    double *d_init = at<double>(h->arena, o_init);
+    b.pairs = p->pair_mode == 0 ? d_pairs : nullptr; b.init = h_init ? d_init : nullptr; b.B = B; b.p = p;
+    b.T = at<double>(h->arena, o_T); b.err = at<double>(h->arena, o_err); b.passes = at<int32_t>(h->arena, o_passes);
+    b.hist = at<double>(h->arena, o_hist); b.corr = at<int32_t>(h->arena, o_corr); b.stream = st;
+    if (p->pair_mode == 0) CU(cudaMemcpyAsync(d_pairs, h_pairs, nbP, cudaMemcpyHostToDevice, st));
+    if (h_init) CU(cudaMemcpyAsync(d_init, h_init, nbI, cudaMemcpyHostToDevice, st));
+    if (nbH) CU(cudaMemsetAsync(b.hist, 0, nbH, st));
+    if (nbC) CU(cudaMemsetAsync(b.corr, 0xff, nbC, st));
     Split sp;
-    if (needs_split(h, longest, B, p)) {
-        std::vector<int64_t> off((size_t)n_scans + 1);
+    if (split) {
+        if (!cloud && (rc = table_host_offsets(h, &off))) return rc;
         std::vector<int32_t> order((size_t)B);
-        CU(cudaMemcpyAsync(off.data(), offsets, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        sp = split_queue(h, off.data(), h_pairs, B, nullptr, order.data(), nullptr);
-        if ((rc = h->s_order.reserve(sizeof(int32_t) * (size_t)B))) return rc;
-        CU(cudaMemcpyAsync(h->s_order.p, order.data(), sizeof(int32_t) * (size_t)B, cudaMemcpyHostToDevice, st));
-        b.order = (const int32_t *)h->s_order.p; b.split = &sp;
+        sp = split_queue(h, off, h_pairs, B, nullptr, order.data(), nullptr);
+        int32_t *d_order = at<int32_t>(h->arena, o_order);
+        CU(cudaMemcpyAsync(d_order, order.data(), sizeof(int32_t) * (size_t)B, cudaMemcpyHostToDevice, st));
+        b.order = d_order; b.split = &sp;
     }
     if ((rc = launch(h, b))) return rc;
-    CU(cudaMemcpyAsync(h_T, h->s_T.p, nbI, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(h_err, h->s_err.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(h_passes, h->s_passes.p, sizeof(int32_t) * (size_t)B, cudaMemcpyDeviceToHost, st));
-    if (nbH) CU(cudaMemcpyAsync(h_hist, h->s_hist.p, nbH, cudaMemcpyDeviceToHost, st));
-    if (nbC) CU(cudaMemcpyAsync(h_corr, h->s_corr.p, nbC, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_T, b.T, nbI, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_err, b.err, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_passes, b.passes, sizeof(int32_t) * (size_t)B, cudaMemcpyDeviceToHost, st));
+    if (nbH) CU(cudaMemcpyAsync(h_hist, b.hist, nbH, cudaMemcpyDeviceToHost, st));
+    if (nbC) CU(cudaMemcpyAsync(h_corr, b.corr, nbC, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return 0;
 }
@@ -928,7 +964,7 @@ int icpb_run_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, i
     if (rc || B == 0) return rc;
     if (p->pair_mode == 0 && (rc = check_pairs(h_pairs, B, h->n_scans))) return rc;
     ON_DEVICE(h);
-    return run_host_common(h, h->xy, h->offsets, h->n_scans, h->longest, h_pairs, h_init, B, p,
+    return run_host_common(h, nullptr, nullptr, h->n_scans, h->longest, h_pairs, h_init, B, p,
                            h_T, h_err, h_passes, h_hist, h_corr);
 }
 
@@ -969,12 +1005,6 @@ int check_composed(const double *init, int64_t B, const double *S, int32_t K)
     return 0;
 }
 
-// Device-side arrays of one multi-start call, carved out of one buffer (256-byte aligned).
-struct MsArrays {
-    int32_t *pairs = nullptr, *pair_order = nullptr, *passes = nullptr, *start = nullptr;
-    double *init = nullptr, *starts = nullptr, *T = nullptr, *err = nullptr;
-};
-
 int run_multistart(icpb_ctx *h, const int32_t *h_pairs, const double *h_init, int64_t B, const double *h_starts,
                    int32_t K, const icpb_params *p_in, double *h_T, double *h_err, int32_t *h_passes, int32_t *h_start,
                    double *h_err_all, int32_t *h_passes_all)
@@ -983,73 +1013,64 @@ int run_multistart(icpb_ctx *h, const int32_t *h_pairs, const double *h_init, in
     cudaStream_t st = h->stream;
     const int64_t per = kMaxMultistart / K;                           // pairs per slice
     const int64_t n_max = B < per ? B : per, q_max = n_max * K;
-    // per-pair arrays of a slice and the K starts
-    size_t used = 0;
-    auto carve = [&](size_t bytes) { const size_t o = used; used += (bytes + 255) & ~size_t(255); return o; };
-    const size_t o_pairs = carve(8 * (size_t)n_max), o_init = carve(h_init ? 48 * (size_t)n_max : 0);
-    const size_t o_order = carve(4 * (size_t)n_max), o_starts = carve(48 * (size_t)K);
-    const size_t o_T = carve(48 * (size_t)n_max), o_err = carve(8 * (size_t)n_max);
-    const size_t o_passes = carve(4 * (size_t)n_max), o_start = carve(4 * (size_t)n_max);
-    if ((rc = h->s_ms.reserve(used))) return rc;
-    unsigned char *base = (unsigned char *)h->s_ms.p;
-    MsArrays d;
-    d.pairs = (int32_t *)(base + o_pairs); d.init = h_init ? (double *)(base + o_init) : nullptr;
-    d.pair_order = (int32_t *)(base + o_order); d.starts = (double *)(base + o_starts);
-    d.T = (double *)(base + o_T); d.err = (double *)(base + o_err);
-    d.passes = (int32_t *)(base + o_passes); d.start = (int32_t *)(base + o_start);
-    // the expanded problems of a slice, in the host entry point's scratch
-    if ((rc = h->s_pairs.reserve(8 * (size_t)q_max)) || (rc = h->s_init.reserve(48 * (size_t)q_max)) ||
-        (rc = h->s_T.reserve(48 * (size_t)q_max)) || (rc = h->s_err.reserve(8 * (size_t)q_max)) ||
-        (rc = h->s_passes.reserve(4 * (size_t)q_max)))
-        return rc;
-    int32_t *epairs = (int32_t *)h->s_pairs.p, *epasses = (int32_t *)h->s_passes.p;
-    double *eG = (double *)h->s_init.p, *eT = (double *)h->s_T.p, *eerr = (double *)h->s_err.p;
-    CU(cudaMemcpyAsync(d.starts, h_starts, 48 * (size_t)K, cudaMemcpyHostToDevice, st));
+    // a slice's pairs, guesses, queue order and results, the K starts, then the slice's expanded problems
+    // (a queue order only on a table that may be split: split_queue)
+    Carve c;
+    const size_t o_pairs = c(8 * (size_t)n_max), o_init = c(h_init ? 48 * (size_t)n_max : 0);
+    const size_t o_order = c(4 * (size_t)n_max), o_starts = c(48 * (size_t)K);
+    const size_t o_T = c(48 * (size_t)n_max), o_err = c(8 * (size_t)n_max);
+    const size_t o_passes = c(4 * (size_t)n_max), o_start = c(4 * (size_t)n_max);
+    const size_t o_epairs = c(8 * (size_t)q_max), o_eG = c(48 * (size_t)q_max), o_eT = c(48 * (size_t)q_max);
+    const size_t o_eerr = c(8 * (size_t)q_max), o_epasses = c(4 * (size_t)q_max);
+    const size_t o_eorder = c(fits_smem(h, h->longest) ? 0 : 4 * (size_t)q_max);
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    int32_t *d_pairs = at<int32_t>(h->arena, o_pairs), *d_order = at<int32_t>(h->arena, o_order);
+    double *d_init = h_init ? at<double>(h->arena, o_init) : nullptr, *d_starts = at<double>(h->arena, o_starts);
+    double *d_T = at<double>(h->arena, o_T), *d_err = at<double>(h->arena, o_err);
+    int32_t *d_passes = at<int32_t>(h->arena, o_passes), *d_start = at<int32_t>(h->arena, o_start);
+    int32_t *epairs = at<int32_t>(h->arena, o_epairs), *epasses = at<int32_t>(h->arena, o_epasses);
+    double *eG = at<double>(h->arena, o_eG), *eT = at<double>(h->arena, o_eT), *eerr = at<double>(h->arena, o_eerr);
+    int32_t *eorder = at<int32_t>(h->arena, o_eorder);
+    CU(cudaMemcpyAsync(d_starts, h_starts, 48 * (size_t)K, cudaMemcpyHostToDevice, st));
     icpb_params p = *p_in;
     p.k_first = 0; p.k_stride = 0;
-    std::vector<int64_t> off;                                         // the table's offsets, for a split
     std::vector<int32_t> pair_order;
     for (int64_t p0 = 0; p0 < B; p0 += per) {
         const int64_t n = B - p0 < per ? B - p0 : per, nq = n * K;
         p.k_block = nq;
-        CU(cudaMemcpyAsync(d.pairs, h_pairs + 2 * p0, 8 * (size_t)n, cudaMemcpyHostToDevice, st));
-        if (h_init) CU(cudaMemcpyAsync(d.init, h_init + 6 * p0, 48 * (size_t)n, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_pairs, h_pairs + 2 * p0, 8 * (size_t)n, cudaMemcpyHostToDevice, st));
+        if (h_init) CU(cudaMemcpyAsync(d_init, h_init + 6 * p0, 48 * (size_t)n, cudaMemcpyHostToDevice, st));
         Split sp;
         const bool split = needs_split(h, h->longest, nq, &p);
         if (split) {
-            if (off.empty()) {
-                off.resize((size_t)h->n_scans + 1);
-                CU(cudaMemcpyAsync(off.data(), h->offsets, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, st));
-                CU(cudaStreamSynchronize(st));
-            }
+            const int64_t *off;
+            if ((rc = table_host_offsets(h, &off))) return rc;
             // the slice's pairs in queue order; the expansion turns every pair into its K problems
             pair_order.resize((size_t)n);
-            const Split ps = split_queue(h, off.data(), h_pairs + 2 * p0, n, nullptr, pair_order.data(), nullptr);
+            const Split ps = split_queue(h, off, h_pairs + 2 * p0, n, nullptr, pair_order.data(), nullptr);
             sp.ns = ps.ns * K; sp.Ls = ps.Ls; sp.Ll = ps.Ll;
-            if ((rc = h->s_order.reserve(4 * (size_t)q_max))) return rc;
-            CU(cudaMemcpyAsync(d.pair_order, pair_order.data(), 4 * (size_t)n, cudaMemcpyHostToDevice, st));
+            CU(cudaMemcpyAsync(d_order, pair_order.data(), 4 * (size_t)n, cudaMemcpyHostToDevice, st));
         }
         int64_t blocks = (nq + icpb::kMultistartThreads - 1) / icpb::kMultistartThreads;
         if (blocks > 16 * (int64_t)h->sm_count) blocks = 16 * (int64_t)h->sm_count;
         icpb::multistart_expand_kernel<<<(unsigned)blocks, icpb::kMultistartThreads, 0, st>>>(
-            d.pairs, d.init, d.starts, K, n, split ? d.pair_order : nullptr, epairs, eG,
-            split ? (int32_t *)h->s_order.p : nullptr);
+            d_pairs, d_init, d_starts, K, n, split ? d_order : nullptr, epairs, eG, split ? eorder : nullptr);
         CU(cudaGetLastError());
         Batch b;
         b.xy = h->xy; b.offsets = h->offsets; b.n_scans = h->n_scans; b.longest = h->longest;
         b.pairs = epairs; b.init = eG; b.B = nq; b.p = &p;
         b.T = eT; b.err = eerr; b.passes = epasses; b.stream = st;
-        if (split) { b.order = (const int32_t *)h->s_order.p; b.split = &sp; }
+        if (split) { b.order = eorder; b.split = &sp; }
         if ((rc = launch(h, b))) return rc;
         blocks = (n + icpb::kMultistartThreads - 1) / icpb::kMultistartThreads;
         if (blocks > 16 * (int64_t)h->sm_count) blocks = 16 * (int64_t)h->sm_count;
         icpb::multistart_select_kernel<<<(unsigned)blocks, icpb::kMultistartThreads, 0, st>>>(
-            eT, eerr, epasses, K, n, d.T, d.err, d.passes, d.start);
+            eT, eerr, epasses, K, n, d_T, d_err, d_passes, d_start);
         CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(h_T + 6 * p0, d.T, 48 * (size_t)n, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(h_err + p0, d.err, 8 * (size_t)n, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(h_passes + p0, d.passes, 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(h_start + p0, d.start, 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_T + 6 * p0, d_T, 48 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_err + p0, d_err, 8 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_passes + p0, d_passes, 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_start + p0, d_start, 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
         // problem p_local * K + k is row p, column k of the (B, K) arrays
         if (h_err_all) CU(cudaMemcpyAsync(h_err_all + p0 * K, eerr, 8 * (size_t)nq, cudaMemcpyDeviceToHost, st));
         if (h_passes_all) CU(cudaMemcpyAsync(h_passes_all + p0 * K, epasses, 4 * (size_t)nq, cudaMemcpyDeviceToHost, st));
@@ -1356,16 +1377,44 @@ void get_transforms(double *t6, const double *src, int32_t ld, int64_t n)
     for (int64_t b = 0; b < n; ++b) memcpy(t6 + 6 * b, src + 9 * b, 6 * sizeof(double));
 }
 
-// icpb_align_host_accept's results: the n records the kernel appended as pairs finished (n < 0: more pairs
-// passed than the capacity, and -n of them), fetched and put in ascending pair order.
-int deliver_accepted(icpb_ctx *h, const AcceptHost *acc, int64_t n, cudaStream_t st)
+// align_impl's two per-pair blocks, each sent in one copy, at the same offsets in the pinned staging and in
+// its device mirror:  up = [init | pairs | seg | order],  down = [T | err | passes | timeout word], 8-byte
+// members first; after them the accepted count of icpb_align_host_accept.
+struct AlignBlocks {
+    struct Ptrs {
+        double *init; int32_t *pairs, *seg, *order;
+        double *T, *err; int32_t *passes, *timeout;
+        int64_t *accepted;
+    };
+    size_t init = 0, pairs, seg, order, up;                  // up: the end of the up block
+    size_t T, err, passes, timeout, down, accepted, bytes;   // down: bytes of the down block, T to timeout
+    explicit AlignBlocks(int64_t B)
+    {
+        const size_t n = (size_t)B;
+        pairs = init + sizeof(double) * 6 * n; seg = pairs + sizeof(int32_t) * 2 * n;
+        order = seg + sizeof(int32_t) * n; up = order + sizeof(int32_t) * n;
+        T = up; err = T + sizeof(double) * 6 * n; passes = err + sizeof(double) * n;
+        timeout = passes + sizeof(int32_t) * n; down = timeout + sizeof(int32_t) - T;
+        accepted = (timeout + sizeof(int32_t) + 7) & ~size_t(7); bytes = accepted + sizeof(int64_t);
+    }
+    Ptrs ptrs(void *base) const
+    {
+        unsigned char *b = (unsigned char *)base;
+        return {(double *)(b + init), (int32_t *)(b + pairs), (int32_t *)(b + seg), (int32_t *)(b + order),
+                (double *)(b + T), (double *)(b + err), (int32_t *)(b + passes), (int32_t *)(b + timeout),
+                (int64_t *)(b + accepted)};
+    }
+};
+
+// icpb_align_host_accept's results: the n records the kernel appended at d_rec as pairs finished (n < 0: more
+// pairs passed than the capacity, and -n of them), fetched and put in ascending pair order.
+int deliver_accepted(const AcceptHost *acc, const double *d_rec, int64_t n, cudaStream_t st)
 {
     *acc->n_out = n < 0 ? -n : n;
     if (n < 0) return fail(ICPB_EINVAL, "icpb_align_host_accept: more pairs accepted than the capacity given%s");
     std::vector<double> rec(8 * (size_t)n);
     if (n > 0) {
-        CU(cudaMemcpyAsync(rec.data(), (double *)h->s_hist.p + 2, sizeof(double) * 8 * (size_t)n,
-                           cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(rec.data(), d_rec, sizeof(double) * 8 * (size_t)n, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
     }
     std::vector<int64_t> idx((size_t)n);
@@ -1383,12 +1432,12 @@ int deliver_accepted(icpb_ctx *h, const AcceptHost *acc, int64_t n, cudaStream_t
     return 0;
 }
 
-// Every pair's results, from the pinned download area [T | err | passes] into the caller's arrays.
-void deliver_all(const double *down, int64_t B, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes)
+// Every pair's results, from the pinned down block into the caller's arrays.
+void deliver_all(const AlignBlocks::Ptrs &pin, int64_t B, double *h_T, int32_t T_ld, double *h_err, int32_t *h_passes)
 {
-    put_transforms(h_T, T_ld, down, B);
-    memcpy(h_err, down + 6 * B, sizeof(double) * (size_t)B);
-    memcpy(h_passes, down + 7 * B, sizeof(int32_t) * (size_t)B);
+    put_transforms(h_T, T_ld, pin.T, B);
+    memcpy(h_err, pin.err, sizeof(double) * (size_t)B);
+    memcpy(h_passes, pin.passes, sizeof(int32_t) * (size_t)B);
 }
 
 // A call without pairs: the table goes up whole (planned as one piece), and the handle owns it once it has landed.
@@ -1412,37 +1461,29 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     ON_DEVICE(h);
     const size_t nb_xy = sizeof(double) * 2 * (size_t)h_offsets[n_scans];
     const size_t nb_off = sizeof(int64_t) * (size_t)(n_scans + 1);
-    if ((rc = h->own_xy.reserve(nb_xy))) return rc;
-    if ((rc = h->own_off.reserve(nb_off))) return rc;
     if (src.scan_xy && (rc = h->stage_xy.reserve(nb_xy))) return rc;
     int nseg = 0;
     int64_t seg_end[kMaxSegments];                            // exclusive scan id
     if ((rc = icpb_plan_upload(h_offsets, n_scans, B == 0 ? 1 : h->tune_segments, seg_end, &nseg))) return rc;
-    // pinned staging, 8-byte members first:  up = [init | pairs | seg | order],  down = [T | err | passes]
-    const size_t nbI = sizeof(double) * 6 * (size_t)B, nbE = sizeof(double) * (size_t)B, nb4 = sizeof(int32_t) * (size_t)B;
-    const size_t nb_up = nbI + 4 * nb4, nb_down = nbI + nbE + nb4 + sizeof(int32_t);   // + the "upload timed out" word
-    if ((rc = h->stage.reserve(nb_up + nb_down + 32))) return rc;
-    if ((rc = h->s_init.reserve(nb_up))) return rc;
-    if ((rc = h->s_T.reserve(nb_down))) return rc;
+    // the per-pair blocks, pinned and on the device; on the device also the accepted records
+    const AlignBlocks blk(B);
+    Carve c;
+    const size_t o_blk = c(blk.bytes), o_rec = c(acc ? sizeof(double) * 8 * (size_t)acc->cap : 0);
+    if ((rc = h->stage.reserve(blk.bytes))) return rc;
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    unsigned char *pin_base = (unsigned char *)h->stage.p, *dev_base = at<unsigned char>(h->arena, o_blk);
+    const AlignBlocks::Ptrs pin = blk.ptrs(pin_base), dev = blk.ptrs(dev_base);
+    double *d_rec = at<double>(h->arena, o_rec);
     icpb_epilogue ep_acc;
     if (acc) {
-        // acceptance on the device: compact records + their count in device scratch, fetched at the end
-        if ((rc = h->s_hist.reserve(sizeof(double) * 8 * (size_t)acc->cap + 16))) return rc;
+        // acceptance on the device: compact records and their count, fetched at the end
         if (ep) ep_acc = *ep; else memset(&ep_acc, 0, sizeof ep_acc);
         ep_acc.accept_thresh = acc->thresh; ep_acc.accept_cap = acc->cap;
-        ep_acc.d_accept_count = (int64_t *)h->s_hist.p;
-        ep_acc.d_accept_rec = (double *)h->s_hist.p + 2;
+        ep_acc.d_accept_count = dev.accepted;
+        ep_acc.d_accept_rec = d_rec;
         ep_acc.d_accept_peer_ptrs = nullptr; ep_acc.d_accept_count_peer_ptrs = nullptr;
         ep = &ep_acc;
     }
-    double *pinit = (double *)h->stage.p;
-    int32_t *ppairs = (int32_t *)(pinit + 6 * B), *pseg = ppairs + 2 * B, *porder = pseg + B;
-    double *tT = (double *)((char *)h->stage.p + nb_up);
-    int32_t *tP = (int32_t *)(tT + 7 * B);
-    double *d_init = (double *)h->s_init.p;
-    int32_t *d_pairs = (int32_t *)(d_init + 6 * B), *d_seg = d_pairs + 2 * B, *d_order = d_seg + B;
-    double *d_T = (double *)h->s_T.p, *d_err = d_T + 6 * B;
-    int32_t *d_passes = (int32_t *)(d_err + B);
 
     // The packers (list input) start now, so they work while the caller's pairs and initial guesses are checked
     ListPacker packer;
@@ -1451,35 +1492,37 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     if ((rc = check_align_inputs(h_pairs, h_init, init_ld, B, n_scans))) return rc;
     // ---- from here on the handle's table is being replaced: a failure leaves it without one ----
     drop_table(h);
+    if ((rc = h->own_xy.reserve(nb_xy))) return rc;
+    if ((rc = h->own_off.reserve(nb_off))) return rc;
     if (B == 0) return upload_only(h, src, packer, up_xy, n_scans, longest);
     cudaStream_t cp = h->stream, cp2 = h->cstream[1], cs = h->cstream[0];
     // The first pieces start NOW, before the per-pair staging below: the copy engine works while the
     // host sorts and packs (everything has been validated above; nothing below can fail on user input).
     CUA(cudaMemsetAsync(h->arrived_dev, 0, sizeof(int32_t), cp));
-    CUA(cudaEventRecord(h->seg_ev[1], cp));                   // the counter is zero before the kernel may start
+    CUA(cudaEventRecord(h->counter_zeroed, cp));              // the counter is zero before the kernel may start
     int n_sent = 0;
     if (!src.scan_xy)
         for (; n_sent < (nseg < 4 ? nseg : 4); ++n_sent) CUA(enqueue_piece(h, up_xy, h_offsets, seg_end, n_sent));
     const QueueOrder qo = order_queue(h, h_offsets, n_scans, longest, seg_end, nseg, h_pairs, B, p,
-                                      tP /* the download area is free until the end */, porder, pseg);
-    memcpy(ppairs, h_pairs, 2 * nb4);
-    if (h_init) get_transforms(pinit, h_init, init_ld, B);
-    // the small per-pair block goes up on a second copy stream, beside the pieces already in flight
-    CUA(cudaMemsetAsync(d_passes + B, 0, sizeof(int32_t), cp2));
+                                      pin.passes /* the down block is free until the end */, pin.order, pin.seg);
+    memcpy(pin.pairs, h_pairs, sizeof(int32_t) * 2 * (size_t)B);
+    if (h_init) get_transforms(pin.init, h_init, init_ld, B);
+    // the up block goes on a second copy stream, beside the pieces already in flight: from the guesses (or the
+    // pairs) to the piece numbers (or the queue order)
+    CUA(cudaMemsetAsync(dev.timeout, 0, sizeof(int32_t), cp2));
     CUA(cudaMemcpyAsync(h->own_off.p, h_offsets, nb_off, cudaMemcpyHostToDevice, cp2));
-    const size_t nb_idx = (qo.in_order ? 3 : 4) * nb4;        // pairs, seg (, order)
-    if (h_init) CUA(cudaMemcpyAsync(d_init, pinit, nbI + nb_idx, cudaMemcpyHostToDevice, cp2));
-    else        CUA(cudaMemcpyAsync(d_pairs, ppairs, nb_idx, cudaMemcpyHostToDevice, cp2));
-    CUA(cudaEventRecord(h->seg_ev[0], cp2));
+    const size_t up0 = h_init ? blk.init : blk.pairs, up1 = qo.in_order ? blk.order : blk.up;
+    CUA(cudaMemcpyAsync(dev_base + up0, pin_base + up0, up1 - up0, cudaMemcpyHostToDevice, cp2));
+    CUA(cudaEventRecord(h->inputs_up, cp2));
     // ONE launch over all pairs, in arrival order; its CTAs wait on the segment counter
-    CUA(cudaStreamWaitEvent(cs, h->seg_ev[0], 0));
-    CUA(cudaStreamWaitEvent(cs, h->seg_ev[1], 0));
+    CUA(cudaStreamWaitEvent(cs, h->inputs_up, 0));
+    CUA(cudaStreamWaitEvent(cs, h->counter_zeroed, 0));
     Batch bt;
     bt.xy = (const double *)h->own_xy.p; bt.offsets = (const int64_t *)h->own_off.p; bt.n_scans = n_scans;
-    bt.longest = longest; bt.pairs = d_pairs; bt.init = h_init ? d_init : nullptr; bt.B = B; bt.p = p;
-    bt.T = d_T; bt.err = d_err; bt.passes = d_passes;
-    bt.stream = cs; bt.ep = ep; bt.order = qo.in_order ? nullptr : d_order;
-    bt.seg_of_pair = d_seg; bt.arrived = h->arrived_dev; bt.upload_timeout = d_passes + B;
+    bt.longest = longest; bt.pairs = dev.pairs; bt.init = h_init ? dev.init : nullptr; bt.B = B; bt.p = p;
+    bt.T = dev.T; bt.err = dev.err; bt.passes = dev.passes;
+    bt.stream = cs; bt.ep = ep; bt.order = qo.in_order ? nullptr : dev.order;
+    bt.seg_of_pair = dev.seg; bt.arrived = h->arrived_dev; bt.upload_timeout = dev.timeout;
     bt.split = qo.split ? &qo.sp : nullptr;
     if ((rc = launch(h, bt))) return align_abort(h, rc);
     for (int k = n_sent; k < nseg; ++k) {
@@ -1488,34 +1531,33 @@ int align_impl(icpb_handle h, const TableSrc &src, int64_t n_scans, int64_t long
     }
     if (packer.finish()) {
         // the kernel is waiting for pieces that will not come: raise its give-up flag, drain, report
-        CUA(cudaMemcpyAsync(d_passes + B, h->seg_vals_pinned + 1, sizeof(int32_t), cudaMemcpyHostToDevice, cp));
+        CUA(cudaMemcpyAsync(dev.timeout, h->seg_vals_pinned + 1, sizeof(int32_t), cudaMemcpyHostToDevice, cp));
         return align_abort(h, fail(ICPB_EINVAL, "scan table holds non-finite coordinates or coordinates beyond ICPB_MAX_COORD%s"));
     }
-    CUA(cudaEventRecord(h->done_ev[0], cs));
-    CUA(cudaStreamWaitEvent(cp, h->done_ev[0], 0));
-    int64_t *acc_cnt = (int64_t *)(tP + B + 2);               // pinned: [timeout word | pad | accepted count]
+    CUA(cudaEventRecord(h->kernel_done, cs));
+    CUA(cudaStreamWaitEvent(cp, h->kernel_done, 0));
     if (!acc) {
-        CUA(cudaMemcpyAsync(tT, d_T, nb_down, cudaMemcpyDeviceToHost, cp));
+        CUA(cudaMemcpyAsync(pin.T, dev.T, blk.down, cudaMemcpyDeviceToHost, cp));
     } else {                                                  // the timeout word and the count, not the results
-        CUA(cudaMemcpyAsync(tP + B, d_passes + B, sizeof(int32_t), cudaMemcpyDeviceToHost, cp));
-        CUA(cudaMemcpyAsync(acc_cnt, h->s_hist.p, sizeof(int64_t), cudaMemcpyDeviceToHost, cp));
+        CUA(cudaMemcpyAsync(pin.timeout, dev.timeout, sizeof(int32_t), cudaMemcpyDeviceToHost, cp));
+        CUA(cudaMemcpyAsync(pin.accepted, dev.accepted, sizeof(int64_t), cudaMemcpyDeviceToHost, cp));
     }
     CUA(cudaStreamSynchronize(cp));
-    if (tP[B] != 0) {
+    if (*pin.timeout != 0) {
         // a CTA gave up waiting for its scans (see the kernel): by now the whole table is resident,
         // so run the batch again without the streaming protocol
         Batch again = bt;
         again.seg_of_pair = nullptr; again.arrived = nullptr; again.upload_timeout = nullptr;
         again.stream = cp;
         if ((rc = launch(h, again))) return align_abort(h, rc);
-        if (!acc) CUA(cudaMemcpyAsync(tT, d_T, nb_down, cudaMemcpyDeviceToHost, cp));
-        else      CUA(cudaMemcpyAsync(acc_cnt, h->s_hist.p, sizeof(int64_t), cudaMemcpyDeviceToHost, cp));
+        if (!acc) CUA(cudaMemcpyAsync(pin.T, dev.T, blk.down, cudaMemcpyDeviceToHost, cp));
+        else      CUA(cudaMemcpyAsync(pin.accepted, dev.accepted, sizeof(int64_t), cudaMemcpyDeviceToHost, cp));
         CUA(cudaStreamSynchronize(cp));
     }
     // only now does the handle own the new table
-    set_table(h, bt.xy, bt.offsets, n_scans, longest);
-    if (acc) return deliver_accepted(h, acc, *acc_cnt, cp);
-    deliver_all(tT, B, h_T, T_ld, h_err, h_passes);
+    set_table(h, bt.xy, bt.offsets, n_scans, longest, h_offsets);
+    if (acc) return deliver_accepted(acc, d_rec, *pin.accepted, cp);
+    deliver_all(pin, B, h_T, T_ld, h_err, h_passes);
     return 0;
 }
 
@@ -1641,17 +1683,10 @@ int icpb_icp_pair_host(icpb_handle h, const double *h_src_xy, int64_t n_src,
     icpb_params q = *p;
     q.pair_mode = 0; q.k_first = 0; q.k_block = 1; q.k_stride = 0;
     ON_DEVICE(h);
-    const size_t nb = sizeof(double) * 2 * (size_t)(n_src + n_dst);
-    if ((rc = h->s_pair_xy.reserve(nb))) return rc;
-    if ((rc = h->s_pair_off.reserve(sizeof(int64_t) * 3))) return rc;
+    const double *const cloud[2] = {h_src_xy, h_dst_xy};
     const int64_t off[3] = {0, n_src, n_src + n_dst};
     const int32_t pair[2] = {0, 1};
-    double *dxy = (double *)h->s_pair_xy.p;
-    CU(cudaMemcpyAsync(dxy, h_src_xy, sizeof(double) * 2 * (size_t)n_src, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(dxy + 2 * n_src, h_dst_xy, sizeof(double) * 2 * (size_t)n_dst, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->s_pair_off.p, off, sizeof off, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaStreamSynchronize(h->stream));       // `off` lives on this stack frame
-    return run_host_common(h, dxy, (const int64_t *)h->s_pair_off.p, 2, n_src > n_dst ? n_src : n_dst,
+    return run_host_common(h, cloud, off, 2, n_src > n_dst ? n_src : n_dst,
                            pair, h_init6, 1, &q, h_T6, h_err, h_passes, h_hist, h_corr);
 }
 
@@ -1663,16 +1698,17 @@ int icpb_fit_pairs_host(icpb_handle h, const double *h_a_xy, const double *h_b_x
     ON_DEVICE(h);
     int rc;
     const size_t nb = sizeof(double) * 2 * (size_t)n;
-    if ((rc = h->s_pair_xy.reserve(2 * nb))) return rc;
-    if ((rc = h->s_T.reserve(sizeof(double) * 8))) return rc;
-    double *da = (double *)h->s_pair_xy.p, *db = da + 2 * n;
+    double out[7];                                            // [T (6) | error]
+    Carve c;
+    const size_t o_a = c(nb), o_b = c(nb), o_out = c(sizeof out);
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    double *da = at<double>(h->arena, o_a), *db = at<double>(h->arena, o_b), *dout = at<double>(h->arena, o_out);
     CU(cudaMemcpyAsync(da, h_a_xy, nb, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(db, h_b_xy, nb, cudaMemcpyHostToDevice, h->stream));
     icpb::fit_pairs_kernel<<<1, 256, 0, h->stream>>>((const double2 *)da, (const double2 *)db, (int)n,
-                                                     (double *)h->s_T.p, (double *)h->s_T.p + 6);
+                                                     dout, dout + 6);
     CU(cudaGetLastError());
-    double out[7];
-    CU(cudaMemcpyAsync(out, h->s_T.p, sizeof out, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(out, dout, sizeof out, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
     memcpy(h_T6, out, 6 * sizeof(double));
     *h_err = out[6];
@@ -1680,14 +1716,10 @@ int icpb_fit_pairs_host(icpb_handle h, const double *h_a_xy, const double *h_b_x
 }
 
 static int upload_poses(icpb_handle h, const double *h_xy, const double *h_travelled, int64_t n,
-                        double **d_xy, double **d_trav)
+                        double *d_xy, double *d_trav)
 {
-    int rc;
-    if ((rc = h->s_pair_xy.reserve(sizeof(double) * 3 * (size_t)n))) return rc;
-    *d_xy = (double *)h->s_pair_xy.p;
-    *d_trav = *d_xy + 2 * n;
-    CU(cudaMemcpyAsync(*d_xy, h_xy, sizeof(double) * 2 * (size_t)n, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(*d_trav, h_travelled, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_xy, h_xy, sizeof(double) * 2 * (size_t)n, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_trav, h_travelled, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
     return 0;
 }
 
@@ -1715,18 +1747,20 @@ int icpb_proximity_closest(icpb_handle h, const double *h_xy, const double *h_tr
     int rc = proximity_check(h_xy, h_travelled, n, min_dist_along_path, "icpb_proximity_closest");
     if (rc) return rc;
     ON_DEVICE(h);
-    double *d_xy, *d_trav;
-    rc = upload_poses(h, h_xy, h_travelled, n, &d_xy, &d_trav);
-    if (rc) return rc;
-    if ((rc = h->s_passes.reserve(sizeof(int32_t) * (size_t)n))) return rc;
-    if ((rc = h->s_err.reserve(sizeof(double) * (size_t)n))) return rc;
+    Carve c;
+    const size_t o_xy = c(sizeof(double) * 2 * (size_t)n), o_trav = c(sizeof(double) * (size_t)n);
+    const size_t o_closest = c(sizeof(int32_t) * (size_t)n), o_dist = c(sizeof(double) * (size_t)n);
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    double *d_xy = at<double>(h->arena, o_xy), *d_trav = at<double>(h->arena, o_trav);
+    int32_t *d_closest = at<int32_t>(h->arena, o_closest);
+    double *d_dist = at<double>(h->arena, o_dist);
+    if ((rc = upload_poses(h, h_xy, h_travelled, n, d_xy, d_trav))) return rc;
     const unsigned grid = (unsigned)((n * 32 + 255) / 256);
     icpb::proximity_closest_kernel<<<grid, 256, 0, h->stream>>>((const double2 *)d_xy, d_trav, (int)n,
-                                                                min_dist_along_path, max_dist,
-                                                                (int32_t *)h->s_passes.p, (double *)h->s_err.p);
+                                                                min_dist_along_path, max_dist, d_closest, d_dist);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(h_closest, h->s_passes.p, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaMemcpyAsync(h_dist, h->s_err.p, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(h_closest, d_closest, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(h_dist, d_dist, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
     return 0;
 }
@@ -1741,11 +1775,18 @@ int icpb_proximity_pairs(icpb_handle h, const double *h_xy, const double *h_trav
     int rc = proximity_check(h_xy, h_travelled, n, min_dist_along_path, "icpb_proximity_pairs");
     if (rc) return rc;
     ON_DEVICE(h);
-    double *d_xy, *d_trav;
-    rc = upload_poses(h, h_xy, h_travelled, n, &d_xy, &d_trav);
-    if (rc) return rc;
-    if ((rc = h->s_T.reserve(sizeof(int64_t) * 2 * (size_t)n))) return rc;
-    int64_t *d_count = (int64_t *)h->s_T.p, *d_off = d_count + n;
+    // The pairs are carved at the caller's capacity (the count from a capacity-0 call; n * n bounds any
+    // count): the arena is reserved before the count is known, and a later reservation would free the poses.
+    const int64_t rows = capacity < n * n ? capacity : n * n;
+    Carve c;
+    const size_t o_xy = c(sizeof(double) * 2 * (size_t)n), o_trav = c(sizeof(double) * (size_t)n);
+    const size_t o_count = c(sizeof(int64_t) * (size_t)n), o_off = c(sizeof(int64_t) * (size_t)n);
+    const size_t o_pairs = c(sizeof(int32_t) * 2 * (size_t)rows);
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    double *d_xy = at<double>(h->arena, o_xy), *d_trav = at<double>(h->arena, o_trav);
+    int64_t *d_count = at<int64_t>(h->arena, o_count), *d_off = at<int64_t>(h->arena, o_off);
+    int32_t *d_pairs = at<int32_t>(h->arena, o_pairs);
+    if ((rc = upload_poses(h, h_xy, h_travelled, n, d_xy, d_trav))) return rc;
     const unsigned grid = (unsigned)((n * 32 + 255) / 256);
     icpb::proximity_pairs_kernel<false><<<grid, 256, 0, h->stream>>>((const double2 *)d_xy, d_trav, (int)n,
                                                                      min_dist_along_path, max_dist,
@@ -1759,13 +1800,12 @@ int icpb_proximity_pairs(icpb_handle h, const double *h_xy, const double *h_trav
     *n_pairs = total;
     if (capacity == 0 || total == 0) return 0;                                // size query
     if (total > capacity) return fail(ICPB_EINVAL, "icpb_proximity_pairs: capacity too small%s");
-    if ((rc = h->s_pairs.reserve(sizeof(int32_t) * 2 * (size_t)total))) return rc;
     CU(cudaMemcpyAsync(d_off, off.data(), sizeof(int64_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
     icpb::proximity_pairs_kernel<true><<<grid, 256, 0, h->stream>>>((const double2 *)d_xy, d_trav, (int)n,
                                                                     min_dist_along_path, max_dist,
-                                                                    nullptr, d_off, (int32_t *)h->s_pairs.p);
+                                                                    nullptr, d_off, d_pairs);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(h_pairs, h->s_pairs.p, sizeof(int32_t) * 2 * (size_t)total, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(h_pairs, d_pairs, sizeof(int32_t) * 2 * (size_t)total, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
     return 0;
 }
@@ -1814,8 +1854,10 @@ int icpb_compose_chain_gpu(icpb_handle h, const double *pose0, const double *h_T
         return fail(ICPB_EINVAL, "icpb_compose_chain_gpu: bad argument%s");
     ON_DEVICE(h);
     int rc;
-    if ((rc = h->s_pair_xy.reserve(sizeof(double) * (6 * (size_t)n + 3 * (size_t)(n + 1))))) return rc;
-    double *d_T = (double *)h->s_pair_xy.p, *d_P = d_T + 6 * n;
+    Carve c;
+    const size_t o_T = c(sizeof(double) * 6 * (size_t)n), o_P = c(sizeof(double) * 3 * (size_t)(n + 1));
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    double *d_T = at<double>(h->arena, o_T), *d_P = at<double>(h->arena, o_P);
     if (n > 0) CU(cudaMemcpyAsync(d_T, h_T6, sizeof(double) * 6 * (size_t)n, cudaMemcpyHostToDevice, h->stream));
     if ((rc = icpb_compose_chain_device(h, pose0, d_T, n, d_P, h->stream))) return rc;
     CU(cudaMemcpyAsync(h_poses_out, d_P, sizeof(double) * 3 * (size_t)(n + 1), cudaMemcpyDeviceToHost, h->stream));
@@ -1849,14 +1891,18 @@ int icpb_pose_graph_sgd(icpb_handle h, double *h_poses, int64_t n, const int32_t
     if (ve.empty() || n_steps == 0) return 0;
     ON_DEVICE(h);
     const size_t E = ve.size() / 2, N = (size_t)n;
-    // [RECA 10E | tf 6E | dW 4E | REC 10E | ES 23E | poses 3N | M 3N | P 3N] doubles, then [edges 2E] int32
-    // (RECA first: its 80-byte records are read as 16-byte pairs)
-    const size_t n_dbl = 10 * E + 6 * E + 4 * E + 10 * E + 23 * E + 3 * N + 3 * N + 3 * N;
+    // (RECA's 80-byte records are read as 16-byte pairs: the 256-byte alignment of a carved array covers it)
+    const size_t D = sizeof(double);
+    Carve c;
+    const size_t o_RECA = c(D * 10 * E), o_tf = c(D * 6 * E), o_dW = c(D * 4 * E), o_REC = c(D * 10 * E);
+    const size_t o_ES = c(D * 23 * E), o_poses = c(D * 3 * N), o_M = c(D * 3 * N), o_P = c(D * 3 * N);
+    const size_t o_edges = c(sizeof(int32_t) * 2 * E);
     int rc;
-    if ((rc = h->s_sgd.reserve(sizeof(double) * n_dbl + sizeof(int32_t) * 2 * E))) return rc;
-    double *d_RECA = (double *)h->s_sgd.p, *d_tf = d_RECA + 10 * E, *d_dW = d_tf + 6 * E;
-    double *d_REC = d_dW + 4 * E, *d_ES = d_REC + 10 * E, *d_poses = d_ES + 23 * E, *d_M = d_poses + 3 * N, *d_P = d_M + 3 * N;
-    int32_t *d_edges = (int32_t *)(d_P + 3 * N);
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    double *d_RECA = at<double>(h->arena, o_RECA), *d_tf = at<double>(h->arena, o_tf), *d_dW = at<double>(h->arena, o_dW);
+    double *d_REC = at<double>(h->arena, o_REC), *d_ES = at<double>(h->arena, o_ES);
+    double *d_poses = at<double>(h->arena, o_poses), *d_M = at<double>(h->arena, o_M), *d_P = at<double>(h->arena, o_P);
+    int32_t *d_edges = at<int32_t>(h->arena, o_edges);
     CU(cudaMemcpyAsync(d_poses, h_poses, sizeof(double) * 3 * N, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(d_tf, vt.data(), sizeof(double) * 6 * E, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(d_edges, ve.data(), sizeof(int32_t) * 2 * E, cudaMemcpyHostToDevice, h->stream));
@@ -1940,10 +1986,12 @@ int icpb_occupancy_grid_bounds(icpb_handle h, const double *h_poses, int64_t n, 
     if (!isfinite(min_width) || !isfinite(min_height))
         return fail(ICPB_EINVAL, "icpb_occupancy_grid_bounds: non-finite minimum size%s");
     ON_DEVICE(h);
-    if ((rc = h->s_grid.reserve(sizeof(double) * 4 * (size_t)n + 4 * sizeof(unsigned long long)))) return rc;
-    unsigned long long *d_mm = (unsigned long long *)h->s_grid.p;
-    double *d_poses = (double *)(d_mm + 4);
     const unsigned long long init[4] = {~0ULL, ~0ULL, 0ULL, 0ULL};
+    Carve c;
+    const size_t o_mm = c(sizeof init), o_poses = c(sizeof(double) * 4 * (size_t)n);
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    unsigned long long *d_mm = at<unsigned long long>(h->arena, o_mm);
+    double *d_poses = at<double>(h->arena, o_poses);
     const std::vector<double> rec = pose_records(h_poses, n);
     CU(cudaMemcpyAsync(d_mm, init, sizeof init, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(d_poses, rec.data(), sizeof(double) * 4 * (size_t)n, cudaMemcpyHostToDevice, h->stream));
@@ -1989,11 +2037,13 @@ int icpb_occupancy_grid_update(icpb_handle h, const double *h_poses, int64_t n, 
     CU(cudaMemcpy(&n_points, h->offsets + n, sizeof n_points, cudaMemcpyDeviceToHost));
     if (n_points >= 0x7ffffffeLL) return fail(ICPB_EINVAL, "icpb_occupancy_grid_update: more than 2^31 - 2 beams in one call%s");
     const size_t cells = (size_t)height * (size_t)width;
-    const size_t words = 4 * cells;
-    if ((rc = h->s_grid.reserve(sizeof(double) * 4 * (size_t)n + sizeof(uint32_t) * words + cells + 64))) return rc;
-    double *d_poses = (double *)h->s_grid.p;
-    uint32_t *d_words = (uint32_t *)(d_poses + 4 * (size_t)n);
-    int8_t *d_grid = (int8_t *)(d_words + words);
+    const size_t words = 4 * cells;                          // [last_hit | n_miss | n_hit | miss_after], per cell
+    Carve c;
+    const size_t o_poses = c(sizeof(double) * 4 * (size_t)n), o_words = c(sizeof(uint32_t) * words), o_grid = c(cells);
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    double *d_poses = at<double>(h->arena, o_poses);
+    uint32_t *d_words = at<uint32_t>(h->arena, o_words);
+    int8_t *d_grid = at<int8_t>(h->arena, o_grid);
     const std::vector<double> rec = pose_records(h_poses, n);
     CU(cudaMemcpyAsync(d_poses, rec.data(), sizeof(double) * 4 * (size_t)n, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(d_grid, h_grid, cells, cudaMemcpyHostToDevice, h->stream));
