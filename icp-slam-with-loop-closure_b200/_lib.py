@@ -23,7 +23,8 @@ EXPORTS = ["icpb_default_params", "icpb_abi_version", "icpb_create", "icpb_destr
            "icpb_run_device_gather", "icpb_pose_graph_sgd", "icpb_occupancy_grid_bounds",
            "icpb_occupancy_grid_update", "icpb_run_device_ex", "icpb_align_host_ex", "icpb_align_host_scans",
            "icpb_set_tuning", "icpb_scan_count", "icpb_align_host_accept",
-           "icpb_compose_chain_device", "icpb_compose_chain_gpu", "icpb_run_multistart_host"]
+           "icpb_compose_chain_device", "icpb_compose_chain_gpu", "icpb_run_multistart_host",
+           "icpb_set_submaps"]
 
 
 class IcpbParams(ctypes.Structure):
@@ -64,6 +65,7 @@ def sources():
                                               os.path.join(c, "icpb_grid.cuh"),
                                               os.path.join(c, "icpb_compose.cuh"),
                                               os.path.join(c, "icpb_multistart.cuh"),
+                                              os.path.join(c, "icpb_submaps.cuh"),
                                               os.path.join(_ROOT, "include", "icpb.h")]
 
 
@@ -161,6 +163,7 @@ def lib() -> ctypes.CDLL:
     L.icpb_destroy.argtypes = [vp]
     L.icpb_upload_scans.argtypes = [vp, dp, vp, i64]
     L.icpb_set_scans_device.argtypes = [vp, dp, vp, i64, i64]
+    L.icpb_set_submaps.argtypes = [vp, i32p, vp, dp, i64]
     L.icpb_run_device.argtypes = [vp, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p, dp, i32p, vp]
     L.icpb_run_device_gather.argtypes = [vp, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p, vp,
                                          ctypes.c_int32, i64, vp]

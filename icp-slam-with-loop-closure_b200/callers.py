@@ -157,8 +157,51 @@ def _multistart_accept(lidar_points, pairs, starts, thresh, epsilon, max_iters, 
     return rows, _icp.MultiStartResult(res.T[rows], res.error[rows], res.iters[rows], start=res.start[rows])
 
 
+def submap_window_members(n_scans: int, targets, window: int) -> list:
+    """The members of the submap around each target scan i: scans max(0, i - window) .. min(n - 1, i + window)."""
+    return [np.arange(max(0, i - window), min(n_scans - 1, i + window) + 1) for i in targets]
+
+
+def submap_window_transforms(poses, targets, members) -> list:
+    """Member s of the submap around target i is placed in scan i's frame by inv(pose_to_mat(P_i)) @
+    pose_to_mat(P_s); scan i itself by the exact identity, so a one-member submap reproduces scan i bit for bit."""
+    mats = poses_to_mats(poses)
+    out = []
+    for i, mem in zip(targets, members):
+        T = np.linalg.inv(mats[i]) @ mats[mem]
+        T[mem == i] = np.eye(3)
+        T[:, 2] = (0.0, 0.0, 1.0)
+        out.append(T)
+    return out
+
+
+def _submap_accept(poses, lidar_points, cand, starts, thresh, window, epsilon, max_iters, device):
+    """Every candidate's source scan j aligned onto the submap around its target i (``submap_window_*``),
+    built on the device from the resident table; the pairs whose (best) error is below ``thresh``: (rows,
+    result of those rows).  The submaps are dropped again afterwards, leaving the scan table resident."""
+    e = _icp.engine(device)
+    if not (isinstance(lidar_points, _icp.ScanTable) and e.table is lidar_points):
+        e.set_scans(lidar_points)
+    n = e.table.n_scans
+    targets, sub = np.unique(cand[:, 0], return_inverse=True)
+    members = submap_window_members(n, targets, window)
+    ids = e.set_submaps(members, submap_window_transforms(poses, targets, members))
+    try:
+        pairs = np.stack((cand[:, 1], ids[sub]), axis=1).astype(np.int32)
+        if starts is not None:
+            res = e.run_multistart(pairs, starts, None, epsilon=epsilon, max_iters=max_iters)
+        else:
+            res = e.run(pairs, None, epsilon=epsilon, max_iters=max_iters)
+    finally:
+        e.set_submaps([], [])
+    rows = np.nonzero(res.error < thresh)[0]
+    if starts is not None:
+        return rows, _icp.MultiStartResult(res.T[rows], res.error[rows], res.iters[rows], start=res.start[rows])
+    return rows, _icp.BatchResult(res.T[rows], res.error[rows], res.iters[rows])
+
+
 def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist=1, err_thresh=110,
-                            max_iters=100, epsilon=0.05, device=None, starts=None):
+                            max_iters=100, epsilon=0.05, device=None, starts=None, submap_window=None):
     """Loop-closure constraints the reference's ``detect_proximity`` would add, in its order.
 
     ICP is a pure function of its inputs, so every candidate is aligned in one batch
@@ -171,12 +214,24 @@ def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist
     ``starts`` ((K, 3, 3), e.g. ``icp.heading_starts(8)``): for revisits whose relative heading is
     unknown, every candidate is aligned from each start with ``icp_multistart`` and its best start is
     the one tested against the threshold; the BatchResult is then a MultiStartResult (``start`` says
-    which start won)."""
+    which start won).
+
+    ``submap_window`` (an integer w >= 0): scan-to-submap matching.  The target of candidate (i, j) is scan i
+    merged with its neighbours i - w .. i + w (clipped to the trajectory), each placed in scan i's frame by
+    ``poses`` (``IcpEngine.set_submaps``), so a source that overlaps scan i only partly still finds its
+    structure.  The submap sits in scan i's frame, so the constraint (i, j, T) keeps its meaning, and the
+    error is still an SSE over scan j's points, so ``err_thresh`` keeps its scale.  w = 0 gives exactly the
+    constraints of ``submap_window=None``."""
+    if submap_window is not None and (int(submap_window) != submap_window or submap_window < 0):
+        raise ValueError("submap_window must be an integer >= 0")
     cand = proximity_candidates(poses, min_dist_along_path, max_dist, device)
     if len(cand) == 0:
         return [], None
     pairs = np.stack((cand[:, 1], cand[:, 0]), axis=1).astype(np.int32)
-    if starts is not None:
+    if submap_window is not None:
+        rows, res = _submap_accept(poses, lidar_points, cand, starts, err_thresh, int(submap_window), epsilon,
+                                   max_iters, device)
+    elif starts is not None:
         rows, res = _multistart_accept(lidar_points, pairs, starts, err_thresh, epsilon, max_iters, device)
     else:
         # the `error < err_thresh` test runs in the kernel epilogue: only the candidates that pass it come

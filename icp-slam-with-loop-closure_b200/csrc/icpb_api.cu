@@ -25,6 +25,7 @@
 #include "icpb_grid.cuh"
 #include "icpb_compose.cuh"
 #include "icpb_multistart.cuh"
+#include "icpb_submaps.cuh"
 
 namespace {
 
@@ -294,6 +295,9 @@ struct icpb_ctx {
     const double *xy = nullptr;
     const int64_t *offsets = nullptr;
     int64_t n_scans = 0, longest = 0;
+    // the base table: scans [0, n_base) of the table, the ones set by the caller; icpb_set_submaps appends
+    // the submaps after them (n_base = n_scans without submaps)
+    int64_t n_base = 0, base_longest = 0;
     std::vector<int64_t> host_off;                  // the table's offsets on the host (table_host_offsets)
     // queue counters
     unsigned long long *queue = nullptr;      // kQueueWords: kQueueRing counters, the work counter, then the
@@ -343,12 +347,14 @@ bool fits_smem(const icpb_ctx *h, int64_t n)
     return L.bytes != 0x7fffffff && L.bytes <= h->smem_limit;
 }
 
-// The handle's scan table; a new table has no staging images yet (ensure_prep).  off_host: the offsets
-// on the host, kept when a batch on the table may be split by scan length (null for a borrowed table).
+// The handle's scan table; a new table has no staging images yet (ensure_prep) and no submaps (it is all
+// base; icpb_set_submaps restores its own base afterwards).  off_host: the offsets on the host, kept when a
+// batch on the table may be split by scan length (null for a borrowed table).
 void set_table(icpb_ctx *h, const double *xy, const int64_t *off, int64_t n_scans, int64_t longest,
                const int64_t *off_host)
 {
     h->prep_for = nullptr; h->xy = xy; h->offsets = off; h->n_scans = n_scans; h->longest = longest;
+    h->n_base = n_scans; h->base_longest = longest;
     h->host_off.clear();
     if (off_host && !fits_smem(h, longest)) h->host_off.assign(off_host, off_host + n_scans + 1);
 }
@@ -966,6 +972,138 @@ int icpb_run_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, i
     ON_DEVICE(h);
     return run_host_common(h, nullptr, nullptr, h->n_scans, h->longest, h_pairs, h_init, B, p,
                            h_T, h_err, h_passes, h_hist, h_corr);
+}
+
+}  // extern "C"
+
+namespace {
+
+// One pass of the merge kernel over the submaps' n_pts points: check mode (out == nullptr) or write mode.
+cudaError_t merge_submaps(icpb_ctx *h, const int64_t *src, const int64_t *mout, const double *T, int64_t n_members,
+                          int64_t n_pts, double *out, int32_t *bad)
+{
+    int64_t blocks = (n_pts + icpb::kSubmapThreads - 1) / icpb::kSubmapThreads;
+    if (blocks > 16 * (int64_t)h->sm_count) blocks = 16 * (int64_t)h->sm_count;
+    icpb::submap_merge_kernel<<<(unsigned)blocks, icpb::kSubmapThreads, 0, h->stream>>>(
+        (const double2 *)h->xy, src, mout, T, n_members, (double2 *)out, bad);
+    return cudaGetLastError();
+}
+
+// Write mode of icpb_set_submaps, after the check: the base into xy / off unless it is already there, the
+// submaps' offsets and points after it.
+cudaError_t write_submaps(icpb_ctx *h, double *xy, int64_t *off, const int64_t *comb, int64_t n_submaps,
+                          const int64_t *src, const int64_t *mout, const double *T, int64_t n_members)
+{
+    const int64_t nb = h->n_base, base_pts = comb[nb];
+    cudaStream_t st = h->stream;
+    cudaError_t e = cudaSuccess;
+    if (xy != h->xy)
+        e = cudaMemcpyAsync(xy, h->xy, sizeof(double) * 2 * (size_t)base_pts, cudaMemcpyDeviceToDevice, st);
+    if (e == cudaSuccess && off != h->offsets)
+        e = cudaMemcpyAsync(off, h->offsets, sizeof(int64_t) * (size_t)(nb + 1), cudaMemcpyDeviceToDevice, st);
+    if (e == cudaSuccess)
+        e = cudaMemcpyAsync(off + nb + 1, comb + nb + 1, sizeof(int64_t) * (size_t)n_submaps, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess)
+        e = merge_submaps(h, src, mout, T, n_members, comb[nb + n_submaps] - base_pts, xy + 2 * base_pts, nullptr);
+    const cudaError_t s = cudaStreamSynchronize(st);
+    return e != cudaSuccess ? e : s;
+}
+
+}  // namespace
+
+extern "C" {
+
+int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_submap_off,
+                     const double *h_member_T, int64_t n_submaps)
+{
+    if (!h) return fail(ICPB_EINVAL, "handle is null%s");
+    if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
+    if (n_submaps < 0 || !h_submap_off) return fail(ICPB_EINVAL, "icpb_set_submaps: negative count or null offsets%s");
+    if (h_submap_off[0] != 0) return fail(ICPB_EINVAL, "icpb_set_submaps: submap offsets must start at 0%s");
+    for (int64_t m = 0; m < n_submaps; ++m)
+        if (h_submap_off[m + 1] <= h_submap_off[m])
+            return fail(ICPB_EINVAL, "icpb_set_submaps: submap offsets must increase strictly (a submap needs a member)%s");
+    const int64_t n_mem = h_submap_off[n_submaps], nb = h->n_base;
+    if (n_mem > 0 && (!h_members || !h_member_T)) return fail(ICPB_EINVAL, "icpb_set_submaps: null members or transforms%s");
+    for (int64_t k = 0; k < n_mem; ++k)
+        if (h_members[k] < 0 || h_members[k] >= nb)
+            return fail(ICPB_EINVAL, "icpb_set_submaps: a member is not a scan of the base table%s");
+    for (int64_t k = 0; k < 2 * n_mem; ++k) {
+        const double *r = h_member_T + 3 * k;
+        if (!(fabs(r[0]) <= ICPB_MAX_GUESS_LINEAR) || !(fabs(r[1]) <= ICPB_MAX_GUESS_LINEAR) ||
+            !(fabs(r[2]) <= ICPB_MAX_GUESS_SHIFT))
+            return fail(ICPB_EINVAL, "icpb_set_submaps: a member transform holds non-finite values or values beyond "
+                                     "the bounds of icpb.h%s");
+    }
+    ON_DEVICE(h);
+    int rc;
+    const int64_t *off;                                       // the base's offsets are the first nb + 1
+    if ((rc = table_host_offsets(h, &off))) return rc;
+    // the combined table's offsets, every member's first base point and its first point in the submaps
+    std::vector<int64_t> comb(off, off + nb + 1), src((size_t)n_mem), mout((size_t)n_mem + 1);
+    comb.resize((size_t)(nb + n_submaps + 1));
+    const int64_t base_longest = h->base_longest;
+    int64_t longest = base_longest;
+    mout[0] = 0;
+    for (int64_t m = 0; m < n_submaps; ++m) {
+        for (int64_t k = h_submap_off[m]; k < h_submap_off[m + 1]; ++k) {
+            const int32_t s = h_members[k];
+            src[(size_t)k] = off[s];
+            mout[(size_t)k + 1] = mout[(size_t)k] + (off[s + 1] - off[s]);
+        }
+        const int64_t len = mout[(size_t)h_submap_off[m + 1]] - mout[(size_t)h_submap_off[m]];
+        if (icpb::smem_layout(len, 8).bytes == 0x7fffffff) {
+            snprintf(g_err, sizeof g_err, "icpb_set_submaps: a submap of %lld points is beyond the kernel's 32-bit "
+                     "layout offsets", (long long)len);
+            return ICPB_ETOOLONG;
+        }
+        comb[(size_t)(nb + m + 1)] = comb[(size_t)(nb + m)] + len;
+        if (len > longest) longest = len;
+    }
+    if (n_submaps == 0) {                                     // the base table alone, where it is
+        if (h->n_scans != nb) set_table(h, h->xy, h->offsets, nb, base_longest, comb.data());
+        return 0;
+    }
+    // check mode: nothing is written until every merged coordinate is known to be within ICPB_MAX_COORD
+    cudaStream_t st = h->stream;
+    Carve c;
+    const size_t o_src = c(8 * (size_t)n_mem), o_mout = c(8 * (size_t)(n_mem + 1));
+    const size_t o_T = c(48 * (size_t)n_mem), o_bad = c(sizeof(int32_t));
+    if ((rc = h->arena.reserve(c.used))) return rc;
+    const int64_t *d_src = at<int64_t>(h->arena, o_src), *d_mout = at<int64_t>(h->arena, o_mout);
+    const double *d_T = at<double>(h->arena, o_T);
+    int32_t *d_bad = at<int32_t>(h->arena, o_bad), bad = 0;
+    CU(cudaMemcpyAsync((void *)d_src, src.data(), 8 * (size_t)n_mem, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync((void *)d_mout, mout.data(), 8 * (size_t)(n_mem + 1), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync((void *)d_T, h_member_T, 48 * (size_t)n_mem, cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(d_bad, 0, sizeof(int32_t), st));
+    const int64_t n_pts = mout[(size_t)n_mem];
+    CU(merge_submaps(h, d_src, d_mout, d_T, n_mem, n_pts, nullptr, d_bad));
+    CU(cudaMemcpyAsync(&bad, d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (bad) return fail(ICPB_EINVAL, "icpb_set_submaps: a merged coordinate is non-finite or beyond ICPB_MAX_COORD%s");
+    // write mode, into the handle's own table buffers.  One that is too small is replaced by a new block, which
+    // is filled before the old one is freed: the resident table stays whole until the new one is (DevBuf::reserve
+    // would free first).
+    const size_t nb_xy = sizeof(double) * 2 * (size_t)comb.back(), nb_off = sizeof(int64_t) * comb.size();
+    DevBuf nxy, noff;
+    if (nb_xy > h->own_xy.cap && (rc = nxy.reserve(nb_xy))) return rc;
+    if (nb_off > h->own_off.cap && (rc = noff.reserve(nb_off))) { nxy.release(); return rc; }
+    double *xy = (double *)(nxy.p ? nxy.p : h->own_xy.p);
+    int64_t *doff = (int64_t *)(noff.p ? noff.p : h->own_off.p);
+    const cudaError_t e = write_submaps(h, xy, doff, comb.data(), n_submaps, d_src, d_mout, d_T, n_mem);
+    if (e != cudaSuccess) {
+        nxy.release(); noff.release();
+        // a failure part-way through writes into the resident table's own buffers leaves it half written
+        if (xy == h->xy || doff == h->offsets) drop_table(h);
+        snprintf(g_err, sizeof g_err, "icpb_set_submaps: %s", cudaGetErrorString(e));
+        return (int)e;
+    }
+    if (nxy.p) { h->own_xy.release(); h->own_xy = nxy; }
+    if (noff.p) { h->own_off.release(); h->own_off = noff; }
+    set_table(h, xy, doff, nb + n_submaps, longest, comb.data());
+    h->n_base = nb; h->base_longest = base_longest;
+    return 0;
 }
 
 }  // extern "C"

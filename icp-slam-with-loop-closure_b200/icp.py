@@ -13,6 +13,8 @@ plus the batched entry point ``icp_batch`` that replaces the reference's joblib 
 (scripts/main.py:240-247, src/loop_closure_detection.py:134-142,
 src/pose_graph_optimization.py:60-68) with one kernel launch, and ``icp_multistart``, which aligns
 every pair from K start transforms and keeps the best one (``heading_starts``, ``compose_starts``).
+``IcpEngine.set_submaps`` merges resident scans into submaps on the device, for scan-to-submap matching;
+``merge_scans`` builds the same submaps on the host, bit for bit.
 
 There is no CPU fallback: without libicpb.so and a B200 every call raises.
 """
@@ -28,7 +30,7 @@ from . import _lib
 from ._lib import IcpbError  # noqa: F401  (re-exported)
 from .synth import pose_to_mat
 
-__all__ = ["icp", "icp_iteration", "icp_batch", "icp_multistart", "heading_starts", "compose_starts",
+__all__ = ["icp", "icp_iteration", "icp_batch", "icp_multistart", "heading_starts", "compose_starts", "merge_scans",
            "get_correspondences", "get_closest_point", "get_transform", "get_error",
            "ScanTable", "ScanList", "IcpEngine", "BatchResult", "MultiStartResult", "engine", "make_epilogue"]
 
@@ -194,6 +196,49 @@ def compose_starts(init, starts) -> np.ndarray:
     return G
 
 
+def _submap_args(members, transforms, n_base: int):
+    """The arguments of ``merge_scans`` / ``IcpEngine.set_submaps`` checked: one 1-D array of base scan ids
+    in [0, n_base) per submap, at least one each, and one (k_m, 3, 3) SE(2)-shaped transform per member within
+    the guess bounds.  Returns (list of int32 id arrays, list of (k_m, 6) top rows)."""
+    if len(members) != len(transforms):
+        raise ValueError(f"{len(members)} member lists but {len(transforms)} transform lists")
+    ids, rows = [], []
+    for m, (mem, T) in enumerate(zip(members, transforms)):
+        a = np.asarray(mem)
+        if a.ndim != 1 or len(a) == 0 or (a.dtype.kind not in "iu"):
+            raise ValueError(f"submap {m}: members must be a non-empty 1-D array of scan ids")
+        if a.min() < 0 or a.max() >= n_base:
+            raise ValueError(f"submap {m}: a member is not a scan of the base table (0 .. {n_base - 1})")
+        T = np.asarray(T, dtype=np.float64)
+        if T.shape != (len(a), 3, 3):
+            raise ValueError(f"submap {m}: transforms have shape {T.shape}; expected ({len(a)}, 3, 3)")
+        ids.append(a.astype(np.int32))
+        rows.append(_to6(T))
+    return ids, rows
+
+
+def merge_scans(scans, members, transforms) -> list:
+    """Submaps built on the host with the library's bits: submap m is the scans ``members[m]`` (base scan ids)
+    in order, member k's points mapped by ``transforms[m][k]`` ((k_m, 3, 3) SE(2)-shaped, into the submap's
+    frame) as ``x' = (T00*x + T01*y) + T02``, ``y' = (T10*x + T11*y) + T12`` -- element-wise, every product
+    and sum rounded on its own, which is what ``IcpEngine.set_submaps`` computes on the device (a matrix
+    product ``@`` may fuse or reorder them, and then the bits depend on the BLAS build).  Returns one
+    (n_m, 2) float64 array per submap."""
+    if isinstance(scans, ScanTable):
+        o = scans.offsets
+        scans = [scans.xy[o[s]:o[s + 1]] for s in range(scans.n_scans)]
+    ids, rows = _submap_args(members, transforms, len(scans))
+    out = []
+    for mem, T6 in zip(ids, rows):
+        parts = []
+        for s, t in zip(mem, T6):
+            p = np.asarray(scans[s], dtype=np.float64)
+            x, y = p[:, 0], p[:, 1]
+            parts.append(np.stack(((t[0] * x + t[1] * y) + t[2], (t[3] * x + t[4] * y) + t[5]), axis=1))
+        out.append(np.concatenate(parts))
+    return out
+
+
 class ScanList:
     """The reference's ``lidar_points`` as it is -- a sequence of separate (m_i, 2) float64 arrays in
     pageable memory (src/dataloader.py:110-112) -- described by a pointer and a length per scan for
@@ -284,6 +329,7 @@ class IcpEngine:
         _lib.check(self._L.icpb_create(self.device, ctypes.byref(self._h)), "icpb_create")
         self.table: ScanTable | None = None
         self._keep = None
+        self._base = None              # (base table, table with submaps) while set_submaps' table is resident
 
     def close(self):
         if self._h:
@@ -317,6 +363,37 @@ class IcpEngine:
                                                  table.longest), "icpb_set_scans_device")
         self.table = table
         self._keep = (xy_t, offsets_t)
+
+    # -- submaps ------------------------------------------------------------------------------
+    def set_submaps(self, members, transforms) -> np.ndarray:
+        """Scans of the resident (base) table merged on the device into submaps appended to it
+        (icpb_set_submaps): submap m is the base scans ``members[m]`` in order, member k mapped into the
+        submap's frame by ``transforms[m][k]`` ((k_m, 3, 3)), with the bits of ``merge_scans``.  Returns the
+        submaps' scan ids, n_base .. n_base + M - 1, for ``run``, ``run_multistart`` and ``run_device``.  A
+        call replaces the previous submaps; ``set_submaps([], [])`` leaves the base table alone.  ValueError
+        for bad arguments and for merged coordinates beyond the library's bound, with the table unchanged."""
+        if self.table is None:
+            raise ValueError("no scan table set")
+        # the base: the table as the caller set it, unless this engine's own submaps are resident
+        base = self._base[0] if self._base is not None and self._base[1] is self.table else self.table
+        ids, rows = _submap_args(members, transforms, base.n_scans)
+        sub_off = np.concatenate(([0], np.cumsum([len(a) for a in ids]))).astype(np.int64)
+        mem = np.ascontiguousarray(np.concatenate(ids) if ids else np.zeros(0, np.int32))
+        T6 = np.ascontiguousarray(np.concatenate(rows) if rows else np.zeros((0, 6)))
+        try:
+            _lib.check(self._L.icpb_set_submaps(self._h, _ptr(mem), _ptr(sub_off), _ptr(T6), len(ids)),
+                       "icpb_set_submaps")
+        except Exception:
+            if self._L.icpb_scan_count(self._h) == 0:           # failed part-way: the library dropped the table
+                self.table, self._base = None, None
+            raise
+        if ids:
+            lengths = np.concatenate((base.lengths, [int(base.lengths[a].sum()) for a in ids]))
+            self.table = ScanTable.from_lengths(lengths)
+            self._base = (base, self.table)
+        else:
+            self.table, self._base = base, None
+        return np.arange(base.n_scans, base.n_scans + len(ids))
 
     # -- host-buffer run (the reference-facing call) -----------------------------------------
     def run(self, pairs, init_transforms=None, epsilon=0.01, max_iters=100, stopping_thresh=0.0001,

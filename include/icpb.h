@@ -123,6 +123,41 @@ int icpb_set_scans_device(icpb_handle h, const double *d_xy, const int64_t *d_of
                           int64_t n_scans, int64_t longest_scan);
 
 /*
+ * Submaps: scans of the resident table merged on the device into new scans appended to it -- the target of
+ * scan-to-submap matching (a revisiting scan aligned onto scan i together with its neighbours, placed by the
+ * current poses, instead of onto scan i alone).  The base table is the one last set by icpb_upload_scans,
+ * icpb_set_scans_device or an icpb_align_host* call, with n_base scans.
+ *   h_submap_off  n_submaps + 1 offsets into h_members: [0] = 0, strictly increasing (every submap has a member)
+ *   h_members     base scan ids in [0, n_base); a scan may be a member of several submaps, and more than once of one
+ *   h_member_T    one 2x3 transform per member (6 doubles, the usual row layout): it maps the member's points into
+ *                 the submap's frame
+ * Submap m becomes scan n_base + m of the resident table: its members' points in member order, each mapped as
+ *     x' = (T00*x + T01*y) + T02        y' = (T10*x + T11*y) + T12
+ * with every product and sum rounded to nearest on its own (no FMA contraction; numpy's element-wise * and +
+ * give the same bits), so a submap can be restated on the host and every alignment against it checked bit for
+ * bit.  Every entry point that reads the resident table sees the submaps (icpb_run_host, icpb_run_device*,
+ * icpb_run_multistart_host, pair_mode 1 over the whole table), and icpb_scan_count reports n_base + n_submaps.
+ * A call replaces the submaps of the previous call; n_submaps = 0 goes back to the base table alone.  A call
+ * that sets a new table drops the submaps.
+ * Memory: the table with its submaps is one table in memory the handle owns.  A borrowed base
+ * (icpb_set_scans_device) is copied there, and from then on the handle no longer reads the caller's buffers
+ * (they are never written); call icpb_set_scans_device again after changing them.  A table whose longest
+ * submap does not fit shared memory gets no staging images: its short pairs stage per pair, like those of
+ * any table holding scans beyond shared memory.
+ * Rejected before anything is written, leaving the resident table (submaps included) as it was:
+ *   ICPB_ENOSCANS  no table is set;
+ *   ICPB_EINVAL    null pointers, a negative count, bad offsets, a member id outside the base table (a submap
+ *                  id included), a transform outside the guess bounds (ICPB_MAX_GUESS_LINEAR / _SHIFT, NaN
+ *                  included), and any merged coordinate beyond ICPB_MAX_COORD -- scans and transforms within
+ *                  their bounds can still merge to coordinates of ~2e13; the device tests every merged point in
+ *                  a pass of its own before the table is written;
+ *   ICPB_ETOOLONG  a submap beyond the alignment kernel's 32-bit layout offsets (~100 M points).
+ * Synchronous.  Like icpb_upload_scans, it must not overlap an asynchronous icpb_run_device* on the same handle.
+ */
+int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_submap_off,
+                     const double *h_member_T, int64_t n_submaps);
+
+/*
  * B independent icp() calls (src/icp.py:72-97) in one launch -- replaces the joblib fan-out
  * `Parallel(...)(delayed(icp.icp)(...) for ...)` of scripts/main.py:240-247,
  * src/loop_closure_detection.py:134-142 and src/pose_graph_optimization.py:60-68.
@@ -412,8 +447,8 @@ int icpb_set_tuning(icpb_handle h, const char *key, int64_t value);
 /* Number of alignment-kernel launches made through this handle (bench.py's gpu_launches). */
 int64_t icpb_launch_count(icpb_handle h);
 
-/* Scans of the table resident on the handle's device, 0 when there is none (never set, or an
- * icpb_align_host* call failed part-way and left the buffer half written). */
+/* Scans of the table resident on the handle's device (submaps included), 0 when there is none (never set,
+ * or an icpb_align_host* or icpb_set_submaps call failed part-way and left the buffer half written). */
 int64_t icpb_scan_count(icpb_handle h);
 
 /* Optional instrumentation: while enabled, launches add the point-pair distance evaluations
