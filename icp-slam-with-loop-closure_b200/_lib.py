@@ -15,17 +15,6 @@ FLAG_EXHAUSTIVE = 1
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo",
               "-Xcompiler", "-fPIC", "-shared"]
 
-EXPORTS = ["icpb_default_params", "icpb_abi_version", "icpb_create", "icpb_destroy",
-           "icpb_upload_scans", "icpb_set_scans_device", "icpb_run_device", "icpb_run_host",
-           "icpb_icp_pair_host", "icpb_get_kernel_info", "icpb_launch_count", "icpb_last_error",
-           "icpb_count_work", "icpb_read_work", "icpb_align_host", "icpb_align_host_ld", "icpb_plan_upload", "icpb_fit_pairs_host",
-           "icpb_proximity_closest", "icpb_proximity_pairs", "icpb_compose_chain",
-           "icpb_run_device_gather", "icpb_pose_graph_sgd", "icpb_occupancy_grid_bounds",
-           "icpb_occupancy_grid_update", "icpb_run_device_ex", "icpb_align_host_ex", "icpb_align_host_scans",
-           "icpb_set_tuning", "icpb_scan_count", "icpb_align_host_accept",
-           "icpb_compose_chain_device", "icpb_compose_chain_gpu", "icpb_run_multistart_host",
-           "icpb_set_submaps"]
-
 
 class IcpbParams(ctypes.Structure):
     _fields_ = [("epsilon", ctypes.c_double), ("stopping_thresh", ctypes.c_double),
@@ -55,6 +44,57 @@ class IcpbKernelInfo(ctypes.Structure):
 
 class IcpbError(RuntimeError):
     pass
+
+
+# Every export of include/icpb.h, declared once: name -> (restype, argtypes).  Pointers are void *: numpy
+# arrays go in through `ptr`, torch tensors as c_void_p(t.data_ptr()), out-scalars through ctypes.byref.
+_v, _i, _i32, _i64, _f64 = ctypes.c_void_p, ctypes.c_int, ctypes.c_int32, ctypes.c_int64, ctypes.c_double
+_P, _E = ctypes.POINTER(IcpbParams), ctypes.POINTER(IcpbEpilogue)
+_f64p, _i64p = ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_int64)
+SIGNATURES = {
+    "icpb_default_params": (None, [_P]),
+    "icpb_abi_version": (_i, []),
+    "icpb_create": (_i, [_i, ctypes.POINTER(_v)]),
+    "icpb_destroy": (_i, [_v]),
+    "icpb_upload_scans": (_i, [_v, _v, _v, _i64]),
+    "icpb_set_scans_device": (_i, [_v, _v, _v, _i64, _i64]),
+    "icpb_set_submaps": (_i, [_v, _v, _v, _v, _i64]),
+    "icpb_run_device": (_i, [_v, _v, _v, _i64, _P, _v, _v, _v, _v, _v, _v]),
+    "icpb_run_device_gather": (_i, [_v, _v, _v, _i64, _P, _v, _v, _v, _v, _i32, _i64, _v]),
+    "icpb_run_device_ex": (_i, [_v, _v, _v, _i64, _P, _v, _v, _v, _E, _v]),
+    "icpb_run_host": (_i, [_v, _v, _v, _i64, _P, _v, _v, _v, _v, _v]),
+    "icpb_run_multistart_host": (_i, [_v, _v, _v, _i64, _v, _i32, _P, _v, _v, _v, _v, _v, _v]),
+    "icpb_align_host": (_i, [_v, _v, _v, _i64, _v, _v, _i64, _P, _v, _v, _v]),
+    "icpb_plan_upload": (_i, [_v, _i64, _i32, _v, _v]),
+    "icpb_align_host_ld": (_i, [_v, _v, _v, _i64, _v, _v, _i32, _i64, _P, _v, _i32, _v, _v]),
+    "icpb_align_host_ex": (_i, [_v, _v, _v, _i64, _v, _v, _i32, _i64, _P, _v, _i32, _v, _v, _E]),
+    "icpb_align_host_scans": (_i, [_v, _v, _v, _i64, _v, _v, _i32, _i64, _P, _v, _i32, _v, _v, _E]),
+    "icpb_align_host_accept": (_i, [_v, _v, _v, _v, _v, _i64, _v, _v, _i32, _i64, _P, _f64, _i64, _i64p,
+                                    _v, _v, _i32, _v, _v]),
+    "icpb_icp_pair_host": (_i, [_v, _v, _i64, _v, _i64, _v, _P, _v, _v, _v, _v, _v]),
+    "icpb_fit_pairs_host": (_i, [_v, _v, _v, _i64, _v, _v]),
+    "icpb_proximity_closest": (_i, [_v, _v, _v, _i64, _f64, _f64, _v, _v]),
+    "icpb_proximity_pairs": (_i, [_v, _v, _v, _i64, _f64, _f64, _i64, _v, _i64p]),
+    "icpb_compose_chain": (_i, [_v, _v, _i64, _v]),
+    "icpb_compose_chain_device": (_i, [_v, _v, _v, _i64, _v, _v]),
+    "icpb_compose_chain_gpu": (_i, [_v, _v, _v, _i64, _v]),
+    "icpb_pose_graph_sgd": (_i, [_v, _v, _i64, _v, _v, _i64, _v, _i32, _f64]),
+    "icpb_occupancy_grid_bounds": (_i, [_v, _v, _i64, _f64, _f64, _f64, _f64p, _f64p, _i64p, _i64p]),
+    "icpb_occupancy_grid_update": (_i, [_v, _v, _i64, _v, _i64, _i64, _f64, _f64, _f64, _i32, _i32]),
+    "icpb_get_kernel_info": (_i, [_v, _i64, ctypes.POINTER(IcpbKernelInfo)]),
+    "icpb_set_tuning": (_i, [_v, ctypes.c_char_p, _i64]),
+    "icpb_launch_count": (_i64, [_v]),
+    "icpb_scan_count": (_i64, [_v]),
+    "icpb_count_work": (_i, [_v, _i]),
+    "icpb_read_work": (_i, [_v, ctypes.POINTER(ctypes.c_uint64)]),
+    "icpb_last_error": (ctypes.c_char_p, []),
+}
+EXPORTS = list(SIGNATURES)
+
+
+def ptr(a):
+    """A numpy array's data as a void * argument (None stays a null pointer)."""
+    return None if a is None else ctypes.c_void_p(a.ctypes.data)
 
 
 def sources():
@@ -155,58 +195,9 @@ def lib() -> ctypes.CDLL:
         except (subprocess.CalledProcessError, OSError) as exc:
             raise IcpbError(f"{SO_PATH} is missing and could not be built ({exc}); there is no CPU fallback") from exc
     L = ctypes.CDLL(SO_PATH)
-    vp, i64, i32p, dp = ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p
-    L.icpb_default_params.argtypes = [ctypes.POINTER(IcpbParams)]
-    L.icpb_default_params.restype = None
-    L.icpb_abi_version.restype = ctypes.c_int
-    L.icpb_create.argtypes = [ctypes.c_int, ctypes.POINTER(vp)]
-    L.icpb_destroy.argtypes = [vp]
-    L.icpb_upload_scans.argtypes = [vp, dp, vp, i64]
-    L.icpb_set_scans_device.argtypes = [vp, dp, vp, i64, i64]
-    L.icpb_set_submaps.argtypes = [vp, i32p, vp, dp, i64]
-    L.icpb_run_device.argtypes = [vp, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p, dp, i32p, vp]
-    L.icpb_run_device_gather.argtypes = [vp, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p, vp,
-                                         ctypes.c_int32, i64, vp]
-    L.icpb_run_device_ex.argtypes = [vp, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p,
-                                     ctypes.POINTER(IcpbEpilogue), vp]
-    L.icpb_align_host_ex.argtypes = [vp, dp, vp, i64, i32p, dp, ctypes.c_int32, i64, ctypes.POINTER(IcpbParams),
-                                     dp, ctypes.c_int32, dp, i32p, ctypes.POINTER(IcpbEpilogue)]
-    L.icpb_align_host_scans.argtypes = [vp, vp, vp, i64, i32p, dp, ctypes.c_int32, i64, ctypes.POINTER(IcpbParams),
-                                        dp, ctypes.c_int32, dp, i32p, ctypes.POINTER(IcpbEpilogue)]
-    L.icpb_set_tuning.argtypes = [vp, ctypes.c_char_p, i64]
-    L.icpb_align_host_accept.argtypes = [vp, dp, vp, vp, vp, i64, i32p, dp, ctypes.c_int32, i64,
-                                         ctypes.POINTER(IcpbParams), ctypes.c_double, i64,
-                                         ctypes.POINTER(ctypes.c_int64), vp, dp, ctypes.c_int32, dp, i32p]
-    L.icpb_run_host.argtypes = [vp, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p, dp, i32p]
-    L.icpb_run_multistart_host.argtypes = [vp, i32p, dp, i64, dp, ctypes.c_int32, ctypes.POINTER(IcpbParams),
-                                           dp, dp, i32p, i32p, dp, i32p]
-    L.icpb_align_host.argtypes = [vp, dp, vp, i64, i32p, dp, i64, ctypes.POINTER(IcpbParams), dp, dp, i32p]
-    L.icpb_align_host_ld.argtypes = [vp, dp, vp, i64, i32p, dp, ctypes.c_int32, i64, ctypes.POINTER(IcpbParams),
-                                     dp, ctypes.c_int32, dp, i32p]
-    L.icpb_proximity_closest.argtypes = [vp, dp, dp, i64, ctypes.c_double, ctypes.c_double, i32p, dp]
-    L.icpb_proximity_pairs.argtypes = [vp, dp, dp, i64, ctypes.c_double, ctypes.c_double, i64, i32p,
-                                       ctypes.POINTER(ctypes.c_int64)]
-    L.icpb_compose_chain.argtypes = [dp, dp, i64, dp]
-    L.icpb_compose_chain_device.argtypes = [vp, dp, dp, i64, dp, vp]
-    L.icpb_compose_chain_gpu.argtypes = [vp, dp, dp, i64, dp]
-    L.icpb_pose_graph_sgd.argtypes = [vp, dp, i64, i32p, dp, i64, dp, ctypes.c_int32, ctypes.c_double]
-    L.icpb_occupancy_grid_bounds.argtypes = [vp, dp, i64, ctypes.c_double, ctypes.c_double, ctypes.c_double,
-                                             ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double),
-                                             ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]
-    L.icpb_occupancy_grid_update.argtypes = [vp, dp, i64, vp, i64, i64, ctypes.c_double, ctypes.c_double,
-                                             ctypes.c_double, ctypes.c_int32, ctypes.c_int32]
-    L.icpb_fit_pairs_host.argtypes = [vp, dp, dp, i64, dp, dp]
-    L.icpb_icp_pair_host.argtypes = [vp, dp, i64, dp, i64, dp, ctypes.POINTER(IcpbParams), dp, dp, i32p, dp, i32p]
-    L.icpb_get_kernel_info.argtypes = [vp, i64, ctypes.POINTER(IcpbKernelInfo)]
-    L.icpb_launch_count.argtypes = [vp]
-    L.icpb_launch_count.restype = ctypes.c_int64
-    L.icpb_scan_count.argtypes = [vp]
-    L.icpb_scan_count.restype = ctypes.c_int64
-    L.icpb_last_error.restype = ctypes.c_char_p
-    L.icpb_count_work.argtypes = [vp, ctypes.c_int]
-    L.icpb_read_work.argtypes = [vp, ctypes.POINTER(ctypes.c_uint64)]
-    for name in EXPORTS:
-        getattr(L, name)
+    for name, (restype, argtypes) in SIGNATURES.items():
+        fn = getattr(L, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = L
     return L
 

@@ -16,6 +16,7 @@ from __future__ import annotations
 
 import numpy as np
 
+from . import _lib
 from . import icp as _icp
 from .synth import mat_to_pose, pose_to_mat
 
@@ -80,24 +81,21 @@ def compose_chain(pose0, transforms) -> np.ndarray:
     """Serial SE(2) prefix product of scripts/main.py:249-256:
     ``pose_i = mat_to_pose(pose_to_mat(pose_{i-1}) @ T_{i-1})``; (n + 1, 3) poses from n transforms.
     Runs in the library's C host loop (the reference's Python loop costs ~100 ms at n = 5,000)."""
-    T = np.asarray(transforms, dtype=np.float64)
-    T6 = np.ascontiguousarray(T[:, :2, :].reshape(-1, 6))
+    T6 = _icp._top_rows(transforms).reshape(-1, 6)
     p0 = np.ascontiguousarray(pose0, dtype=np.float64)
     out = np.empty((len(T6) + 1, 3))
-    _icp._lib.check(_icp._lib.lib().icpb_compose_chain(_icp._ptr(p0), _icp._ptr(T6), len(T6), _icp._ptr(out)),
-                    "icpb_compose_chain")
+    _lib.check(_lib.lib().icpb_compose_chain(_lib.ptr(p0), _lib.ptr(T6), len(T6), _lib.ptr(out)), "icpb_compose_chain")
     return out
 
 
 def compose_chain_gpu(pose0, transforms, device=None) -> np.ndarray:
     """`compose_chain` through the device scan (icpb_compose_chain_gpu): same poses to rounding."""
-    T = np.asarray(transforms, dtype=np.float64)
-    T6 = np.ascontiguousarray(T[:, :2, :].reshape(-1, 6))
+    T6 = _icp._top_rows(transforms).reshape(-1, 6)
     p0 = np.ascontiguousarray(pose0, dtype=np.float64)
     out = np.empty((len(T6) + 1, 3))
     e = _icp.engine(device)
-    _icp._lib.check(e._L.icpb_compose_chain_gpu(e._h, _icp._ptr(p0), _icp._ptr(T6), len(T6), _icp._ptr(out)),
-                    "icpb_compose_chain_gpu")
+    _lib.check(_lib.lib().icpb_compose_chain_gpu(e._h, _lib.ptr(p0), _lib.ptr(T6), len(T6), _lib.ptr(out)),
+               "icpb_compose_chain_gpu")
     return out
 
 
@@ -121,9 +119,9 @@ def proximity_candidates(poses, min_dist_along_path=2, max_dist=1, device=None):
     closest = np.empty(n, dtype=np.int32)
     dist = np.empty(n)
     e = _icp.engine(device)
-    _icp._lib.check(e._L.icpb_proximity_closest(e._h, _icp._ptr(xy), _icp._ptr(trav), n,
-                                                ctypes.c_double(min_dist_along_path), ctypes.c_double(max_dist),
-                                                _icp._ptr(closest), _icp._ptr(dist)), "icpb_proximity_closest")
+    _lib.check(_lib.lib().icpb_proximity_closest(e._h, _lib.ptr(xy), _lib.ptr(trav), n,
+                                                 ctypes.c_double(min_dist_along_path), ctypes.c_double(max_dist),
+                                                 _lib.ptr(closest), _lib.ptr(dist)), "icpb_proximity_closest")
     i = np.nonzero(closest >= 0)[0]
     out = np.stack((i, closest[i].astype(np.int64)), axis=1)[::-1]
     return np.ascontiguousarray(out, dtype=np.int64).reshape(-1, 2)
@@ -139,12 +137,12 @@ def proximity_pairs(poses, min_dist_along_path=2, max_dist=1, device=None) -> np
     trav = _travelled(xy)
     e = _icp.engine(device)
     total = ctypes.c_int64()
-    args = (e._h, _icp._ptr(xy), _icp._ptr(trav), n, ctypes.c_double(min_dist_along_path), ctypes.c_double(max_dist))
-    _icp._lib.check(e._L.icpb_proximity_pairs(*args, 0, None, ctypes.byref(total)), "icpb_proximity_pairs")
+    args = (e._h, _lib.ptr(xy), _lib.ptr(trav), n, ctypes.c_double(min_dist_along_path), ctypes.c_double(max_dist))
+    _lib.check(_lib.lib().icpb_proximity_pairs(*args, 0, None, ctypes.byref(total)), "icpb_proximity_pairs")
     pairs = np.empty((total.value, 2), dtype=np.int32)
     if total.value:
-        _icp._lib.check(e._L.icpb_proximity_pairs(*args, total.value, _icp._ptr(pairs), ctypes.byref(total)),
-                        "icpb_proximity_pairs")
+        _lib.check(_lib.lib().icpb_proximity_pairs(*args, total.value, _lib.ptr(pairs), ctypes.byref(total)),
+                   "icpb_proximity_pairs")
     return pairs
 
 
@@ -154,7 +152,7 @@ def _multistart_accept(lidar_points, pairs, starts, thresh, epsilon, max_iters, 
     MultiStartResult of those rows).  The threshold runs on the host over B results, not B * K."""
     res = _icp.icp_multistart(lidar_points, pairs, starts, None, epsilon=epsilon, max_iters=max_iters, device=device)
     rows = np.nonzero(res.error < thresh)[0]
-    return rows, _icp.MultiStartResult(res.T[rows], res.error[rows], res.iters[rows], start=res.start[rows])
+    return rows, res.take(rows)
 
 
 def submap_window_members(n_scans: int, targets, window: int) -> list:
@@ -180,9 +178,7 @@ def _submap_accept(poses, lidar_points, cand, starts, thresh, window, epsilon, m
     built on the device from the resident table; the pairs whose (best) error is below ``thresh``: (rows,
     result of those rows).  The submaps are dropped again afterwards, leaving the scan table resident."""
     e = _icp.engine(device)
-    if not (isinstance(lidar_points, _icp.ScanTable) and e.table is lidar_points):
-        e.set_scans(lidar_points)
-    n = e.table.n_scans
+    n = e.ensure_scans(lidar_points).n_scans
     targets, sub = np.unique(cand[:, 0], return_inverse=True)
     members = submap_window_members(n, targets, window)
     ids = e.set_submaps(members, submap_window_transforms(poses, targets, members))
@@ -195,9 +191,7 @@ def _submap_accept(poses, lidar_points, cand, starts, thresh, window, epsilon, m
     finally:
         e.set_submaps([], [])
     rows = np.nonzero(res.error < thresh)[0]
-    if starts is not None:
-        return rows, _icp.MultiStartResult(res.T[rows], res.error[rows], res.iters[rows], start=res.start[rows])
-    return rows, _icp.BatchResult(res.T[rows], res.error[rows], res.iters[rows])
+    return rows, res.take(rows)
 
 
 def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist=1, err_thresh=110,

@@ -13,6 +13,8 @@ from __future__ import annotations
 
 import numpy as np
 
+from .icp import _to33, _top_rows, make_epilogue
+
 RECORD_WIDTH = 8     # T (6 doubles), error, passes
 
 
@@ -36,17 +38,14 @@ def shard_all_pairs(n_problems: int, rank: int, world: int, block: int = 4096):
 
 def pack_records(T: np.ndarray, error: np.ndarray, passes: np.ndarray) -> np.ndarray:
     rec = np.empty((len(error), RECORD_WIDTH))
-    rec[:, :6] = np.asarray(T)[:, :2, :].reshape(-1, 6)
+    rec[:, :6] = _top_rows(T)
     rec[:, 6] = error
     rec[:, 7] = passes
     return rec
 
 
 def unpack_records(rec: np.ndarray):
-    T = np.zeros((len(rec), 3, 3))
-    T[:, :2, :] = rec[:, :6].reshape(-1, 2, 3)
-    T[:, 2, 2] = 1.0
-    return T, rec[:, 6].copy(), rec[:, 7].astype(np.int32)
+    return _to33(rec[:, :6]), rec[:, 6].copy(), rec[:, 7].astype(np.int32)
 
 
 def all_gather_records(local: np.ndarray, n_problems: int, block: int = 4096, group=None, device=None):
@@ -135,7 +134,6 @@ class FusedGather:
         self._any = self.hdl or self.acc_hdl
 
     def epilogue(self, accept_thresh=None):
-        from .icp import make_epilogue
         row0, rb, rs = global_rows(self.n_problems, self.rank, self.world, self.block)
         kw = {}
         if self.accept_cap > 0 and accept_thresh is not None:
@@ -179,10 +177,7 @@ def unpack_accepted(rec: np.ndarray):
     tag = rec[:, 7].copy().view(np.int64)
     rows, passes = tag >> 16, (tag & 0xffff).astype(np.int32)
     order = np.argsort(rows, kind="stable")
-    T = np.zeros((len(rec), 3, 3))
-    T[:, :2, :] = rec[:, :6].reshape(-1, 2, 3)
-    T[:, 2, 2] = 1.0
-    return rows[order], T[order], rec[order, 6].copy(), passes[order]
+    return rows[order], _to33(rec[:, :6])[order], rec[order, 6].copy(), passes[order]
 
 
 def icp_batch_sharded_fused(eng, scans, pairs, init_transforms, gather: FusedGather, accept_thresh=None,

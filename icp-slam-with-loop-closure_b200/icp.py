@@ -22,7 +22,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from dataclasses import dataclass
+from dataclasses import dataclass, fields
 
 import numpy as np
 
@@ -118,6 +118,11 @@ class BatchResult:
     def __len__(self):
         return len(self.error)
 
+    def take(self, rows) -> "BatchResult":
+        """The results of problems ``rows`` (an index array or a mask), as a result of the same kind."""
+        return type(self)(**{f.name: None if getattr(self, f.name) is None else getattr(self, f.name)[rows]
+                             for f in fields(self)})
+
 
 @dataclass
 class MultiStartResult(BatchResult):
@@ -128,15 +133,12 @@ class MultiStartResult(BatchResult):
     iters_all: np.ndarray | None = None        # (B, K) int32
 
 
-def _to6(T) -> np.ndarray:
+_ptr = _lib.ptr
+
+
+def _top_rows(T) -> np.ndarray:
+    """(..., 3, 3) -> the (..., 6) top two rows, contiguous float64; ``_to33`` is the inverse."""
     T = np.asarray(T, dtype=np.float64)
-    if T.shape[-2:] != (3, 3):
-        raise ValueError(f"transform has shape {T.shape}; expected (..., 3, 3)")
-    if not (np.all(T[..., 2, 0] == 0) and np.all(T[..., 2, 1] == 0) and np.all(T[..., 2, 2] == 1)):
-        raise ValueError("transform bottom row must be [0, 0, 1] (an SE(2) matrix)")
-    if not (np.all(np.abs(T[..., :2, :2]) <= MAX_GUESS_LINEAR) and np.all(np.abs(T[..., :2, 2]) <= MAX_GUESS_SHIFT)):
-        raise ValueError(f"transform holds non-finite values or values beyond the bounds of include/icpb.h "
-                         f"(|linear part| <= {MAX_GUESS_LINEAR:g}, |translation| <= {MAX_GUESS_SHIFT:g})")
     return np.ascontiguousarray(T[..., :2, :].reshape(T.shape[:-2] + (6,)))
 
 
@@ -147,21 +149,53 @@ def _to33(T6: np.ndarray) -> np.ndarray:
     return out
 
 
-def _ptr(a):
-    return None if a is None else ctypes.c_void_p(a.ctypes.data)
-
-
-def _rows6(T, n, name) -> np.ndarray:
-    """(n, 3, 3) SE(2)-shaped matrices (n None: any number) -> (n, 6) top rows, with the shape, the
-    bottom rows and finiteness checked; the bounds are the library's to check (on the composed guesses)."""
+def _to6(T, bounds: bool = True, name: str = "transform") -> np.ndarray:
+    """SE(2)-shaped (..., 3, 3) matrices -> their (..., 6) top rows, with the bottom rows checked and every value
+    within the guess bounds of include/icpb.h; with ``bounds=False`` only finite (multi-start: the library checks
+    the bounds on the guesses it composes)."""
     T = np.asarray(T, dtype=np.float64)
-    if T.ndim != 3 or T.shape[1:] != (3, 3) or (n is not None and len(T) != n):
-        raise ValueError(f"{name} has shape {T.shape}; expected ({'K' if n is None else n}, 3, 3)")
+    if T.shape[-2:] != (3, 3):
+        raise ValueError(f"{name} has shape {T.shape}; expected (..., 3, 3)")
     if not (np.all(T[..., 2, 0] == 0) and np.all(T[..., 2, 1] == 0) and np.all(T[..., 2, 2] == 1)):
         raise ValueError(f"{name}: bottom row must be [0, 0, 1] (an SE(2) matrix)")
-    if not np.isfinite(T).all():
+    if bounds:
+        if not (np.all(np.abs(T[..., :2, :2]) <= MAX_GUESS_LINEAR) and np.all(np.abs(T[..., :2, 2]) <= MAX_GUESS_SHIFT)):
+            raise ValueError(f"{name} holds non-finite values or values beyond the bounds of include/icpb.h "
+                             f"(|linear part| <= {MAX_GUESS_LINEAR:g}, |translation| <= {MAX_GUESS_SHIFT:g})")
+    elif not np.isfinite(T).all():
         raise ValueError(f"{name} holds non-finite values")
-    return np.ascontiguousarray(T[..., :2, :].reshape(T.shape[:-2] + (6,)))
+    return _top_rows(T)
+
+
+def _mats(T, n, name) -> np.ndarray:
+    """``T`` as a contiguous float64 (n, 3, 3) array (n None: any number of matrices), else ValueError."""
+    T = np.ascontiguousarray(T, dtype=np.float64)
+    if T.ndim != 3 or T.shape[1:] != (3, 3) or (n is not None and len(T) != n):
+        raise ValueError(f"{name} has shape {T.shape}; expected ({'K' if n is None else n}, 3, 3)")
+    return T
+
+
+def _pairs(pairs) -> np.ndarray:
+    """(B, 2) (source, target) scan ids as a contiguous int32 array, else ValueError."""
+    a = np.ascontiguousarray(pairs, dtype=np.int32)
+    if a.size == 0:
+        a = a.reshape(0, 2)
+    if a.ndim != 2 or a.shape[1] != 2:
+        raise ValueError(f"pairs has shape {a.shape}; expected (B, 2) of (source, target) scan ids")
+    return a
+
+
+def _check_buffer(t, dtype, numel: int, name: str):
+    """A torch tensor handed to a kernel: ValueError unless it holds ``numel`` elements of ``dtype``,
+    contiguous, on a CUDA device (a kernel would read or write past a wrong one)."""
+    if t.dtype != dtype:
+        raise ValueError(f"{name} is {t.dtype}; expected {dtype}")
+    if t.numel() != numel:
+        raise ValueError(f"{name} holds {t.numel()} elements; expected {numel}")
+    if not t.is_contiguous():
+        raise ValueError(f"{name} is not contiguous")
+    if not t.is_cuda:
+        raise ValueError(f"{name} is not on a CUDA device")
 
 
 def heading_starts(k: int) -> np.ndarray:
@@ -292,7 +326,10 @@ def make_epilogue(peer_ptrs_dev=0, n_peers=0, rank=0, row0=0, row_block=0, row_s
     return ep
 
 
-def _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive=False) -> _lib.IcpbParams:
+def _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive=False, B=1,
+            all_pairs: tuple | None = None) -> _lib.IcpbParams:
+    """icpb_params for a batch of B explicit pairs, or of the all-pairs index space
+    ``all_pairs = (k_first, k_block, k_stride, B)``: linear indices over i<j decoded on the device."""
     p = _lib.default_params()
     p.flags = _lib.FLAG_EXHAUSTIVE if exhaustive else 0
     p.epsilon = float(epsilon)
@@ -302,7 +339,24 @@ def _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive=False
         raise ValueError("max_iters must be an integer")
     p.max_iters = max(min(mi, 2 ** 31 - 8), -2)
     p.rotation_only = 1 if rotation_only else 0
+    if all_pairs is not None:
+        p.pair_mode = 1
+        p.k_first, p.k_block, p.k_stride, _ = (int(v) for v in all_pairs)
+    else:
+        p.k_block = max(int(B), 1)
     return p
+
+
+def _upload_args(scans):
+    """``scans`` for a call that uploads them itself: (the ScanTable resident once the call succeeds, the object
+    that owns the host arrays during the call, the library's (xy, offsets, scan_ptrs, scan_lens) with either
+    the packed pair or the list pair null).  A ScanTable known only by its lengths is rejected here."""
+    if isinstance(scans, ScanTable):
+        if scans.xy is None:
+            raise ValueError("this ScanTable only describes a resident table; pass the scans themselves")
+        return scans, scans, (_ptr(scans.xy), _ptr(scans.offsets), None, None)
+    sl = scans if isinstance(scans, ScanList) else ScanList(scans)
+    return ScanTable.from_lengths(sl.lens), sl, (None, None, _ptr(sl.ptrs), _ptr(sl.lens))
 
 
 def max_passes(max_iters: int) -> int:
@@ -329,7 +383,7 @@ class IcpEngine:
         _lib.check(self._L.icpb_create(self.device, ctypes.byref(self._h)), "icpb_create")
         self.table: ScanTable | None = None
         self._keep = None
-        self._base = None              # (base table, table with submaps) while set_submaps' table is resident
+        self._base = None              # the base table while this engine's submaps are resident
 
     def close(self):
         if self._h:
@@ -347,22 +401,37 @@ class IcpEngine:
         _lib.check(self._L.icpb_set_tuning(self._h, key.encode(), int(value)), "icpb_set_tuning")
 
     # -- scan table -----------------------------------------------------------------------
+    def _replace_table(self, table: ScanTable, fn: str, *args, keep=None, base=None):
+        """Call ``fn``, a library call that replaces the resident table, and mirror what it left: on success
+        ``table`` (``keep``: tensors a borrowed table lives in; ``base``: see set_submaps).  A call that fails
+        either left the previous table in place or dropped it (icpb_scan_count 0)."""
+        try:
+            _lib.check(getattr(self._L, fn)(self._h, *args), fn)
+        except Exception:
+            if self._L.icpb_scan_count(self._h) == 0:
+                self.table = self._keep = self._base = None
+            raise
+        self.table, self._keep, self._base = table, keep, base
+
+    def is_resident(self, scans) -> bool:
+        """True when ``scans`` is the ScanTable resident on the device: there is nothing to upload."""
+        return isinstance(scans, ScanTable) and scans is self.table
+
+    def ensure_scans(self, scans) -> ScanTable:
+        """``set_scans(scans)`` unless ``scans`` is the ScanTable already resident; returns the resident table."""
+        return self.table if self.is_resident(scans) else self.set_scans(scans)
+
     def set_scans(self, scans) -> ScanTable:
         table = scans if isinstance(scans, ScanTable) else ScanTable(scans)
-        _lib.check(self._L.icpb_upload_scans(self._h, _ptr(table.xy), _ptr(table.offsets), table.n_scans),
-                   "icpb_upload_scans")
-        self.table = table
-        self._keep = None
+        self._replace_table(table, "icpb_upload_scans", _ptr(table.xy), _ptr(table.offsets), table.n_scans)
         return table
 
     def set_scans_device(self, xy_t, offsets_t, table: ScanTable):
         """Borrow a scan table already resident in HBM (torch CUDA tensors)."""
         assert xy_t.is_cuda and offsets_t.is_cuda and xy_t.is_contiguous() and offsets_t.is_contiguous()
-        _lib.check(self._L.icpb_set_scans_device(self._h, ctypes.c_void_p(xy_t.data_ptr()),
-                                                 ctypes.c_void_p(offsets_t.data_ptr()), table.n_scans,
-                                                 table.longest), "icpb_set_scans_device")
-        self.table = table
-        self._keep = (xy_t, offsets_t)
+        self._replace_table(table, "icpb_set_scans_device", ctypes.c_void_p(xy_t.data_ptr()),
+                            ctypes.c_void_p(offsets_t.data_ptr()), table.n_scans, table.longest,
+                            keep=(xy_t, offsets_t))
 
     # -- submaps ------------------------------------------------------------------------------
     def set_submaps(self, members, transforms) -> np.ndarray:
@@ -374,25 +443,16 @@ class IcpEngine:
         for bad arguments and for merged coordinates beyond the library's bound, with the table unchanged."""
         if self.table is None:
             raise ValueError("no scan table set")
-        # the base: the table as the caller set it, unless this engine's own submaps are resident
-        base = self._base[0] if self._base is not None and self._base[1] is self.table else self.table
+        base = self._base if self._base is not None else self.table
         ids, rows = _submap_args(members, transforms, base.n_scans)
         sub_off = np.concatenate(([0], np.cumsum([len(a) for a in ids]))).astype(np.int64)
         mem = np.ascontiguousarray(np.concatenate(ids) if ids else np.zeros(0, np.int32))
         T6 = np.ascontiguousarray(np.concatenate(rows) if rows else np.zeros((0, 6)))
-        try:
-            _lib.check(self._L.icpb_set_submaps(self._h, _ptr(mem), _ptr(sub_off), _ptr(T6), len(ids)),
-                       "icpb_set_submaps")
-        except Exception:
-            if self._L.icpb_scan_count(self._h) == 0:           # failed part-way: the library dropped the table
-                self.table, self._base = None, None
-            raise
+        table = base
         if ids:
-            lengths = np.concatenate((base.lengths, [int(base.lengths[a].sum()) for a in ids]))
-            self.table = ScanTable.from_lengths(lengths)
-            self._base = (base, self.table)
-        else:
-            self.table, self._base = base, None
+            table = ScanTable.from_lengths(np.concatenate((base.lengths, [int(base.lengths[a].sum()) for a in ids])))
+        self._replace_table(table, "icpb_set_submaps", _ptr(mem), _ptr(sub_off), _ptr(T6), len(ids),
+                            keep=self._keep, base=base if ids else None)
         return np.arange(base.n_scans, base.n_scans + len(ids))
 
     # -- host-buffer run (the reference-facing call) -----------------------------------------
@@ -403,28 +463,14 @@ class IcpEngine:
         force) instead of the default exact chunk pruning; the results are identical."""
         if self.table is None:
             raise ValueError("no scan table set")
-        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive)
-        if all_pairs is not None:
-            # (k_first, k_block, k_stride, B): linear indices over i<j decoded on the device
-            p.pair_mode = 1
-            p.k_first, p.k_block, p.k_stride, B = (int(v) for v in all_pairs)
-            pairs_a = None
-        else:
-            pairs_a = np.ascontiguousarray(pairs, dtype=np.int32)
-            if pairs_a.size == 0:
-                pairs_a = pairs_a.reshape(0, 2)
-            if pairs_a.ndim != 2 or pairs_a.shape[1] != 2:
-                raise ValueError(f"pairs has shape {pairs_a.shape}; expected (B, 2) of (source, target) scan ids")
+        pairs_a = None
+        if all_pairs is None:
+            pairs_a = _pairs(pairs)
             if pairs_a.size and (pairs_a.min() < 0 or pairs_a.max() >= self.table.n_scans):
                 raise ValueError("pair index out of range")
-            B = len(pairs_a)
-            p.k_block = max(B, 1)
-        init6 = None
-        if init_transforms is not None:
-            it = np.asarray(init_transforms, dtype=np.float64)
-            if it.shape != (B, 3, 3):
-                raise ValueError(f"init_transforms has shape {it.shape}; expected ({B}, 3, 3)")
-            init6 = _to6(it)
+        B = len(pairs_a) if all_pairs is None else int(all_pairs[3])
+        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive, B, all_pairs)
+        init6 = None if init_transforms is None else _to6(_mats(init_transforms, B, "init_transforms"))
         cap = max_passes(p.max_iters) if return_history else 0
         if cap > 4096:
             raise ValueError("return_history with max_iters > 4094 is not supported")
@@ -454,16 +500,14 @@ class IcpEngine:
         composed guesses against its bounds (ValueError)."""
         if self.table is None:
             raise ValueError("no scan table set")
-        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive)
-        pairs_a = np.ascontiguousarray(pairs, dtype=np.int32)
-        if pairs_a.size == 0:
-            pairs_a = pairs_a.reshape(0, 2)
-        if pairs_a.ndim != 2 or pairs_a.shape[1] != 2:
-            raise ValueError(f"pairs has shape {pairs_a.shape}; expected (B, 2) of (source, target) scan ids")
+        pairs_a = _pairs(pairs)
         B = len(pairs_a)
-        S6 = _rows6(starts, None, "starts")
+        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive, B)
+        S6 = _to6(_mats(starts, None, "starts"), bounds=False, name="starts")
         K = len(S6)
-        init6 = None if init_transforms is None else _rows6(init_transforms, B, "init_transforms")
+        init6 = None
+        if init_transforms is not None:
+            init6 = _to6(_mats(init_transforms, B, "init_transforms"), bounds=False, name="init_transforms")
         T6, err = np.empty((B, 6)), np.empty(B)
         passes, start = np.empty(B, dtype=np.int32), np.empty(B, dtype=np.int32)
         err_all = np.empty((B, K)) if return_all else None
@@ -482,35 +526,20 @@ class IcpEngine:
         ScanTable (packed, ideally pinned) or the reference's own list of (m_i, 2) arrays, which the
         library packs into pinned staging with a few host threads while earlier pieces are on the wire.
         ``epilogue``: fused all-gather / acceptance of the records (multi-GPU, see dist.FusedGather)."""
-        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive)
-        pairs_a = np.ascontiguousarray(pairs, dtype=np.int32)
-        if pairs_a.size == 0:
-            pairs_a = pairs_a.reshape(0, 2)
-        if pairs_a.ndim != 2 or pairs_a.shape[1] != 2:
-            raise ValueError(f"pairs has shape {pairs_a.shape}; expected (B, 2) of (source, target) scan ids")
+        pairs_a = _pairs(pairs)
         B = len(pairs_a)
-        p.k_block = max(B, 1)
-        init33 = None
-        if init_transforms is not None:
-            # the reference's (B, 3, 3) matrices go to the library as they are: it checks the pair
-            # indices, the bottom rows and finiteness while it stages them (ICPB_EINVAL -> ValueError)
-            init33 = np.ascontiguousarray(init_transforms, dtype=np.float64)
-            if init33.shape != (B, 3, 3):
-                raise ValueError(f"init_transforms has shape {init33.shape}; expected ({B}, 3, 3)")
-        T33 = np.empty((B, 3, 3))
-        err = np.empty(B)
-        passes = np.empty(B, dtype=np.int32)
-        ep = ctypes.byref(epilogue) if epilogue is not None else None
-        prev, self.table = (self.table, self._keep), None
-        try:
-            table = self._align_call(scans, pairs_a, init33, B, p, T33, err, passes, ep)
-        except Exception:
-            # rejected before anything was touched (bad pairs / guesses): the old table is still there;
-            # failed part-way: the library has dropped it (icpb_scan_count == 0)
-            if self._L.icpb_scan_count(self._h) > 0:
-                self.table, self._keep = prev
-            raise
-        self.table, self._keep = table, None
+        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive, B)
+        # the reference's (B, 3, 3) matrices go to the library as they are: it checks the pair
+        # indices, the bottom rows and finiteness while it stages them (ICPB_EINVAL -> ValueError)
+        init33 = None if init_transforms is None else _mats(init_transforms, B, "init_transforms")
+        table, _held, (xy, off, scan_ptrs, scan_lens) = _upload_args(scans)
+        T33, err, passes = np.empty((B, 3, 3)), np.empty(B), np.empty(B, dtype=np.int32)
+        args = (table.n_scans, _ptr(pairs_a), _ptr(init33), 9, B, ctypes.byref(p), _ptr(T33), 9, _ptr(err),
+                _ptr(passes), ctypes.byref(epilogue) if epilogue is not None else None)
+        if xy is not None:
+            self._replace_table(table, "icpb_align_host_ex", xy, off, *args)
+        else:
+            self._replace_table(table, "icpb_align_host_scans", scan_ptrs, scan_lens, *args)
         return BatchResult(T33, err, passes, None, None)
 
     def align_accept(self, scans, pairs, accept_thresh, init_transforms=None, epsilon=0.01, max_iters=100,
@@ -519,113 +548,45 @@ class IcpEngine:
         (src/loop_closure_detection.py:35-39, :155-159) and the compaction run in the kernel epilogue and
         only the accepted constraints come back.  Returns (rows, BatchResult): `rows` are ascending
         indices into `pairs`, the BatchResult holds their results."""
-        p = _params(epsilon, max_iters, stopping_thresh, rotation_only)
-        pairs_a = np.ascontiguousarray(pairs, dtype=np.int32).reshape(-1, 2)
+        pairs_a = _pairs(pairs)
         B = len(pairs_a)
         if B == 0:
             return np.zeros(0, dtype=np.int64), BatchResult(np.zeros((0, 3, 3)), np.zeros(0), np.zeros(0, dtype=np.int32))
-        p.k_block = B
-        init33 = None
-        if init_transforms is not None:
-            init33 = np.ascontiguousarray(init_transforms, dtype=np.float64)
-            if init33.shape != (B, 3, 3):
-                raise ValueError(f"init_transforms has shape {init33.shape}; expected ({B}, 3, 3)")
-        if isinstance(scans, ScanTable) and self.table is scans:
-            # the table is already resident: nothing to upload, so nothing to overlap with -- align on it
-            # and filter the (B x 60 byte) results on the host
+        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, B=B)
+        init33 = None if init_transforms is None else _mats(init_transforms, B, "init_transforms")
+        if self.is_resident(scans):
+            # nothing to upload, so nothing to overlap with: align on the resident table and filter the
+            # (B x 60 byte) results on the host
             res = self.run(pairs_a, init_transforms, epsilon, max_iters, stopping_thresh, rotation_only)
             keep = np.nonzero(res.error < accept_thresh)[0]
-            return keep, BatchResult(res.T[keep], res.error[keep], res.iters[keep])
+            return keep, res.take(keep)
+        table, _held, table_args = _upload_args(scans)
         rows = np.empty(B, dtype=np.int64)
         T33, err, passes = np.empty((B, 3, 3)), np.empty(B), np.empty(B, dtype=np.int32)
         n = ctypes.c_int64()
-        prev, self.table = (self.table, self._keep), None
-        try:
-            if isinstance(scans, ScanTable):
-                table, xy, off, ptrs, lens, ns = scans, _ptr(scans.xy), _ptr(scans.offsets), None, None, scans.n_scans
-            else:
-                sl = scans if isinstance(scans, ScanList) else ScanList(scans)
-                table, xy, off, ptrs, lens, ns = ScanTable.from_lengths(sl.lens), None, None, _ptr(sl.ptrs), _ptr(sl.lens), sl.n_scans
-            _lib.check(self._L.icpb_align_host_accept(self._h, xy, off, ptrs, lens, ns, _ptr(pairs_a), _ptr(init33), 9, B,
-                                                      ctypes.byref(p), float(accept_thresh), B, ctypes.byref(n),
-                                                      _ptr(rows), _ptr(T33), 9, _ptr(err), _ptr(passes)),
-                       "icpb_align_host_accept")
-        except Exception:
-            if self._L.icpb_scan_count(self._h) > 0:
-                self.table, self._keep = prev
-            raise
-        self.table, self._keep = table, None
+        self._replace_table(table, "icpb_align_host_accept", *table_args, table.n_scans, _ptr(pairs_a), _ptr(init33),
+                            9, B, ctypes.byref(p), float(accept_thresh), B, ctypes.byref(n), _ptr(rows), _ptr(T33),
+                            9, _ptr(err), _ptr(passes))
         k = int(n.value)
         return rows[:k].copy(), BatchResult(T33[:k].copy(), err[:k].copy(), passes[:k].copy())
-
-    def _align_call(self, scans, pairs_a, init33, B, p, T33, err, passes, ep):
-        if isinstance(scans, ScanTable):
-            table = scans
-            if table.xy is None:
-                raise ValueError("this ScanTable only describes a resident table; pass the scans themselves")
-            _lib.check(self._L.icpb_align_host_ex(self._h, _ptr(table.xy), _ptr(table.offsets), table.n_scans,
-                                                  _ptr(pairs_a), _ptr(init33), 9, B, ctypes.byref(p),
-                                                  _ptr(T33), 9, _ptr(err), _ptr(passes), ep), "icpb_align_host")
-        else:
-            sl = scans if isinstance(scans, ScanList) else ScanList(scans)
-            _lib.check(self._L.icpb_align_host_scans(self._h, _ptr(sl.ptrs), _ptr(sl.lens), sl.n_scans,
-                                                     _ptr(pairs_a), _ptr(init33), 9, B, ctypes.byref(p),
-                                                     _ptr(T33), 9, _ptr(err), _ptr(passes), ep),
-                       "icpb_align_host_scans")
-            table = ScanTable.from_lengths(sl.lens)
-        return table
 
     # -- device-buffer run (inputs and outputs resident in HBM; torch tensors) ---------------
     def run_device(self, pairs_t, init_t, out_T, out_err, out_passes, epsilon=0.01, max_iters=100,
                    stopping_thresh=0.0001, rotation_only=False, all_pairs: tuple | None = None,
                    stream=None, exhaustive: bool = False):
         """Asynchronous launch on torch's current stream (or `stream`, a raw cudaStream_t int).
-        pairs_t (B,2) int32, init_t (B,6) float64 or None, outputs (B,6) f64, (B,) f64, (B,) i32."""
-        import torch
-        p = _params(epsilon, max_iters, stopping_thresh, rotation_only, exhaustive)
-        if all_pairs is not None:
-            p.pair_mode = 1
-            p.k_first, p.k_block, p.k_stride, B = (int(v) for v in all_pairs)
-        else:
-            B = int(pairs_t.shape[0])
-            p.k_block = max(B, 1)
-            assert pairs_t.dtype == torch.int32 and pairs_t.is_cuda and pairs_t.is_contiguous()
-        assert out_T.dtype == torch.float64 and out_T.numel() == 6 * B and out_T.is_contiguous()
-        assert out_err.dtype == torch.float64 and out_err.numel() == B
-        assert out_passes.dtype == torch.int32 and out_passes.numel() == B
-        if init_t is not None:
-            assert init_t.dtype == torch.float64 and init_t.numel() == 6 * B and init_t.is_contiguous()
-        if stream is None:
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-        vp = ctypes.c_void_p
-        _lib.check(self._L.icpb_run_device(self._h, vp(pairs_t.data_ptr()) if all_pairs is None else None,
-                                           vp(init_t.data_ptr()) if init_t is not None else None, B,
-                                           ctypes.byref(p), vp(out_T.data_ptr()), vp(out_err.data_ptr()),
-                                           vp(out_passes.data_ptr()), None, None, vp(stream)),
-                   "icpb_run_device")
+        pairs_t (B,2) int32, init_t (B,6) float64 or None, outputs (B,6) f64, (B,) f64, (B,) i32;
+        ValueError for a buffer of another dtype or size, not contiguous or not on the device."""
+        self._run_device(pairs_t, init_t, out_T, out_err, out_passes, None, all_pairs, stream,
+                         (epsilon, max_iters, stopping_thresh, rotation_only, exhaustive))
 
     def run_device_ex(self, pairs_t, init_t, out_T, out_err, out_passes, epilogue: _lib.IcpbEpilogue | None,
                       epsilon=0.01, max_iters=100, stopping_thresh=0.0001, rotation_only=False,
                       all_pairs: tuple | None = None, stream=None):
         """`run_device` with kernel epilogues (icpb_run_device_ex): the fused all-gather of the
         constraint records into every rank's buffer and/or the acceptance test + compaction."""
-        import torch
-        p = _params(epsilon, max_iters, stopping_thresh, rotation_only)
-        if all_pairs is not None:
-            p.pair_mode = 1
-            p.k_first, p.k_block, p.k_stride, B = (int(v) for v in all_pairs)
-        else:
-            B = int(pairs_t.shape[0])
-            p.k_block = max(B, 1)
-        if stream is None:
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-        vp = ctypes.c_void_p
-        _lib.check(self._L.icpb_run_device_ex(self._h, vp(pairs_t.data_ptr()) if all_pairs is None else None,
-                                              vp(init_t.data_ptr()) if init_t is not None else None, B,
-                                              ctypes.byref(p), vp(out_T.data_ptr()), vp(out_err.data_ptr()),
-                                              vp(out_passes.data_ptr()),
-                                              ctypes.byref(epilogue) if epilogue is not None else None, vp(stream)),
-                   "icpb_run_device_ex")
+        self._run_device(pairs_t, init_t, out_T, out_err, out_passes, epilogue, all_pairs, stream,
+                         (epsilon, max_iters, stopping_thresh, rotation_only, False))
 
     def run_device_gather(self, pairs_t, init_t, out_T, out_err, out_passes, peer_ptrs_dev: int, n_peers: int,
                           row0: int, epsilon=0.01, max_iters=100, stopping_thresh=0.0001, rotation_only=False,
@@ -638,6 +599,28 @@ class IcpEngine:
         self.run_device_ex(pairs_t, init_t, out_T, out_err, out_passes, ep, epsilon, max_iters, stopping_thresh,
                            rotation_only, stream=stream)
 
+    def _run_device(self, pairs_t, init_t, out_T, out_err, out_passes, epilogue, all_pairs, stream, params):
+        """The one launch behind the run_device* methods: icpb_run_device_ex, which with a null epilogue is
+        icpb_run_device without history or correspondences.  ``params``: _params' leading arguments."""
+        import torch
+        B = int(pairs_t.shape[0]) if all_pairs is None else int(all_pairs[3])
+        p = _params(*params, B=B, all_pairs=all_pairs)
+        if all_pairs is None:
+            _check_buffer(pairs_t, torch.int32, 2 * B, "pairs_t")
+        if init_t is not None:
+            _check_buffer(init_t, torch.float64, 6 * B, "init_t")
+        _check_buffer(out_T, torch.float64, 6 * B, "out_T")
+        _check_buffer(out_err, torch.float64, B, "out_err")
+        _check_buffer(out_passes, torch.int32, B, "out_passes")
+        if stream is None:
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+        vp = ctypes.c_void_p
+        _lib.check(self._L.icpb_run_device_ex(self._h, vp(pairs_t.data_ptr()) if all_pairs is None else None,
+                                              vp(init_t.data_ptr()) if init_t is not None else None, B,
+                                              ctypes.byref(p), vp(out_T.data_ptr()), vp(out_err.data_ptr()),
+                                              vp(out_passes.data_ptr()),
+                                              ctypes.byref(epilogue) if epilogue is not None else None, vp(stream)),
+                   "icpb_run_device_ex")
     # -- one pair given as two arrays ------------------------------------------------------------
     def pair(self, src_xy, dst_xy, init6, p: _lib.IcpbParams, want_hist: bool, want_corr: bool):
         src = np.ascontiguousarray(src_xy, dtype=np.float64)
@@ -790,12 +773,9 @@ def icp_batch(scans, pairs, init_transforms=None, epsilon=0.01, max_iters=100, s
     for every pair.
     """
     e = engine(device)
-    if isinstance(scans, ScanTable) and e.table is scans:          # already resident
-        return e.run(pairs, init_transforms, epsilon, max_iters, stopping_thresh, rotation_only,
-                     return_history, return_correspondences)
-    if not (return_history or return_correspondences):
+    if not (return_history or return_correspondences or e.is_resident(scans)):
         return e.align(scans, pairs, init_transforms, epsilon, max_iters, stopping_thresh, rotation_only)
-    e.set_scans(scans)
+    e.ensure_scans(scans)
     return e.run(pairs, init_transforms, epsilon, max_iters, stopping_thresh, rotation_only,
                  return_history, return_correspondences)
 
@@ -810,7 +790,6 @@ def icp_multistart(scans, pairs, starts, init_transforms=None, epsilon=0.01, max
     adds every start's error and pass count, (B, K).  ``scans`` is uploaded unless it is the ScanTable
     already resident on the device."""
     e = engine(device)
-    if not (isinstance(scans, ScanTable) and e.table is scans):
-        e.set_scans(scans)
+    e.ensure_scans(scans)
     return e.run_multistart(pairs, starts, init_transforms, epsilon, max_iters, stopping_thresh, rotation_only,
                             return_all)

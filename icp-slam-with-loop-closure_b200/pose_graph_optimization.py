@@ -15,8 +15,6 @@ No CPU fallback: without libicpb.so and a B200 these raise.
 """
 from __future__ import annotations
 
-import ctypes
-
 import numpy as np
 
 from . import _lib
@@ -57,8 +55,7 @@ def edge_arrays(pose_graph):
                 raise ValueError(f"edge ({a}, {b}) carries a transform of shape {T.shape}; expected (3, 3)")
             if not (T[2, 0] == 0.0 and T[2, 1] == 0.0 and T[2, 2] == 1.0):
                 raise ValueError(f"edge ({a}, {b}): the transform's bottom row is not [0, 0, 1]")
-    return (np.asarray(ab, dtype=np.int32).reshape(-1, 2),
-            np.ascontiguousarray(tf[:, :2, :]).reshape(-1, 6))
+    return np.asarray(ab, dtype=np.int32).reshape(-1, 2), _icp._top_rows(tf)
 
 
 def sgd_steps(poses, edges_ab, edges_T6, learning_rates, loop_closure_uncertainty=0.1, device=None):
@@ -72,11 +69,10 @@ def sgd_steps(poses, edges_ab, edges_T6, learning_rates, loop_closure_uncertaint
         raise ValueError("edges and transforms differ in length")
     lrs = np.ascontiguousarray(learning_rates, dtype=np.float64).reshape(-1)
     eng = _icp.engine(device)
-    vp = ctypes.c_void_p
-    _lib.check(_lib.lib().icpb_pose_graph_sgd(eng._h, vp(poses.ctypes.data), len(poses),
-                                               vp(ab.ctypes.data) if len(ab) else None,
-                                               vp(T6.ctypes.data) if len(ab) else None, len(ab),
-                                               vp(lrs.ctypes.data) if len(lrs) else None, len(lrs),
+    _lib.check(_lib.lib().icpb_pose_graph_sgd(eng._h, _lib.ptr(poses), len(poses),
+                                               _lib.ptr(ab) if len(ab) else None,
+                                               _lib.ptr(T6) if len(ab) else None, len(ab),
+                                               _lib.ptr(lrs) if len(lrs) else None, len(lrs),
                                                float(loop_closure_uncertainty)),
                "icpb_pose_graph_sgd")
     return poses

@@ -35,18 +35,13 @@ def _stage(poses, lidar_points, device):
     if n_scans != len(poses):
         raise ValueError(f"{len(poses)} poses for {n_scans} scans")
     eng = _icp.engine(device)
-    if isinstance(lidar_points, _icp.ScanTable):
-        if eng.table is not lidar_points:
-            eng.set_scans(lidar_points)
-    else:
-        eng.set_scans(lidar_points)
+    eng.ensure_scans(lidar_points)
     return eng, poses
 
 
 def _update(eng, poses, grid, cell_width, min_x, min_y, k_hit, k_miss):
-    vp = ctypes.c_void_p
-    _lib.check(_lib.lib().icpb_occupancy_grid_update(eng._h, vp(poses.ctypes.data), len(poses),
-                                                     vp(grid.ctypes.data), grid.shape[0], grid.shape[1],
+    _lib.check(_lib.lib().icpb_occupancy_grid_update(eng._h, _lib.ptr(poses), len(poses),
+                                                     _lib.ptr(grid), grid.shape[0], grid.shape[1],
                                                      float(min_x), float(min_y), float(cell_width),
                                                      k_hit, k_miss),
                "icpb_occupancy_grid_update")
@@ -58,7 +53,7 @@ def produce_occupancy_grid(poses, lidar_points, cell_width, min_width=0, min_hei
     eng, poses = _stage(poses, lidar_points, device)
     min_x, min_y = ctypes.c_double(), ctypes.c_double()
     h, w = ctypes.c_int64(), ctypes.c_int64()
-    _lib.check(_lib.lib().icpb_occupancy_grid_bounds(eng._h, ctypes.c_void_p(poses.ctypes.data), len(poses),
+    _lib.check(_lib.lib().icpb_occupancy_grid_bounds(eng._h, _lib.ptr(poses), len(poses),
                                                      float(cell_width), float(min_width), float(min_height),
                                                      ctypes.byref(min_x), ctypes.byref(min_y),
                                                      ctypes.byref(h), ctypes.byref(w)),
