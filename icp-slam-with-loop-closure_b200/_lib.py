@@ -59,6 +59,8 @@ SIGNATURES = {
     "icpb_upload_scans": (_i, [_v, _v, _v, _i64]),
     "icpb_set_scans_device": (_i, [_v, _v, _v, _i64, _i64]),
     "icpb_set_submaps": (_i, [_v, _v, _v, _v, _i64]),
+    "icpb_set_submaps_voxel": (_i, [_v, _v, _v, _v, _i64, _f64, _v]),
+    "icpb_read_scans": (_i, [_v, _i64, _i64, _v]),
     "icpb_run_device": (_i, [_v, _v, _v, _i64, _P, _v, _v, _v, _v, _v, _v]),
     "icpb_run_device_gather": (_i, [_v, _v, _v, _i64, _P, _v, _v, _v, _v, _i32, _i64, _v]),
     "icpb_run_device_ex": (_i, [_v, _v, _v, _i64, _P, _v, _v, _v, _E, _v]),

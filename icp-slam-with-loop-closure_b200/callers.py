@@ -173,15 +173,16 @@ def submap_window_transforms(poses, targets, members) -> list:
     return out
 
 
-def _submap_accept(poses, lidar_points, cand, starts, thresh, window, epsilon, max_iters, device):
+def _submap_accept(poses, lidar_points, cand, starts, thresh, window, voxel, epsilon, max_iters, device):
     """Every candidate's source scan j aligned onto the submap around its target i (``submap_window_*``),
-    built on the device from the resident table; the pairs whose (best) error is below ``thresh``: (rows,
-    result of those rows).  The submaps are dropped again afterwards, leaving the scan table resident."""
+    built on the device from the resident table and thinned by ``voxel`` (None: not); the pairs whose (best)
+    error is below ``thresh``: (rows, result of those rows).  The submaps are dropped again afterwards,
+    leaving the scan table resident."""
     e = _icp.engine(device)
     n = e.ensure_scans(lidar_points).n_scans
     targets, sub = np.unique(cand[:, 0], return_inverse=True)
     members = submap_window_members(n, targets, window)
-    ids = e.set_submaps(members, submap_window_transforms(poses, targets, members))
+    ids = e.set_submaps(members, submap_window_transforms(poses, targets, members), voxel=voxel)
     try:
         pairs = np.stack((cand[:, 1], ids[sub]), axis=1).astype(np.int32)
         if starts is not None:
@@ -195,7 +196,8 @@ def _submap_accept(poses, lidar_points, cand, starts, thresh, window, epsilon, m
 
 
 def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist=1, err_thresh=110,
-                            max_iters=100, epsilon=0.05, device=None, starts=None, submap_window=None):
+                            max_iters=100, epsilon=0.05, device=None, starts=None, submap_window=None,
+                            submap_voxel=None):
     """Loop-closure constraints the reference's ``detect_proximity`` would add, in its order.
 
     ICP is a pure function of its inputs, so every candidate is aligned in one batch
@@ -215,16 +217,25 @@ def proximity_loop_closures(poses, lidar_points, min_dist_along_path=2, max_dist
     ``poses`` (``IcpEngine.set_submaps``), so a source that overlaps scan i only partly still finds its
     structure.  The submap sits in scan i's frame, so the constraint (i, j, T) keeps its meaning, and the
     error is still an SSE over scan j's points, so ``err_thresh`` keeps its scale.  w = 0 gives exactly the
-    constraints of ``submap_window=None``."""
+    constraints of ``submap_window=None``.
+
+    ``submap_voxel`` (a cell size, with ``submap_window``): every target submap is thinned on the device to
+    the first point of every grid cell (``IcpEngine.set_submaps(..., voxel=)``), so the copies of one wall
+    that overlapping members bring are kept once.  Source scans are not filtered, so the error is still an
+    SSE over scan j's points and ``err_thresh`` keeps its scale."""
     if submap_window is not None and (int(submap_window) != submap_window or submap_window < 0):
         raise ValueError("submap_window must be an integer >= 0")
+    if submap_voxel is not None:
+        if submap_window is None:
+            raise ValueError("submap_voxel filters the target submaps: it needs submap_window")
+        _icp._voxel_arg(submap_voxel)
     cand = proximity_candidates(poses, min_dist_along_path, max_dist, device)
     if len(cand) == 0:
         return [], None
     pairs = np.stack((cand[:, 1], cand[:, 0]), axis=1).astype(np.int32)
     if submap_window is not None:
-        rows, res = _submap_accept(poses, lidar_points, cand, starts, err_thresh, int(submap_window), epsilon,
-                                   max_iters, device)
+        rows, res = _submap_accept(poses, lidar_points, cand, starts, err_thresh, int(submap_window), submap_voxel,
+                                   epsilon, max_iters, device)
     elif starts is not None:
         rows, res = _multistart_accept(lidar_points, pairs, starts, err_thresh, epsilon, max_iters, device)
     else:

@@ -27,6 +27,9 @@
 #include "icpb_multistart.cuh"
 #include "icpb_submaps.cuh"
 
+#include <cub/device/device_scan.cuh>
+#include <float.h>
+
 namespace {
 
 thread_local char g_err[512] = "";
@@ -978,21 +981,67 @@ int icpb_run_host(icpb_handle h, const int32_t *h_pairs, const double *h_init, i
 
 namespace {
 
+// Blocks of a grid-stride submap kernel over n items (n >= 1).
+unsigned submap_blocks(const icpb_ctx *h, int64_t n)
+{
+    int64_t blocks = (n + icpb::kSubmapThreads - 1) / icpb::kSubmapThreads;
+    if (blocks > 16 * (int64_t)h->sm_count) blocks = 16 * (int64_t)h->sm_count;
+    return (unsigned)blocks;
+}
+
 // One pass of the merge kernel over the submaps' n_pts points: check mode (out == nullptr) or write mode.
 cudaError_t merge_submaps(icpb_ctx *h, const int64_t *src, const int64_t *mout, const double *T, int64_t n_members,
                           int64_t n_pts, double *out, int32_t *bad)
 {
-    int64_t blocks = (n_pts + icpb::kSubmapThreads - 1) / icpb::kSubmapThreads;
-    if (blocks > 16 * (int64_t)h->sm_count) blocks = 16 * (int64_t)h->sm_count;
-    icpb::submap_merge_kernel<<<(unsigned)blocks, icpb::kSubmapThreads, 0, h->stream>>>(
+    icpb::submap_merge_kernel<<<submap_blocks(h, n_pts), icpb::kSubmapThreads, 0, h->stream>>>(
         (const double2 *)h->xy, src, mout, T, n_members, (double2 *)out, bad);
     return cudaGetLastError();
 }
 
+// The voxel filter's scratch in the arena (icpb_set_submaps_voxel): the merged points, per-submap point and
+// hash offsets, the hashes, the keep flags (scanned in place into output positions, one past the end so that
+// the last entry is the total), the kept points before each submap, and the scan's temporary storage.
+struct VoxelScratch {
+    double *pts;
+    int64_t *soff, *hoff, *pos, *kept_off;
+    int32_t *hash;
+    void *tmp;
+    size_t tmp_bytes;
+};
+
+// The filter up to the kept counts, all on the stream: merge into scratch, insert every point's cell, flag
+// the first point of every cell, scan the flags, and gather the scan at the submap boundaries into kept_off.
+// The caller copies kept_off back and synchronises.  h_soff / h_hoff: n_submaps + 1 host offsets.
+int voxel_filter(icpb_ctx *h, const VoxelScratch &v, const int64_t *src, const int64_t *mout, const double *T,
+                 int64_t n_members, const int64_t *h_soff, const int64_t *h_hoff, int64_t n_submaps, double voxel)
+{
+    cudaStream_t st = h->stream;
+    const int64_t n_pts = h_soff[n_submaps], n_slots = h_hoff[n_submaps];
+    CU(merge_submaps(h, src, mout, T, n_members, n_pts, v.pts, nullptr));
+    CU(cudaMemcpyAsync(v.soff, h_soff, 8 * (size_t)(n_submaps + 1), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(v.hoff, h_hoff, 8 * (size_t)(n_submaps + 1), cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(v.hash, 0xff, 4 * (size_t)n_slots, st));
+    CU(cudaMemsetAsync(v.pos, 0, 8 * (size_t)(n_pts + 1), st));
+    icpb::submap_voxel_insert_kernel<<<submap_blocks(h, n_pts), icpb::kSubmapThreads, 0, st>>>(
+        (const double2 *)v.pts, v.soff, v.hoff, n_submaps, voxel, v.hash);
+    CU(cudaGetLastError());
+    icpb::submap_voxel_keep_kernel<<<submap_blocks(h, n_slots), icpb::kSubmapThreads, 0, st>>>(
+        v.hash, v.soff, v.hoff, n_submaps, v.pos);
+    CU(cudaGetLastError());
+    size_t tmp_bytes = v.tmp_bytes;
+    CU(cub::DeviceScan::ExclusiveSum(v.tmp, tmp_bytes, v.pos, v.pos, n_pts + 1, st));
+    icpb::submap_voxel_bounds_kernel<<<submap_blocks(h, n_submaps + 1), icpb::kSubmapThreads, 0, st>>>(
+        v.pos, v.soff, n_submaps, v.kept_off);
+    CU(cudaGetLastError());
+    return 0;
+}
+
 // Write mode of icpb_set_submaps, after the check: the base into xy / off unless it is already there, the
-// submaps' offsets and points after it.
+// submaps' offsets, then their points -- merged from the base (v == nullptr), or the kept points of the voxel
+// filter's merged points in scratch.
 cudaError_t write_submaps(icpb_ctx *h, double *xy, int64_t *off, const int64_t *comb, int64_t n_submaps,
-                          const int64_t *src, const int64_t *mout, const double *T, int64_t n_members)
+                          const int64_t *src, const int64_t *mout, const double *T, int64_t n_members,
+                          const VoxelScratch *v, int64_t n_merged)
 {
     const int64_t nb = h->n_base, base_pts = comb[nb];
     cudaStream_t st = h->stream;
@@ -1003,8 +1052,13 @@ cudaError_t write_submaps(icpb_ctx *h, double *xy, int64_t *off, const int64_t *
         e = cudaMemcpyAsync(off, h->offsets, sizeof(int64_t) * (size_t)(nb + 1), cudaMemcpyDeviceToDevice, st);
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(off + nb + 1, comb + nb + 1, sizeof(int64_t) * (size_t)n_submaps, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess)
+    if (e == cudaSuccess && !v)
         e = merge_submaps(h, src, mout, T, n_members, comb[nb + n_submaps] - base_pts, xy + 2 * base_pts, nullptr);
+    if (e == cudaSuccess && v) {
+        icpb::submap_voxel_scatter_kernel<<<submap_blocks(h, n_merged), icpb::kSubmapThreads, 0, st>>>(
+            (const double2 *)v->pts, v->pos, n_merged, (double2 *)(xy + 2 * base_pts));
+        e = cudaGetLastError();
+    }
     const cudaError_t s = cudaStreamSynchronize(st);
     return e != cudaSuccess ? e : s;
 }
@@ -1016,8 +1070,16 @@ extern "C" {
 int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_submap_off,
                      const double *h_member_T, int64_t n_submaps)
 {
+    return icpb_set_submaps_voxel(h, h_members, h_submap_off, h_member_T, n_submaps, 0.0, nullptr);
+}
+
+int icpb_set_submaps_voxel(icpb_handle h, const int32_t *h_members, const int64_t *h_submap_off,
+                           const double *h_member_T, int64_t n_submaps, double voxel, int64_t *h_submap_len)
+{
     if (!h) return fail(ICPB_EINVAL, "handle is null%s");
     if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
+    if (!(voxel == 0.0 || (voxel >= ICPB_MIN_VOXEL && voxel <= DBL_MAX)))
+        return fail(ICPB_EINVAL, "icpb_set_submaps: voxel must be 0 or a finite size of at least ICPB_MIN_VOXEL%s");
     if (n_submaps < 0 || !h_submap_off) return fail(ICPB_EINVAL, "icpb_set_submaps: negative count or null offsets%s");
     if (h_submap_off[0] != 0) return fail(ICPB_EINVAL, "icpb_set_submaps: submap offsets must start at 0%s");
     for (int64_t m = 0; m < n_submaps; ++m)
@@ -1066,9 +1128,32 @@ int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_s
     }
     // check mode: nothing is written until every merged coordinate is known to be within ICPB_MAX_COORD
     cudaStream_t st = h->stream;
+    const int64_t n_pts = mout[(size_t)n_mem];
+    const bool filter = voxel > 0.0;
+    // the voxel filter: per-submap point offsets in the merged scratch and hash offsets (a power of two of at
+    // least twice the submap's length each)
+    std::vector<int64_t> soff, hoff;
+    if (filter) {
+        soff.resize((size_t)n_submaps + 1); hoff.resize((size_t)n_submaps + 1);
+        soff[0] = hoff[0] = 0;
+        for (int64_t m = 0; m < n_submaps; ++m) {
+            const int64_t len = comb[(size_t)(nb + m + 1)] - comb[(size_t)(nb + m)];
+            int64_t cap = 1;
+            while (cap < 2 * len) cap *= 2;
+            soff[(size_t)m + 1] = soff[(size_t)m] + len;
+            hoff[(size_t)m + 1] = hoff[(size_t)m] + cap;
+        }
+    }
+    VoxelScratch v = {};
+    if (filter)
+        CU(cub::DeviceScan::ExclusiveSum(nullptr, v.tmp_bytes, (int64_t *)nullptr, (int64_t *)nullptr, n_pts + 1, st));
     Carve c;
     const size_t o_src = c(8 * (size_t)n_mem), o_mout = c(8 * (size_t)(n_mem + 1));
     const size_t o_T = c(48 * (size_t)n_mem), o_bad = c(sizeof(int32_t));
+    const size_t o_pts = c(filter ? 16 * (size_t)n_pts : 0), o_soff = c(filter ? 8 * (size_t)(n_submaps + 1) : 0);
+    const size_t o_hoff = c(filter ? 8 * (size_t)(n_submaps + 1) : 0), o_hash = c(filter ? 4 * (size_t)hoff.back() : 0);
+    const size_t o_pos = c(filter ? 8 * (size_t)(n_pts + 1) : 0), o_kept = c(filter ? 8 * (size_t)(n_submaps + 1) : 0);
+    const size_t o_tmp = c(v.tmp_bytes);
     if ((rc = h->arena.reserve(c.used))) return rc;
     const int64_t *d_src = at<int64_t>(h->arena, o_src), *d_mout = at<int64_t>(h->arena, o_mout);
     const double *d_T = at<double>(h->arena, o_T);
@@ -1077,11 +1162,29 @@ int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_s
     CU(cudaMemcpyAsync((void *)d_mout, mout.data(), 8 * (size_t)(n_mem + 1), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync((void *)d_T, h_member_T, 48 * (size_t)n_mem, cudaMemcpyHostToDevice, st));
     CU(cudaMemsetAsync(d_bad, 0, sizeof(int32_t), st));
-    const int64_t n_pts = mout[(size_t)n_mem];
     CU(merge_submaps(h, d_src, d_mout, d_T, n_mem, n_pts, nullptr, d_bad));
+    // the filter runs on scratch whatever the check finds; its kept counts come back with the flag
+    std::vector<int64_t> kept;
+    if (filter) {
+        v.pts = at<double>(h->arena, o_pts); v.soff = at<int64_t>(h->arena, o_soff);
+        v.hoff = at<int64_t>(h->arena, o_hoff); v.hash = at<int32_t>(h->arena, o_hash);
+        v.pos = at<int64_t>(h->arena, o_pos); v.kept_off = at<int64_t>(h->arena, o_kept);
+        v.tmp = at<void>(h->arena, o_tmp);
+        if ((rc = voxel_filter(h, v, d_src, d_mout, d_T, n_mem, soff.data(), hoff.data(), n_submaps, voxel))) return rc;
+        kept.resize((size_t)n_submaps + 1);
+        CU(cudaMemcpyAsync(kept.data(), v.kept_off, 8 * kept.size(), cudaMemcpyDeviceToHost, st));
+    }
     CU(cudaMemcpyAsync(&bad, d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (bad) return fail(ICPB_EINVAL, "icpb_set_submaps: a merged coordinate is non-finite or beyond ICPB_MAX_COORD%s");
+    if (filter) {                                             // the offsets and the longest scan from the kept counts
+        longest = base_longest;
+        for (int64_t m = 0; m < n_submaps; ++m) {
+            const int64_t len = kept[(size_t)m + 1] - kept[(size_t)m];
+            comb[(size_t)(nb + m + 1)] = comb[(size_t)(nb + m)] + len;
+            if (len > longest) longest = len;
+        }
+    }
     // write mode, into the handle's own table buffers.  One that is too small is replaced by a new block, which
     // is filled before the old one is freed: the resident table stays whole until the new one is (DevBuf::reserve
     // would free first).
@@ -1091,7 +1194,8 @@ int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_s
     if (nb_off > h->own_off.cap && (rc = noff.reserve(nb_off))) { nxy.release(); return rc; }
     double *xy = (double *)(nxy.p ? nxy.p : h->own_xy.p);
     int64_t *doff = (int64_t *)(noff.p ? noff.p : h->own_off.p);
-    const cudaError_t e = write_submaps(h, xy, doff, comb.data(), n_submaps, d_src, d_mout, d_T, n_mem);
+    const cudaError_t e = write_submaps(h, xy, doff, comb.data(), n_submaps, d_src, d_mout, d_T, n_mem,
+                                        filter ? &v : nullptr, n_pts);
     if (e != cudaSuccess) {
         nxy.release(); noff.release();
         // a failure part-way through writes into the resident table's own buffers leaves it half written
@@ -1103,6 +1207,24 @@ int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_s
     if (noff.p) { h->own_off.release(); h->own_off = noff; }
     set_table(h, xy, doff, nb + n_submaps, longest, comb.data());
     h->n_base = nb; h->base_longest = base_longest;
+    if (h_submap_len)
+        for (int64_t m = 0; m < n_submaps; ++m) h_submap_len[m] = comb[(size_t)(nb + m + 1)] - comb[(size_t)(nb + m)];
+    return 0;
+}
+
+int icpb_read_scans(icpb_handle h, int64_t first, int64_t count, double *h_xy)
+{
+    if (!h) return fail(ICPB_EINVAL, "handle is null%s");
+    if (!h->xy) return fail(ICPB_ENOSCANS, "no scan table set%s");
+    if (!h_xy || first < 0 || count < 0 || count > h->n_scans - first)
+        return fail(ICPB_EINVAL, "icpb_read_scans: null output or scans outside the table%s");
+    ON_DEVICE(h);
+    int rc;
+    const int64_t *off;
+    if ((rc = table_host_offsets(h, &off))) return rc;
+    const int64_t a = off[first], n = off[first + count] - a;
+    CU(cudaMemcpyAsync(h_xy, h->xy + 2 * a, 16 * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
     return 0;
 }
 

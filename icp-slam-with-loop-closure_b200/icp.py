@@ -14,7 +14,8 @@ plus the batched entry point ``icp_batch`` that replaces the reference's joblib 
 src/pose_graph_optimization.py:60-68) with one kernel launch, and ``icp_multistart``, which aligns
 every pair from K start transforms and keeps the best one (``heading_starts``, ``compose_starts``).
 ``IcpEngine.set_submaps`` merges resident scans into submaps on the device, for scan-to-submap matching;
-``merge_scans`` builds the same submaps on the host, bit for bit.
+``merge_scans`` builds the same submaps on the host, bit for bit, optionally thinned by a voxel filter to
+the first point of every grid cell.
 
 There is no CPU fallback: without libicpb.so and a B200 every call raises.
 """
@@ -40,6 +41,7 @@ __all__ = ["icp", "icp_iteration", "icp_batch", "icp_multistart", "heading_start
 MAX_COORD = 1e10
 MAX_GUESS_LINEAR = 1e3
 MAX_GUESS_SHIFT = 1e12
+MIN_VOXEL = 1e-6               # include/icpb.h: ICPB_MIN_VOXEL, the smallest nonzero submap voxel
 
 
 def _coords_ok(xy) -> bool:
@@ -251,17 +253,46 @@ def _submap_args(members, transforms, n_base: int):
     return ids, rows
 
 
-def merge_scans(scans, members, transforms) -> list:
+def _voxel_arg(voxel) -> float:
+    """``voxel`` of ``merge_scans`` / ``IcpEngine.set_submaps`` as the library's double: None or 0 -> 0.0 (no
+    filter); otherwise a finite cell size >= MIN_VOXEL, else ValueError."""
+    if voxel is None:
+        return 0.0
+    try:
+        v = float(voxel)
+    except (TypeError, ValueError):
+        raise ValueError(f"voxel must be a number, not {voxel!r}") from None
+    if not (v == 0.0 or (MIN_VOXEL <= v < np.inf)):
+        raise ValueError(f"voxel must be None, 0 or a finite size >= {MIN_VOXEL:g}; got {voxel!r}")
+    return v
+
+
+def _first_of_cell(points, voxel: float) -> np.ndarray:
+    """Indices of the points (an (n, 2) array) kept by the voxel filter, in order: the first point of every
+    cell (floor(x / voxel), floor(y / voxel)), the division correctly rounded as the library does."""
+    c = np.floor(points / voxel).astype(np.int64)
+    lo = c.min(axis=0)
+    span = c.max(axis=0) - lo + 1
+    if int(span[0]) <= (1 << 62) // int(span[1]):           # both cell coordinates in one int64 key
+        _, first = np.unique((c[:, 0] - lo[0]) * span[1] + (c[:, 1] - lo[1]), return_index=True)
+    else:
+        _, first = np.unique(c, axis=0, return_index=True)
+    return np.sort(first)                                    # unique's return_index gives first occurrences
+
+
+def merge_scans(scans, members, transforms, voxel=None) -> list:
     """Submaps built on the host with the library's bits: submap m is the scans ``members[m]`` (base scan ids)
     in order, member k's points mapped by ``transforms[m][k]`` ((k_m, 3, 3) SE(2)-shaped, into the submap's
     frame) as ``x' = (T00*x + T01*y) + T02``, ``y' = (T10*x + T11*y) + T12`` -- element-wise, every product
     and sum rounded on its own, which is what ``IcpEngine.set_submaps`` computes on the device (a matrix
-    product ``@`` may fuse or reorder them, and then the bits depend on the BLAS build).  Returns one
-    (n_m, 2) float64 array per submap."""
+    product ``@`` may fuse or reorder them, and then the bits depend on the BLAS build).  ``voxel`` (a cell
+    size, None or 0 for none) keeps of each submap only the first point of every grid cell, in merged order,
+    as ``IcpEngine.set_submaps(..., voxel=)`` does.  Returns one (n_m, 2) float64 array per submap."""
     if isinstance(scans, ScanTable):
         o = scans.offsets
         scans = [scans.xy[o[s]:o[s + 1]] for s in range(scans.n_scans)]
     ids, rows = _submap_args(members, transforms, len(scans))
+    v = _voxel_arg(voxel)
     out = []
     for mem, T6 in zip(ids, rows):
         parts = []
@@ -269,7 +300,12 @@ def merge_scans(scans, members, transforms) -> list:
             p = np.asarray(scans[s], dtype=np.float64)
             x, y = p[:, 0], p[:, 1]
             parts.append(np.stack(((t[0] * x + t[1] * y) + t[2], (t[3] * x + t[4] * y) + t[5]), axis=1))
-        out.append(np.concatenate(parts))
+        sub = np.concatenate(parts)
+        if v:
+            if not _coords_ok(sub):
+                raise ValueError(f"a merged coordinate is non-finite or beyond +-{MAX_COORD:g}; it has no cell")
+            sub = sub[_first_of_cell(sub, v)]
+        out.append(sub)
     return out
 
 
@@ -434,26 +470,46 @@ class IcpEngine:
                             keep=(xy_t, offsets_t))
 
     # -- submaps ------------------------------------------------------------------------------
-    def set_submaps(self, members, transforms) -> np.ndarray:
+    def set_submaps(self, members, transforms, voxel=None) -> np.ndarray:
         """Scans of the resident (base) table merged on the device into submaps appended to it
-        (icpb_set_submaps): submap m is the base scans ``members[m]`` in order, member k mapped into the
-        submap's frame by ``transforms[m][k]`` ((k_m, 3, 3)), with the bits of ``merge_scans``.  Returns the
-        submaps' scan ids, n_base .. n_base + M - 1, for ``run``, ``run_multistart`` and ``run_device``.  A
-        call replaces the previous submaps; ``set_submaps([], [])`` leaves the base table alone.  ValueError
-        for bad arguments and for merged coordinates beyond the library's bound, with the table unchanged."""
+        (icpb_set_submaps_voxel): submap m is the base scans ``members[m]`` in order, member k mapped into the
+        submap's frame by ``transforms[m][k]`` ((k_m, 3, 3)), with the bits of ``merge_scans``.  ``voxel`` (a
+        cell size >= MIN_VOXEL; None or 0 for none) thins every submap on the device to the first point of
+        every grid cell, as ``merge_scans(..., voxel=)`` does.  Returns the submaps' scan ids, n_base ..
+        n_base + M - 1, for ``run``, ``run_multistart`` and ``run_device``; ``table.lengths`` holds their
+        lengths.  A call replaces the previous submaps; ``set_submaps([], [])`` leaves the base table alone.
+        ValueError for bad arguments and for merged coordinates beyond the library's bound, with the table
+        unchanged."""
         if self.table is None:
             raise ValueError("no scan table set")
         base = self._base if self._base is not None else self.table
         ids, rows = _submap_args(members, transforms, base.n_scans)
+        v = _voxel_arg(voxel)
         sub_off = np.concatenate(([0], np.cumsum([len(a) for a in ids]))).astype(np.int64)
         mem = np.ascontiguousarray(np.concatenate(ids) if ids else np.zeros(0, np.int32))
         T6 = np.ascontiguousarray(np.concatenate(rows) if rows else np.zeros((0, 6)))
-        table = base
-        if ids:
-            table = ScanTable.from_lengths(np.concatenate((base.lengths, [int(base.lengths[a].sum()) for a in ids])))
-        self._replace_table(table, "icpb_set_submaps", _ptr(mem), _ptr(sub_off), _ptr(T6), len(ids),
-                            keep=self._keep, base=base if ids else None)
+        lens = np.zeros(len(ids), dtype=np.int64)
+        self._replace_table(base, "icpb_set_submaps_voxel", _ptr(mem), _ptr(sub_off), _ptr(T6), len(ids), v,
+                            _ptr(lens), keep=self._keep, base=base if ids else None)
+        if ids:                                  # the mirror from the lengths the library built
+            self.table = ScanTable.from_lengths(np.concatenate((base.lengths, lens)))
         return np.arange(base.n_scans, base.n_scans + len(ids))
+
+    def read_scans(self, ids) -> list:
+        """The points of resident scans ``ids`` (submaps included) as they are on the device (icpb_read_scans):
+        one (n, 2) float64 array per id."""
+        if self.table is None:
+            raise ValueError("no scan table set")
+        ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+        if ids.size and (ids.min() < 0 or ids.max() >= self.table.n_scans):
+            raise ValueError("scan id out of range")
+        o = self.table.offsets
+        out = []
+        for s in ids:
+            a = np.empty((int(o[s + 1] - o[s]), 2), dtype=np.float64)
+            _lib.check(self._L.icpb_read_scans(self._h, int(s), 1, _ptr(a)), "icpb_read_scans")
+            out.append(a)
+        return out
 
     # -- host-buffer run (the reference-facing call) -----------------------------------------
     def run(self, pairs, init_transforms=None, epsilon=0.01, max_iters=100, stopping_thresh=0.0001,

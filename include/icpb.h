@@ -53,6 +53,9 @@ extern "C" {
 #define ICPB_MAX_COORD        1e10
 #define ICPB_MAX_GUESS_LINEAR 1e3
 #define ICPB_MAX_GUESS_SHIFT  1e12
+/* The smallest nonzero cell size of the submap voxel filter (icpb_set_submaps_voxel): with
+ * |x| <= ICPB_MAX_COORD it keeps |x / voxel| <= 1e16, so every cell coordinate is exact in int64. */
+#define ICPB_MIN_VOXEL        1e-6
 
 /* Occupancy grid (icpb_occupancy_grid_*).  The Bresenham walk runs in 64-bit integers on cell
  * coordinates; with every |cell coordinate| <= ICPB_MAX_GRID_CELL = 2^60 a beam spans
@@ -156,6 +159,37 @@ int icpb_set_scans_device(icpb_handle h, const double *d_xy, const int64_t *d_of
  */
 int icpb_set_submaps(icpb_handle h, const int32_t *h_members, const int64_t *h_submap_off,
                      const double *h_member_T, int64_t n_submaps);
+
+/*
+ * icpb_set_submaps with a voxel filter: each submap is merged exactly as above (the same formula and the same
+ * check), then thinned to the first point of every grid cell.  In the submap's own frame the merged point
+ * (x', y') lies in cell (cx, cy) = ((int64) floor(x' / voxel), (int64) floor(y' / voxel)), the division
+ * correctly rounded (numpy's np.floor(x / v).astype(np.int64) gives the same bits).  A point is kept iff no
+ * earlier point of the same submap, in merged order (member order, then point order within a member), lies in
+ * the same cell; kept points keep their coordinates bit for bit and their merged order.  Cells are per submap.
+ * No averaging: a kept point is a real merged point, so a filtered submap can be restated on the host and every
+ * alignment against it checked bit for bit.
+ *   voxel         0 (no filter: exactly icpb_set_submaps, which is this call with voxel = 0 and
+ *                 h_submap_len = NULL), or a finite cell size >= ICPB_MIN_VOXEL
+ *   h_submap_len  NULL, or n_submaps outputs: each submap's length in the table (its kept count), on success
+ * icpb_scan_count, the offsets, the longest scan, the staging images and the split by scan length all follow
+ * the kept counts: a filtered submap that fits shared memory runs on the shared-memory kernel.
+ * Rejected before anything is written, on top of the rejections of icpb_set_submaps: a voxel that is NaN,
+ * +-inf, negative, or in (0, ICPB_MIN_VOXEL) (ICPB_EINVAL).  ICPB_ETOOLONG is judged on the merged length,
+ * before the filter: a submap beyond ~100 M merged points is refused even if the filter would shrink it.
+ * The resident table is written only once the whole filtered result is known.  Device memory: the handle's
+ * scratch grows to about 16 B (merged points) + 8-16 B (hash) + 8 B (flags and scan) per merged point.
+ * Synchronous; must not overlap an asynchronous icpb_run_device* on the same handle.
+ */
+int icpb_set_submaps_voxel(icpb_handle h, const int32_t *h_members, const int64_t *h_submap_off,
+                           const double *h_member_T, int64_t n_submaps, double voxel,
+                           int64_t *h_submap_len /* n_submaps outputs, may be NULL */);
+
+/* The points of resident scans [first, first + count), submaps included, in table order, into h_xy
+ * (2 doubles per point; the caller sizes it from the offsets).  ICPB_ENOSCANS without a table; ICPB_EINVAL
+ * for a null h_xy or a range outside the table.  Synchronous; like icpb_upload_scans, it must not overlap an
+ * asynchronous icpb_run_device* on the same handle. */
+int icpb_read_scans(icpb_handle h, int64_t first, int64_t count, double *h_xy);
 
 /*
  * B independent icp() calls (src/icp.py:72-97) in one launch -- replaces the joblib fan-out
